@@ -103,6 +103,14 @@ int ssac_push_row(const void* host_row_pinned, void* staging_dev, int64_t row_by
                   const int64_t* nbytes, const int64_t* src_off, int n_fields, double* sum_tree_dev, double* min_tree_dev,
                   int64_t capacity, int64_t tree_idx_off, int64_t tree_val_off, int wait_slot, void* wait_event, void* stream);
 int ssac_push_row_wait(int slot);
+/* ssac_push_row with a list of PER leaf writes instead of one (prioritised frame-deduplicated n-step ring: a push may evict
+ * transitions -- their leaves get sum 0, min +inf -- and add one at max_priority ** alpha).  The staging row holds, at
+ * leaves_off, int64 leaf[n_leaves], then float64 sum value[n_leaves], then float64 min value[n_leaves] (1..256 writes); they
+ * are applied in order (the last write of a leaf wins), each with the ancestor update of ssac_push_row, in the same launch
+ * as the field scatter. */
+int ssac_push_row_leaves(const void* host_row_pinned, void* staging_dev, int64_t row_bytes, int slot, void* const* dsts_dev,
+                         const int64_t* nbytes, const int64_t* src_off, int n_fields, double* sum_tree_dev, double* min_tree_dev,
+                         int64_t capacity, int64_t leaves_off, int n_leaves, int wait_slot, void* wait_event, void* stream);
 /* Fused pixel gather + DrQ / DrQv2 random shift + uint8 -> fp32 + aug_mix: augmentations.py:165-269,
  * learning_utils.py:193-206.   src u8 [capacity, C, H, W] -> dst f32 [B, C, H, W].
  * pad_mode 0: no shift, 1: replicate (DrQv2 integer crop), 2: reflect (DrQ v1), 3: RAD (augmentations.py:129-162:
@@ -143,6 +151,28 @@ int ssac_tree_set(double* sum_tree_dev, double* min_tree_dev, int64_t capacity, 
 int ssac_tree_sample(const double* sum_tree_dev, const double* min_tree_dev, int64_t capacity, int64_t n_filled,
                      const double* u01_dev, int B, double beta, int64_t* idx_out_dev, double* weight_out_dev,
                      void* stream);
+/* Prioritised replay over the frame-deduplicated n-step ring (SURVEY 8f N2).  A transition's leaf is its slot in the FIFO
+ * of valid starts, v mod ring_size (v = running count of starts); the trees have capacity >= ring_size leaves.
+ * scalars_dev = the ring's device int64 {n_valid, v_tail % ring_size, v_tail}; the live leaves are the circular range
+ * [v_tail, v_tail + n_valid) mod ring_size, every other leaf holds (sum 0, min +inf).
+ * ssac_tree_set_live: ssac_tree_set (n <= 1024, last write wins) that drops every id whose slot is not live when the
+ * kernel runs (evicted since it was sampled and not yet reused): a dead leaf never gets priority back. */
+int ssac_tree_set_live(double* sum_tree_dev, double* min_tree_dev, int64_t capacity, int64_t ring_size, const int64_t* scalars_dev,
+                       const int64_t* idx_dev, const double* val_dev, int64_t n, void* stream);
+/* Proportional draw + importance weights + the n-step resolve of ssac_nstep_resolve, in one launch (B <= 1024).
+ *   v_tail == 0 (no start evicted yet): exactly ssac_tree_sample with n_filled = n_valid (mass u * sum(0, n_valid-1)).
+ *   v_tail > 0: mass u * root sum (every live transition can be drawn); weights of replay.py:173-176 with N = n_valid and
+ *     p_min = min root / sum root.
+ * A descent that float64 rounding lands on a dead leaf is moved to the live leaf with the largest index below it, or, when
+ * no live leaf lies below it, to the oldest live leaf: no dead slot is ever returned.  slot_out = leaf ids (what
+ * ssac_tree_set_live takes), j_out (nullable) = FIFO positions (slot - v_tail) mod ring_size, weight_out (nullable)
+ * float64; the remaining arguments and outputs are those of ssac_nstep_resolve. */
+int ssac_nstep_tree_sample(const double* sum_tree_dev, const double* min_tree_dev, int64_t capacity, int64_t ring_size,
+                           const int64_t* scalars_dev, const double* u01_dev, int B, double beta, int64_t* slot_out_dev,
+                           int64_t* j_out_dev, double* weight_out_dev, const int64_t* valid_ring_dev, int n_step,
+                           const double* reward64_dev, const float* reward32_dev, const double* gamma_pows_dev,
+                           const int64_t* first_frame_dev, int64_t* idx_start_dev, int64_t* idx_last_dev, float* R_dev,
+                           int64_t* frame_s_dev, int64_t* frame_s1_dev, void* stream);
 
 /* ---- ensemble MLPs: agent.py:13-40 (Critic), nets/mlps.py:11-41,78-93,113-129 --------------------- */
 /* G independent 3-Linear ReLU MLPs  D -> H -> H -> O.  Parameters: W1 [nets,H,D] b1 [nets,H] W2 [nets,H,H]

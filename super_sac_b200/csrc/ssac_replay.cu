@@ -165,11 +165,13 @@ __global__ void __launch_bounds__(256) scatter_fields_kernel(const uint8_t* __re
   }
 }
 
-// One pushed transition: field scatter (blockIdx.y < n_fields) + the PER leaf / ancestor update (last block row; the
-// leaf index and priority are read from the staging row itself, so there is no dependency between the blocks).
+// One pushed transition: field scatter (blockIdx.y < n_fields) + the PER leaf / ancestor updates (last block row; leaf
+// indices and values are read from the staging row itself, so there is no dependency between the blocks).  Leaf i of the
+// n_leaves writes: int64 at staging + idx_off + 8i, sum value (float64) at sum_off + 8i, min value at min_off + 8i.
 __global__ void __launch_bounds__(256) push_row_kernel(const uint8_t* __restrict__ staging, ScatterArgs a, int n_fields,
                                                        double* __restrict__ sum_tree, double* __restrict__ min_tree,
-                                                       int64_t capacity, int64_t idx_off, int64_t val_off) {
+                                                       int64_t capacity, int64_t idx_off, int64_t sum_off, int64_t min_off,
+                                                       int n_leaves) {
   const int k = blockIdx.y;
   if (k < n_fields) {
     const uint8_t* src = staging + a.src_off[k];
@@ -181,36 +183,39 @@ __global__ void __launch_bounds__(256) push_row_kernel(const uint8_t* __restrict
     } else {
       for (int64_t i = tid; i < n; i += nth) dst[i] = src[i];
     }
-  } else if (blockIdx.x == 0 && sum_tree) {   // block-uniform condition (the branch contains a barrier)
-    // Leaf write + ancestor update of ONE leaf.  The siblings along the path are not touched by this update, so all of
-    // them are fetched in parallel (thread l owns level l, at most 62 levels) and the chain of parent values is then
-    // evaluated by thread 0 with the reference's operand order (left + right, min(left, right)): replay.py:263-281.
+  } else if (blockIdx.x == 0 && sum_tree) {   // block-uniform condition (the branch contains barriers)
+    // Leaf write + ancestor update, one leaf after the other (so the last write of a leaf wins).  The siblings along a
+    // path are not touched by its own update, so all of them are fetched in parallel (thread l owns level l, at most 62
+    // levels) and the chain of parent values is then evaluated by thread 0 with the reference's operand order
+    // (left + right, min(left, right)): replay.py:263-281.
     __shared__ double sib_sum[64], sib_min[64];
-    __shared__ int levels_sh;
     const int l = threadIdx.x;
-    const int64_t leaf = *reinterpret_cast<const int64_t*>(staging + idx_off);
-    const int64_t node0 = leaf + capacity;
     int levels = 0;
     for (int64_t c = capacity; c > 1; c >>= 1) ++levels;
-    if (l < levels && l < 64) {
-      const int64_t sib = (node0 >> l) ^ 1;
-      sib_sum[l] = sum_tree[sib];
-      sib_min[l] = min_tree[sib];
-    }
-    if (l == 0) levels_sh = levels;
-    __syncthreads();
-    if (l == 0) {
-      double vs = *reinterpret_cast<const double*>(staging + val_off), vm = vs;
-      sum_tree[node0] = vs;
-      min_tree[node0] = vm;
-      for (int k = 0; k < levels_sh; ++k) {
-        const int64_t node = node0 >> k;
-        const bool is_left = (node & 1) == 0;
-        vs = is_left ? vs + sib_sum[k] : sib_sum[k] + vs;
-        vm = is_left ? fmin(vm, sib_min[k]) : fmin(sib_min[k], vm);
-        sum_tree[node >> 1] = vs;
-        min_tree[node >> 1] = vm;
+    for (int i = 0; i < n_leaves; ++i) {
+      const int64_t leaf = reinterpret_cast<const int64_t*>(staging + idx_off)[i];
+      const int64_t node0 = leaf + capacity;
+      if (l < levels && l < 64) {
+        const int64_t sib = (node0 >> l) ^ 1;
+        sib_sum[l] = sum_tree[sib];
+        sib_min[l] = min_tree[sib];
       }
+      __syncthreads();
+      if (l == 0) {
+        double vs = reinterpret_cast<const double*>(staging + sum_off)[i];
+        double vm = reinterpret_cast<const double*>(staging + min_off)[i];
+        sum_tree[node0] = vs;
+        min_tree[node0] = vm;
+        for (int k = 0; k < levels; ++k) {
+          const int64_t node = node0 >> k;
+          const bool is_left = (node & 1) == 0;
+          vs = is_left ? vs + sib_sum[k] : sib_sum[k] + vs;
+          vm = is_left ? fmin(vm, sib_min[k]) : fmin(sib_min[k], vm);
+          sum_tree[node >> 1] = vs;
+          min_tree[node >> 1] = vm;
+        }
+      }
+      __syncthreads();   // the next leaf's siblings may lie on this path (global writes are visible block-wide)
     }
   }
 }
@@ -386,11 +391,21 @@ __global__ void __launch_bounds__(256) gather_rad_u8_kernel(const uint8_t* __res
 // float64 segment trees: replay.py:207-353
 // ------------------------------------------------------------------------------------------------
 // small update (n <= 1024): one block, last write wins on duplicate indices (numpy fancy assignment),
-// then the touched ancestors are recomputed level by level.
+// then the touched ancestors are recomputed level by level.  live (nullable, frame-deduplicated n-step ring): device int64
+// {n_valid, v_tail % ring_size}; an index whose FIFO position (idx - v_tail) mod ring_size is not below n_valid names a
+// transition evicted since it was sampled and is dropped (it never gives priority back to a dead leaf).
+__device__ __forceinline__ bool ring_slot_live(int64_t slot, int64_t ring_size, int64_t tail, int64_t n_valid) {
+  if (slot < 0 || slot >= ring_size) return false;
+  int64_t j = (slot - tail) % ring_size;
+  if (j < 0) j += ring_size;
+  return j < n_valid;
+}
+
 __global__ void __launch_bounds__(1024) tree_set_small_kernel(double* __restrict__ sum_tree,
                                                               double* __restrict__ min_tree, int64_t capacity,
                                                               const int64_t* __restrict__ idx,
-                                                              const double* __restrict__ val, int n) {
+                                                              const double* __restrict__ val, int n,
+                                                              const int64_t* __restrict__ live, int64_t ring_size) {
   // "last write wins": the writer of a leaf is the highest position t that names it.  A 2048-slot open-addressing
   // table in shared memory (key = leaf, value = max position) finds it in O(1) expected probes per element.
   constexpr int kSlots = 2048;
@@ -401,8 +416,9 @@ __global__ void __launch_bounds__(1024) tree_set_small_kernel(double* __restrict
   for (int i = t; i < kSlots; i += blockDim.x) { hkey[i] = kEmpty; hval[i] = -1; }
   __syncthreads();
   const unsigned long long key = t < n ? (unsigned long long)idx[t] : 0ull;
+  const bool act = t < n && (!live || ring_slot_live((int64_t)key, ring_size, live[1], live[0]));
   int slot = (int)((key * 0x9E3779B97F4A7C15ull) >> 53);   // top 11 bits
-  if (t < n) {
+  if (act) {
     while (true) {
       const unsigned long long prev = atomicCAS(&hkey[slot], kEmpty, key);
       if (prev == kEmpty || prev == key) { atomicMax(&hval[slot], t); break; }
@@ -411,7 +427,7 @@ __global__ void __launch_bounds__(1024) tree_set_small_kernel(double* __restrict
   }
   __syncthreads();
   int64_t node = 0;
-  if (t < n) {
+  if (act) {
     node = (int64_t)key + capacity;
     if (hval[slot] == t) {   // slot still addresses this thread's key
       sum_tree[node] = val[t];
@@ -421,7 +437,7 @@ __global__ void __launch_bounds__(1024) tree_set_small_kernel(double* __restrict
   __threadfence_block();
   __syncthreads();
   for (int64_t c = capacity; c > 1; c >>= 1) {
-    if (t < n) {
+    if (act) {
       node >>= 1;
       const double a = sum_tree[2 * node], b = sum_tree[2 * node + 1];
       const double ma = min_tree[2 * node], mb = min_tree[2 * node + 1];
@@ -584,45 +600,66 @@ int ssac_push_row_wait(int slot) {
   return 0;
 }
 
-int ssac_push_row(const void* host_row_pinned, void* staging_dev, int64_t row_bytes, int slot, void* const* dsts,
-                  const int64_t* nbytes, const int64_t* src_off, int n_fields, double* sum_tree, double* min_tree,
-                  int64_t capacity, int64_t tree_idx_off, int64_t tree_val_off, int wait_slot, void* wait_event, void* stream) {
+static int push_row_impl(const char* name, const void* host_row_pinned, void* staging_dev, int64_t row_bytes, int slot,
+                         void* const* dsts, const int64_t* nbytes, const int64_t* src_off, int n_fields, double* sum_tree,
+                         double* min_tree, int64_t capacity, int64_t idx_off, int64_t sum_off, int64_t min_off, int n_leaves,
+                         int wait_slot, void* wait_event, void* stream) {
+  const std::string fn(name);
   SSAC_REQUIRE(host_row_pinned && staging_dev && row_bytes > 0 && dsts && nbytes && src_off && n_fields > 0 &&
-                   n_fields < kMaxGatherArrays, "ssac_push_row: bad args (1..15 fields)");
-  SSAC_REQUIRE(slot >= 0 && slot < 64, "ssac_push_row: slot must be in 0..63");
-  SSAC_REQUIRE(!sum_tree || (min_tree && capacity > 0 && (capacity & (capacity - 1)) == 0 && tree_idx_off >= 0 &&
-                             tree_val_off >= 0 && (tree_idx_off & 7) == 0 && (tree_val_off & 7) == 0),
-               "ssac_push_row: bad tree arguments");
+                   n_fields < kMaxGatherArrays, (fn + ": bad args (1..15 fields)").c_str());
+  SSAC_REQUIRE(slot >= 0 && slot < 64, (fn + ": slot must be in 0..63").c_str());
+  SSAC_REQUIRE(!sum_tree || (min_tree && capacity > 0 && (capacity & (capacity - 1)) == 0 && idx_off >= 0 && sum_off >= 0 &&
+                             min_off >= 0 && ((idx_off | sum_off | min_off) & 7) == 0 && n_leaves >= 0 && n_leaves <= 256 &&
+                             idx_off + 8 * (int64_t)n_leaves <= row_bytes && sum_off + 8 * (int64_t)n_leaves <= row_bytes &&
+                             min_off + 8 * (int64_t)n_leaves <= row_bytes),
+               (fn + ": bad tree arguments").c_str());
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess || dev < 0 || dev >= 64) return fail(SSAC_E_BADARG, "ssac_push_row: bad device");
+  if (e != cudaSuccess || dev < 0 || dev >= 64) return fail(SSAC_E_BADARG, (fn + ": bad device").c_str());
   if (!g_push_events[dev][slot]) {
     e = cudaEventCreateWithFlags(&g_push_events[dev][slot], cudaEventDisableTiming);
-    if (e != cudaSuccess) { set_error(std::string("ssac_push_row event: ") + cudaGetErrorString(e)); return (int)e; }
+    if (e != cudaSuccess) { set_error(fn + " event: " + cudaGetErrorString(e)); return (int)e; }
   }
   ScatterArgs a;
   int64_t mx = 0;
   for (int k = 0; k < n_fields; ++k) {
-    SSAC_REQUIRE(dsts[k] && nbytes[k] > 0 && src_off[k] >= 0, "ssac_push_row: bad field");
+    SSAC_REQUIRE(dsts[k] && nbytes[k] > 0 && src_off[k] >= 0, (fn + ": bad field").c_str());
     a.dst[k] = dsts[k]; a.nbytes[k] = nbytes[k]; a.src_off[k] = src_off[k];
     if (nbytes[k] > mx) mx = nbytes[k];
   }
   if (wait_event) {   // (cross-call pipelined updates: the latest gather may still read the ring slot this push overwrites)
     e = cudaStreamWaitEvent((cudaStream_t)stream, (cudaEvent_t)wait_event, 0);
-    if (e != cudaSuccess) { set_error(std::string("ssac_push_row (wait event): ") + cudaGetErrorString(e)); return (int)e; }
+    if (e != cudaSuccess) { set_error(fn + " (wait event): " + cudaGetErrorString(e)); return (int)e; }
   }
   e = cudaMemcpyAsync(staging_dev, host_row_pinned, (size_t)row_bytes, cudaMemcpyHostToDevice, (cudaStream_t)stream);
   if (e == cudaSuccess) e = cudaEventRecord(g_push_events[dev][slot], (cudaStream_t)stream);
-  if (e != cudaSuccess) { set_error(std::string("ssac_push_row copy: ") + cudaGetErrorString(e)); return (int)e; }
+  if (e != cudaSuccess) { set_error(fn + " copy: " + cudaGetErrorString(e)); return (int)e; }
   g_push_recorded[dev][slot] = true;
   int gx = (int)((mx / 16 + 255) / 256);
   if (gx < 1) gx = 1;
   if (gx > 64) gx = 64;
   push_row_kernel<<<dim3(gx, n_fields + 1), 256, 0, (cudaStream_t)stream>>>((const uint8_t*)staging_dev, a, n_fields, sum_tree,
-                                                                           min_tree, capacity, tree_idx_off, tree_val_off);
-  SSAC_CHECK_LAUNCH("ssac_push_row");
+                                                                           min_tree, capacity, idx_off, sum_off, min_off,
+                                                                           n_leaves);
+  SSAC_CHECK_LAUNCH(name);
   if (wait_slot >= 0) return ssac_push_row_wait(wait_slot);   // the row the host fills next (its copy is 63 pushes old)
   return 0;
+}
+
+int ssac_push_row(const void* host_row_pinned, void* staging_dev, int64_t row_bytes, int slot, void* const* dsts,
+                  const int64_t* nbytes, const int64_t* src_off, int n_fields, double* sum_tree, double* min_tree,
+                  int64_t capacity, int64_t tree_idx_off, int64_t tree_val_off, int wait_slot, void* wait_event, void* stream) {
+  return push_row_impl("ssac_push_row", host_row_pinned, staging_dev, row_bytes, slot, dsts, nbytes, src_off, n_fields,
+                       sum_tree, min_tree, capacity, tree_idx_off, tree_val_off, tree_val_off, 1, wait_slot, wait_event, stream);
+}
+
+int ssac_push_row_leaves(const void* host_row_pinned, void* staging_dev, int64_t row_bytes, int slot, void* const* dsts,
+                         const int64_t* nbytes, const int64_t* src_off, int n_fields, double* sum_tree, double* min_tree,
+                         int64_t capacity, int64_t leaves_off, int n_leaves, int wait_slot, void* wait_event, void* stream) {
+  SSAC_REQUIRE(sum_tree && n_leaves > 0, "ssac_push_row_leaves: trees and at least one leaf write required");
+  return push_row_impl("ssac_push_row_leaves", host_row_pinned, staging_dev, row_bytes, slot, dsts, nbytes, src_off, n_fields,
+                       sum_tree, min_tree, capacity, leaves_off, leaves_off + 8 * (int64_t)n_leaves,
+                       leaves_off + 16 * (int64_t)n_leaves, n_leaves, wait_slot, wait_event, stream);
 }
 
 int ssac_gather_aug_u8(const uint8_t* src, float* dst, const int64_t* idx, const int32_t* shift, const float* noise,
@@ -682,38 +719,99 @@ int ssac_gather_aug_u8_ring(const uint8_t* frames, float* dst, const int64_t* fi
 //   when the environment hands out Python / float64 rewards, in float32 (float32(gamma^i) * r_i, NumPy's weak-scalar rule)
 //   when it hands out np.float32 -- and the frame indices of the two observation stacks.
 // ------------------------------------------------------------------------------------------------
+struct NStepResolve {
+  const int64_t* valid_ring;
+  int64_t cap;
+  int n_step;
+  const double* reward64;
+  const float* reward32;
+  const double* gamma_pows;
+  const int64_t* first_frame;
+  int64_t* idx_start;
+  int64_t* idx_last;
+  float* R;
+  int64_t* frame_s;
+  int64_t* frame_s1;
+};
+
+__device__ __forceinline__ void nstep_resolve_one(const NStepResolve& a, int b, int64_t j, int64_t v_tail) {
+  const int64_t cap = a.cap;
+  const int64_t s = a.valid_ring[(v_tail + j) % cap];
+  const int64_t l = (s + a.n_step - 1) % cap;
+  a.idx_start[b] = s;
+  a.idx_last[b] = l;
+  if (a.reward64) {
+    double r = a.reward64[s];
+    for (int i = 1; i < a.n_step; ++i) r = __dadd_rn(r, __dmul_rn(a.gamma_pows[i], a.reward64[(s + i) % cap]));
+    a.R[b] = (float)r;
+  } else {
+    float r = a.reward32[s];
+    for (int i = 1; i < a.n_step; ++i) r = __fadd_rn(r, __fmul_rn((float)a.gamma_pows[i], a.reward32[(s + i) % cap]));
+    a.R[b] = r;
+  }
+  if (a.first_frame) {
+    a.frame_s[b] = a.first_frame[s];
+    a.frame_s1[b] = a.first_frame[l] + 1;   // the next state's stack starts one frame later
+  }
+}
+
 __global__ void __launch_bounds__(256) nstep_resolve_kernel(const int64_t* __restrict__ j, int B,
-                                                            const int64_t* __restrict__ valid_ring,
-                                                            const int64_t* __restrict__ scalars, int64_t cap, int n_step,
-                                                            const double* __restrict__ reward64,
-                                                            const float* __restrict__ reward32,
-                                                            const double* __restrict__ gamma_pows,
-                                                            const int64_t* __restrict__ first_frame,
-                                                            int64_t* __restrict__ idx_start, int64_t* __restrict__ idx_last,
-                                                            float* __restrict__ R, int64_t* __restrict__ frame_s,
-                                                            int64_t* __restrict__ frame_s1) {
+                                                            const int64_t* __restrict__ scalars, NStepResolve a) {
   pdl_wait();
   pdl_trigger();
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const int64_t v_tail = scalars[1];
-  const int64_t s = valid_ring[(v_tail + j[b]) % cap];
-  const int64_t l = (s + n_step - 1) % cap;
-  idx_start[b] = s;
-  idx_last[b] = l;
-  if (reward64) {
-    double r = reward64[s];
-    for (int i = 1; i < n_step; ++i) r = __dadd_rn(r, __dmul_rn(gamma_pows[i], reward64[(s + i) % cap]));
-    R[b] = (float)r;
-  } else {
-    float r = reward32[s];
-    for (int i = 1; i < n_step; ++i) r = __fadd_rn(r, __fmul_rn((float)gamma_pows[i], reward32[(s + i) % cap]));
-    R[b] = r;
+  nstep_resolve_one(a, b, j[b], scalars[1]);
+}
+
+// Prioritised draw over the FIFO of valid starts (leaf of a start = its FIFO counter v mod ring_size) + the resolve above,
+// in one launch.  scalars = {n_valid, v_tail % ring_size, v_tail}.
+//   v_tail == 0 (no start evicted yet): the live leaves are 0 .. n_valid-1 and the draw is exactly tree_sample_kernel's --
+//     mass u * sum(0, n_valid-1) (the reference's prefix total), the same descent, the same weights.
+//   v_tail > 0: the live leaves are the circular range [v_tail, v_tail + n_valid) mod ring_size, dead leaves hold (0, +inf);
+//     mass u * root sum, so every live transition can be drawn.
+// A descent that float64 rounding lands on a dead leaf (it can only overshoot to the right of the mass it belongs to) is
+// moved to the live leaf with the largest index below it; when no live leaf lies below it, to the oldest live leaf.
+__global__ void __launch_bounds__(1024) nstep_tree_sample_kernel(const double* __restrict__ sum_tree,
+                                                                 const double* __restrict__ min_tree, int64_t capacity,
+                                                                 int64_t ring_size, const int64_t* __restrict__ scalars,
+                                                                 const double* __restrict__ u, int B, double beta,
+                                                                 int64_t* __restrict__ slot_out, int64_t* __restrict__ j_out,
+                                                                 double* __restrict__ w_out, NStepResolve a) {
+  __shared__ double total_sh;
+  const int64_t n = scalars[0], tail = scalars[1];
+  const bool evicted = scalars[2] > 0;
+  if (threadIdx.x == 0) total_sh = (evicted || n < 2) ? sum_tree[1] : tree_prefix_total(sum_tree, capacity, n - 2);
+  __syncthreads();
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  double prefix = u[b] * total_sh;
+  int64_t idx = 1;
+  while (idx < capacity) {  // replay.py:320-335
+    idx = 2 * idx;
+    const double v = sum_tree[idx];
+    if (!(v > prefix)) { prefix -= v; idx += 1; }
   }
-  if (first_frame) {
-    frame_s[b] = first_frame[s];
-    frame_s1[b] = first_frame[l] + 1;   // the next state's stack starts one frame later
+  int64_t leaf = idx - capacity;
+  if (!ring_slot_live(leaf, ring_size, tail, n)) {
+    if (leaf >= ring_size) leaf = ring_size - 1;
+    if (!ring_slot_live(leaf, ring_size, tail, n)) {
+      const int64_t head = (tail + n) % ring_size;   // the dead leaves are [head, tail) mod ring_size
+      leaf = (head >= 1 && head <= leaf) ? head - 1 : tail;
+    }
   }
+  int64_t j = (leaf - tail) % ring_size;
+  if (j < 0) j += ring_size;
+  slot_out[b] = leaf;
+  if (j_out) j_out[b] = j;
+  if (w_out) {  // replay.py:173-176 with N = number of live transitions
+    const double sum_all = sum_tree[1];
+    const double p_min = min_tree[1] / sum_all;
+    const double max_weight = pow(p_min * (double)n, -beta);
+    const double p_sample = sum_tree[capacity + leaf] / sum_all;
+    w_out[b] = pow(p_sample * (double)n, -beta) / max_weight;
+  }
+  nstep_resolve_one(a, b, j, tail);
 }
 
 int ssac_nstep_resolve(const int64_t* j_dev, int B, const int64_t* valid_ring_dev, const int64_t* scalars_dev, int64_t cap,
@@ -725,9 +823,9 @@ int ssac_nstep_resolve(const int64_t* j_dev, int B, const int64_t* valid_ring_de
   SSAC_REQUIRE((reward64_dev != nullptr) != (reward32_dev != nullptr), "ssac_nstep_resolve: exactly one reward array");
   SSAC_REQUIRE(B > 0 && cap > 0 && n_step >= 1 && n_step <= cap, "ssac_nstep_resolve: bad sizes");
   SSAC_REQUIRE(!first_frame_dev || (frame_s_dev && frame_s1_dev), "ssac_nstep_resolve: frame outputs missing");
-  launch_pdl(nstep_resolve_kernel, dim3((B + 255) / 256), dim3(256), 0, (cudaStream_t)stream, j_dev, B, valid_ring_dev, scalars_dev,
-             cap, n_step, reward64_dev, reward32_dev, gamma_pows_dev, first_frame_dev, idx_start_dev, idx_last_dev, R_dev,
-             frame_s_dev, frame_s1_dev);
+  const NStepResolve a{valid_ring_dev, cap, n_step, reward64_dev, reward32_dev, gamma_pows_dev, first_frame_dev,
+                       idx_start_dev, idx_last_dev, R_dev, frame_s_dev, frame_s1_dev};
+  launch_pdl(nstep_resolve_kernel, dim3((B + 255) / 256), dim3(256), 0, (cudaStream_t)stream, j_dev, B, scalars_dev, a);
   SSAC_CHECK_LAUNCH("ssac_nstep_resolve");
   return 0;
 }
@@ -738,7 +836,7 @@ int ssac_tree_set(double* sum_tree, double* min_tree, int64_t capacity, const in
   SSAC_REQUIRE(capacity > 0 && (capacity & (capacity - 1)) == 0, "ssac_tree_set: capacity must be a power of two");
   if (n <= 0) return 0;
   if (n <= 1024) {
-    tree_set_small_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(sum_tree, min_tree, capacity, idx, val, (int)n);
+    tree_set_small_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(sum_tree, min_tree, capacity, idx, val, (int)n, nullptr, 0);
     SSAC_CHECK_LAUNCH("ssac_tree_set(small)");
     return 0;
   }
@@ -765,6 +863,40 @@ int ssac_tree_sample(const double* sum_tree, const double* min_tree, int64_t cap
   tree_sample_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(sum_tree, min_tree, capacity, n_filled, u01_dev, B, beta,
                                                            idx_out, w_out);
   SSAC_CHECK_LAUNCH("ssac_tree_sample");
+  return 0;
+}
+
+int ssac_tree_set_live(double* sum_tree, double* min_tree, int64_t capacity, int64_t ring_size, const int64_t* scalars_dev,
+                       const int64_t* idx, const double* val, int64_t n, void* stream) {
+  SSAC_REQUIRE(sum_tree && min_tree && scalars_dev && idx && val, "ssac_tree_set_live: null pointer");
+  SSAC_REQUIRE(capacity > 0 && (capacity & (capacity - 1)) == 0 && ring_size > 0 && ring_size <= capacity,
+               "ssac_tree_set_live: need a power-of-two capacity >= ring_size > 0");
+  SSAC_REQUIRE(n <= 1024, "ssac_tree_set_live: at most 1024 ids per call");
+  if (n <= 0) return 0;
+  tree_set_small_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(sum_tree, min_tree, capacity, idx, val, (int)n, scalars_dev,
+                                                              ring_size);
+  SSAC_CHECK_LAUNCH("ssac_tree_set_live");
+  return 0;
+}
+
+int ssac_nstep_tree_sample(const double* sum_tree, const double* min_tree, int64_t capacity, int64_t ring_size,
+                           const int64_t* scalars_dev, const double* u01_dev, int B, double beta, int64_t* slot_out_dev,
+                           int64_t* j_out_dev, double* weight_out_dev, const int64_t* valid_ring_dev, int n_step,
+                           const double* reward64_dev, const float* reward32_dev, const double* gamma_pows_dev,
+                           const int64_t* first_frame_dev, int64_t* idx_start_dev, int64_t* idx_last_dev, float* R_dev,
+                           int64_t* frame_s_dev, int64_t* frame_s1_dev, void* stream) {
+  SSAC_REQUIRE(sum_tree && min_tree && scalars_dev && u01_dev && slot_out_dev && valid_ring_dev && gamma_pows_dev &&
+                   idx_start_dev && idx_last_dev && R_dev, "ssac_nstep_tree_sample: null pointer");
+  SSAC_REQUIRE(capacity > 0 && (capacity & (capacity - 1)) == 0 && ring_size > 0 && ring_size <= capacity,
+               "ssac_nstep_tree_sample: need a power-of-two capacity >= ring_size > 0");
+  SSAC_REQUIRE((reward64_dev != nullptr) != (reward32_dev != nullptr), "ssac_nstep_tree_sample: exactly one reward array");
+  SSAC_REQUIRE(B > 0 && B <= 1024 && n_step >= 1 && n_step <= ring_size, "ssac_nstep_tree_sample: need 0 < B <= 1024, bad n_step");
+  SSAC_REQUIRE(!first_frame_dev || (frame_s_dev && frame_s1_dev), "ssac_nstep_tree_sample: frame outputs missing");
+  const NStepResolve a{valid_ring_dev, ring_size, n_step, reward64_dev, reward32_dev, gamma_pows_dev, first_frame_dev,
+                       idx_start_dev, idx_last_dev, R_dev, frame_s_dev, frame_s1_dev};
+  nstep_tree_sample_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(sum_tree, min_tree, capacity, ring_size, scalars_dev, u01_dev,
+                                                                 B, beta, slot_out_dev, j_out_dev, weight_out_dev, a);
+  SSAC_CHECK_LAUNCH("ssac_nstep_tree_sample");
   return 0;
 }
 

@@ -436,9 +436,7 @@ def sample_move_and_augment(buffer, batch_size, augmenter, aug_mix, per=True, _i
     """Sample a batch on the device, cast to fp32, augment o and o1 with shared parameters and mix the first
     int(B*aug_mix) augmented rows into the batch (reference learning_utils.py:174-214)."""
     if getattr(buffer, "n_step_mode", False):   # one-step ring, n-step transitions assembled by the sampler (nstep_replay.py)
-        if per:
-            raise NotImplementedError("NStepReplayBuffer samples uniformly")
-        return buffer.nstep_sample_move_and_augment(batch_size, augmenter, aug_mix, _idx=_idx)
+        return buffer.nstep_sample_move_and_augment(batch_size, augmenter, aug_mix, _idx=_idx, per=per)
     assert len(buffer) >= batch_size
     st, dev, B = buffer._storage, buffer.device, batch_size
     if not torch.cuda.is_current_stream_capturing():

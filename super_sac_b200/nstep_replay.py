@@ -20,9 +20,19 @@ transition).
   rewards, float32 for np.float32 rewards), and the next state / done flag are those of step t+n-1.
 
 ``len(buffer)`` is the number of n-step transitions, as in the reference.  The learner keeps using ``gamma ** n_step``
-(main.py:388).  Uniform sampling only (the DrQ / DrQv2 configs that use n-step returns sample uniformly); one
-environment (``num_envs == 1``).  ``learning_utils.sample_move_and_augment`` -- hence every update entry point -- accepts
-this buffer in place of ``ReplayBuffer``.
+(main.py:388).  One environment (``num_envs == 1``).  ``learning_utils.sample_move_and_augment`` -- hence every update
+entry point -- accepts this buffer in place of ``ReplayBuffer``.
+
+Prioritised replay (``prioritized=True``; ``alpha`` / ``beta`` as in ``ReplayBuffer``): a transition is identified by
+its slot in the FIFO of valid starts, ``v % size`` with v the running count of starts, and that slot is its leaf in
+float64 sum / min trees laid out as ``ReplayBuffer``'s (root at 1, leaves at cap2 + i, cap2 = next power of two >= size).
+Until the first start is evicted the v-th start is the v-th tuple the reference's deque pushes, so trees, draws, weights
+and updates are bit-identical to a classic prioritised buffer fed those tuples in push order.  A push writes its leaves in
+the launch of its field scatter (ssac_push_row_leaves): a completed window gets ``max_priority ** alpha``, an evicted
+start (sum 0, min +inf).  After the first eviction a draw covers the whole live mass (root sum) and the weights use N =
+number of live transitions (ssac_nstep_tree_sample, DESIGN 5); ``update_priorities`` drops ids whose transition was
+evicted after it was sampled (ssac_tree_set_live).  ``sample`` / ``update_priorities`` /
+``sample_move_and_augment(per=True)`` raise on a buffer built without ``prioritized=True``.
 """
 import ctypes
 
@@ -30,14 +40,20 @@ import numpy as np
 import torch
 
 from . import _lib, _ops, _rng, augmentations, graphed
+from .replay import PriorityMax
 
 
-class NStepReplayBuffer:
+class NStepReplayBuffer(PriorityMax):
     _STAGE_SLOTS = 16
     n_step_mode = True
 
-    def __init__(self, size, n_step=1, gamma=0.99, frame_stack=1, frame_capacity=None, device=None, validate=True):
+    def __init__(self, size, n_step=1, gamma=0.99, frame_stack=1, frame_capacity=None, device=None, validate=True,
+                 prioritized=False, alpha=0.6, beta=1.0):
         assert n_step >= 1 and frame_stack >= 1 and size > n_step
+        assert alpha >= 0
+        self.prioritized, self.alpha, self.beta = bool(prioritized), alpha, beta
+        self._init_max_priority()
+        self._leaf_writes = []    # (leaf, sum value, min value) of the running push
         self._maxsize, self.n_step, self.gamma, self.frame_stack = int(size), int(n_step), float(gamma), int(frame_stack)
         self.device = torch.device(device if device is not None else "cuda")
         self._frame_cap = int(frame_capacity) if frame_capacity else int(size * 1.05) + 4 * frame_stack + 16
@@ -74,7 +90,7 @@ class NStepReplayBuffer:
         self.done = torch.zeros((cap, 1), dtype=torch.uint8, device=dev)
         self.first_frame = torch.zeros(cap, dtype=torch.int64, device=dev)
         self.valid_ring = torch.zeros(cap, dtype=torch.int64, device=dev)
-        self.scalars = torch.zeros(2, dtype=torch.int64, device=dev)   # {n_valid, v_tail}
+        self.scalars = torch.zeros(3, dtype=torch.int64, device=dev)   # {n_valid, v_tail % size, v_tail}
         self._n_filled_dev = self.scalars[0:1]   # what the index draw kernel reads (learning_utils.draw_for_critic_member)
         self.reward = None   # created by the first reward: float64 or float32 ring (see module docstring)
         self.gamma_pows = torch.tensor([self.gamma ** i for i in range(self.n_step)], dtype=torch.float64, device=dev)
@@ -82,6 +98,17 @@ class NStepReplayBuffer:
         self._first_frame_host = np.zeros(cap, dtype=np.int64)
         # one pinned staging row holds every field of the largest push (an episode start: k + 1 frames per key)
         row = sum((k + 1) * ((r[0].numel() * r.element_size() + 15) // 16 * 16) for r in self.frames.values()) + 16 * 16 + A * 4
+        # ... and the leaf writes of a push: at most k + 2 evicted starts (a push overwrites at most k + 1 frames, each the
+        # first frame of at most one step, plus the step the full ring drops) and the completed window
+        self._max_leaf_writes = k + 3
+        if self.prioritized:
+            cap2 = 1
+            while cap2 < cap:
+                cap2 *= 2
+            self._capacity = cap2
+            self._it_sum = torch.zeros(2 * cap2, dtype=torch.float64, device=dev)
+            self._it_min = torch.full((2 * cap2,), float("inf"), dtype=torch.float64, device=dev)
+            row += 24 * self._max_leaf_writes + 16
         self._stage = torch.empty((self._STAGE_SLOTS, (row + 4095) // 4096 * 4096), dtype=torch.uint8).pin_memory()
         self._stage_dev = torch.empty(self._stage.shape, dtype=torch.uint8, device=dev)
         self._stage_np = self._stage.numpy()
@@ -100,6 +127,8 @@ class NStepReplayBuffer:
         tail = (self._head - self._n_steps) % self._maxsize
         if self._is_start[tail]:
             self._is_start[tail] = False
+            if self.prioritized:
+                self._leaf_writes.append((self._v_tail % self._maxsize, 0.0, float("inf")))
             self._v_tail += 1
         self._n_steps -= 1
 
@@ -164,20 +193,27 @@ class NStepReplayBuffer:
             start = (p - self.n_step + 1) % cap
             self._is_start[start] = True
             fields.append((np.asarray([start], dtype=np.int64), self.valid_ring.data_ptr() + 8 * (self._v_head % cap)))
+            if self.prioritized:   # replay.py:129 (push with priorities=None)
+                v = self._max_priority ** self.alpha
+                self._leaf_writes.append((self._v_head % cap, v, v))
             self._v_head += 1
-        fields.append((np.asarray([self._v_head - self._v_tail, self._v_tail % cap], dtype=np.int64), self.scalars.data_ptr()))
+        fields.append((np.asarray([self._v_head - self._v_tail, self._v_tail % cap, self._v_tail], dtype=np.int64),
+                       self.scalars.data_ptr()))
         end = bool(done) if terminate_traj is None else bool(terminate_traj)
         if end:
             self._ep_len = 0
             self._last_next = None
         elif self._validate:
             self._last_next = {key: np.array(next_state[key], copy=True) for key in self.keys}
-        self._flush(fields)
+        leaves, self._leaf_writes = self._leaf_writes, []
+        self._flush(fields, leaves)
 
-    def _flush(self, fields):
+    def _flush(self, fields, leaves=()):
         """All fields of one push through ONE pinned staging row per <= 15 fields (ssac_push_row: one H2D copy + one
-        scatter kernel)."""
+        scatter kernel).  The leaf writes ride in the last row and its launch (ssac_push_row_leaves)."""
         L = _lib.lib()
+        assert len(leaves) <= self._max_leaf_writes
+        last = (len(fields) - 1) // 15 * 15
         for i in range(0, len(fields), 15):
             chunk = fields[i:i + 15]
             slot = self._stage_next
@@ -191,6 +227,16 @@ class NStepReplayBuffer:
                 dsts[j], nbytes[j], offs[j] = dst, nb, off
                 off += (nb + 15) // 16 * 16
             rb = self._stage.shape[1]
+            if leaves and i == last:
+                m = len(leaves)
+                ids, sums, mins = zip(*leaves)
+                row[off:off + 8 * m].view(np.int64)[:] = ids
+                row[off + 8 * m:off + 16 * m].view(np.float64)[:] = sums
+                row[off + 16 * m:off + 24 * m].view(np.float64)[:] = mins
+                L.push_row_leaves(self._stage.data_ptr() + slot * rb, self._stage_dev.data_ptr() + slot * rb, off + 24 * m, slot,
+                                  dsts, nbytes, offs, n, self._it_sum.data_ptr(), self._it_min.data_ptr(), self._capacity, off, m,
+                                  self._stage_next, None, _lib.stream_ptr())
+                continue
             L.push_row(self._stage.data_ptr() + slot * rb, self._stage_dev.data_ptr() + slot * rb, off, slot, dsts, nbytes, offs, n,
                        None, None, 0, 0, 0, self._stage_next, None, _lib.stream_ptr())
 
@@ -200,18 +246,49 @@ class NStepReplayBuffer:
             out = torch.empty(batch_size, dtype=torch.int64, device=self.device)
         return _rng.source().indices(out, len(self), self._n_filled_dev)
 
+    def _resolve_out(self, B):
+        dev = self.device
+        return dict(start=torch.empty(B, dtype=torch.int64, device=dev), last=torch.empty(B, dtype=torch.int64, device=dev),
+                    R=torch.empty((B, 1), dtype=torch.float32, device=dev), frame_s=torch.empty(B, dtype=torch.int64, device=dev),
+                    frame_s1=torch.empty(B, dtype=torch.int64, device=dev))
+
     def _resolve(self, j):
         """Positions j [B] in the FIFO of valid starts -> dict(start, last, R [B,1], frame_s, frame_s1)."""
-        B, dev = j.shape[0], self.device
-        out = dict(start=torch.empty(B, dtype=torch.int64, device=dev), last=torch.empty(B, dtype=torch.int64, device=dev),
-                   R=torch.empty((B, 1), dtype=torch.float32, device=dev), frame_s=torch.empty(B, dtype=torch.int64, device=dev),
-                   frame_s1=torch.empty(B, dtype=torch.int64, device=dev))
+        B = j.shape[0]
+        out = self._resolve_out(B)
         _lib.lib().nstep_resolve(j.data_ptr(), B, self.valid_ring.data_ptr(), self.scalars.data_ptr(), self._maxsize, self.n_step,
                                  None if self._reward_f32 else self.reward.data_ptr(),
                                  self.reward.data_ptr() if self._reward_f32 else None, self.gamma_pows.data_ptr(),
                                  self.first_frame.data_ptr(), out["start"].data_ptr(), out["last"].data_ptr(), out["R"].data_ptr(),
                                  out["frame_s"].data_ptr(), out["frame_s1"].data_ptr(), _lib.stream_ptr())
         return out
+
+    def _require_prioritized(self, what):
+        if not self.prioritized:
+            raise NotImplementedError(f"{what} needs NStepReplayBuffer(..., prioritized=True): this buffer samples uniformly")
+
+    def sample_per(self, batch_size):
+        """Proportional draw (float64 u from the draw source, replay.py:163-177) + resolve in one launch
+        (ssac_nstep_tree_sample) -> (dict of _resolve plus ``slot`` = leaf ids, ``j`` = FIFO positions; weights float64 [B])."""
+        self._require_prioritized("prioritised sampling")
+        B, dev = batch_size, self.device
+        n = len(self)
+        if n < (2 if self._v_tail == 0 else 1):
+            raise ValueError(f"NStepReplayBuffer: {n} transitions are too few to sample from")
+        u = torch.empty(B, dtype=torch.float64, device=dev)
+        _rng.source().uniform01(u)
+        out = self._resolve_out(B)
+        out["slot"] = torch.empty(B, dtype=torch.int64, device=dev)
+        out["j"] = torch.empty(B, dtype=torch.int64, device=dev)
+        w = torch.empty(B, dtype=torch.float64, device=dev)
+        _lib.lib().nstep_tree_sample(self._it_sum.data_ptr(), self._it_min.data_ptr(), self._capacity, self._maxsize,
+                                     self.scalars.data_ptr(), u.data_ptr(), B, float(self.beta), out["slot"].data_ptr(),
+                                     out["j"].data_ptr(), w.data_ptr(), self.valid_ring.data_ptr(), self.n_step,
+                                     None if self._reward_f32 else self.reward.data_ptr(),
+                                     self.reward.data_ptr() if self._reward_f32 else None, self.gamma_pows.data_ptr(),
+                                     self.first_frame.data_ptr(), out["start"].data_ptr(), out["last"].data_ptr(),
+                                     out["R"].data_ptr(), out["frame_s"].data_ptr(), out["frame_s1"].data_ptr(), _lib.stream_ptr())
+        return out, w
 
     def _gather_obs(self, key, frame_idx, shift, aug, B, aug_rows, use_aug):
         """fp32 observation batch of key ``key`` whose stacks start at frame counters ``frame_idx``."""
@@ -239,18 +316,23 @@ class NStepReplayBuffer:
         _ops.gather_rows([ring], [out], [n], [n], [0 if ring.dtype == torch.float32 else 1], fi, B)
         return out
 
-    def nstep_sample_move_and_augment(self, batch_size, augmenter, aug_mix, _idx=None):
-        """What learning_utils.sample_move_and_augment returns, for this buffer (fusable augmentations only)."""
+    def nstep_sample_move_and_augment(self, batch_size, augmenter, aug_mix, _idx=None, per=False):
+        """What learning_utils.sample_move_and_augment returns, for this buffer (fusable augmentations only).  per=True:
+        prioritised draw, ``imp_weights`` float64 [B] and ``priority_idxs`` = leaf ids (what update_priorities takes)."""
         from . import learning_utils as lu
 
+        if per:
+            self._require_prioritized("sample_move_and_augment(per=True)")
         assert len(self) >= batch_size
         B, dev = batch_size, self.device
         if not torch.cuda.is_current_stream_capturing():
             self.total_sample_calls += 1
         if not (isinstance(augmenter, augmentations.AugmentationSequence) and augmenter.fusable()):
             raise NotImplementedError("NStepReplayBuffer needs a fusable AugmentationSequence (Identity / DrQ / DrQv2)")
-        j = _idx if _idx is not None else self.sample_indices_uniform(B)
-        res = self._resolve(j)
+        if per:
+            res, imp_weights = self.sample_per(B)
+        else:
+            res = self._resolve(_idx if _idx is not None else self.sample_indices_uniform(B))
         aug = augmenter.aug_list[0]
         aug.change_randomization_params(dev)   # once per call; o and o1 share the shifts
         shift = getattr(aug, "shift", None)
@@ -289,8 +371,8 @@ class NStepReplayBuffer:
         rd["primary_batch"] = (o, a, res["R"], o1, d)
         if packed is not None:
             rd["_packed"] = packed
-        rd["priority_idxs"] = res["start"]
-        rd["imp_weights"] = lu._ones1(dev)
+        rd["priority_idxs"] = res["slot"] if per else res["start"]
+        rd["imp_weights"] = imp_weights if per else lu._ones1(dev)
         return rd
 
     # ---- reference API ---------------------------------------------------------------------------------------------
@@ -302,14 +384,16 @@ class NStepReplayBuffer:
 
     def _tuples(self, j):
         res = self._resolve(j)
-        B = j.shape[0]
+        return self._batch_of(res, j.shape[0]), res["start"].cpu().numpy()
+
+    def _batch_of(self, res, B):
         s, s1 = {}, {}
         ident = augmentations.IdentityAug(B)
         for key in self.keys:
             ring = self.frames[key]
             a_, b_ = (self._gather_obs(key, res[f], None, ident, B, 0, False) for f in ("frame_s", "frame_s1"))
             s[key], s1[key] = (a_.to(ring.dtype), b_.to(ring.dtype)) if ring.dtype == torch.uint8 else (a_, b_)
-        return (s, self.action[res["start"]], res["R"], s1, self.done[res["last"]]), res["start"].cpu().numpy()
+        return s, self.action[res["start"]], res["R"], s1, self.done[res["last"]]
 
     def get_all_transitions(self):
         """Every n-step transition currently in the buffer, oldest first."""
@@ -317,10 +401,41 @@ class NStepReplayBuffer:
         return self._tuples(torch.arange(len(self), dtype=torch.int64, device=self.device))[0]
 
     def sample(self, batch_size):
-        raise NotImplementedError("NStepReplayBuffer samples uniformly (the n-step configs of the reference do)")
+        """((s, a, R, s1, d), weights float64 [B], idxs) like ReplayBuffer.sample (idxs = leaf ids)."""
+        self._require_prioritized("NStepReplayBuffer.sample")
+        graphed.join()
+        self.total_sample_calls += 1
+        res, w = self.sample_per(batch_size)
+        return self._batch_of(res, batch_size), w, res["slot"].cpu().numpy()
+
+    def _tree_set_live(self, idx_dev, val_dev):
+        L = _lib.lib()
+        for i in range(0, idx_dev.numel(), 1024):   # in order: the last write of a leaf still wins
+            ii, vv = idx_dev[i:i + 1024], val_dev[i:i + 1024]
+            L.tree_set_live(self._it_sum.data_ptr(), self._it_min.data_ptr(), self._capacity, self._maxsize,
+                            self.scalars.data_ptr(), ii.data_ptr(), vv.data_ptr(), ii.numel(), _lib.stream_ptr())
 
     def update_priorities(self, idxes, priorities):
-        raise NotImplementedError("NStepReplayBuffer has no priorities")
+        """idxes (leaf ids from sample / priority_idxs) / priorities: numpy arrays or device tensors, like
+        ReplayBuffer.update_priorities.  Ids whose transition has been evicted since it was drawn (and whose slot no newer
+        transition has taken) are dropped on the device."""
+        self._require_prioritized("NStepReplayBuffer.update_priorities")
+        assert len(idxes) == len(priorities)
+        if not torch.cuda.is_current_stream_capturing():
+            graphed.join()
+        if torch.is_tensor(priorities):
+            idx_dev = idxes if torch.is_tensor(idxes) else torch.from_numpy(np.asarray(idxes, dtype=np.int64)).to(self.device)
+            pr = priorities.to(torch.float64)
+            self._tree_set_live(idx_dev.to(torch.int64).contiguous(), (pr**self.alpha).contiguous())
+            self._note_priorities_dev(pr)
+            return
+        idxes, priorities = np.asarray(idxes), np.asarray(priorities, dtype=np.float64)
+        assert np.min(priorities) > 0
+        assert np.min(idxes) >= 0
+        assert np.max(idxes) < self._maxsize
+        self._tree_set_live(torch.from_numpy(idxes.astype(np.int64)).to(self.device),
+                            torch.from_numpy(priorities**self.alpha).to(self.device))
+        self._max_priority = max(self._max_priority, float(np.max(priorities)))
 
     def bytes_per_transition(self):
         """Device bytes per stored step (frames once + bookkeeping) -- the reference layout stores 2k frames."""

@@ -110,7 +110,33 @@ class ReplayBufferStorage:
         return s, self.action_stack[:n].cpu().numpy(), self.reward_stack[:n].cpu().numpy(), s1, self.done_stack[:n].cpu().numpy()
 
 
-class ReplayBuffer:
+class PriorityMax:
+    """Running maximum of the priorities given to ``update_priorities`` (replay.py:190), the priority a new transition
+    gets.  Device-tensor updates only record a pending device-side maximum; it is folded into the host value (one sync)
+    when the next push reads it."""
+
+    def _init_max_priority(self):
+        self._max_priority_host = 1.0
+        self._max_priority_dev = None  # pending device-side maximum (folded in lazily: no sync per update)
+
+    @property
+    def _max_priority(self):
+        if self._max_priority_dev is not None:
+            self._max_priority_host = max(self._max_priority_host, float(self._max_priority_dev))
+            self._max_priority_dev = None
+        return self._max_priority_host
+
+    @_max_priority.setter
+    def _max_priority(self, v):
+        self._max_priority_host, self._max_priority_dev = float(v), None
+
+    def _note_priorities_dev(self, pr):
+        """pr: float64 device tensor of new priorities."""
+        m = pr.max()
+        self._max_priority_dev = m if self._max_priority_dev is None else torch.maximum(self._max_priority_dev, m)
+
+
+class ReplayBuffer(PriorityMax):
     """Uniform + prioritised replay (reference replay.py:98-190)."""
 
     def __init__(self, size, alpha=0.6, beta=1.0, device=None):
@@ -124,20 +150,8 @@ class ReplayBuffer:
             cap *= 2
         self._capacity = cap
         self._it_sum = self._it_min = None  # float64 [2*cap] device trees, created with the storage
-        self._max_priority_host = 1.0
-        self._max_priority_dev = None  # pending device-side maximum (folded in lazily: no sync per update)
+        self._init_max_priority()
         self.total_sample_calls = 0
-
-    @property
-    def _max_priority(self):
-        if self._max_priority_dev is not None:
-            self._max_priority_host = max(self._max_priority_host, float(self._max_priority_dev))
-            self._max_priority_dev = None
-        return self._max_priority_host
-
-    @_max_priority.setter
-    def _max_priority(self, v):
-        self._max_priority_host, self._max_priority_dev = float(v), None
 
     def __len__(self):
         return len(self._storage) if self._storage is not None else 0
@@ -314,8 +328,7 @@ class ReplayBuffer:
             idx_dev = idxes if torch.is_tensor(idxes) else torch.from_numpy(np.asarray(idxes, dtype=np.int64)).to(self.device)
             pr = priorities.to(torch.float64)
             self._tree_set(idx_dev, pr**self.alpha)
-            m = pr.max()
-            self._max_priority_dev = m if self._max_priority_dev is None else torch.maximum(self._max_priority_dev, m)
+            self._note_priorities_dev(pr)
             return
         idxes, priorities = np.asarray(idxes), np.asarray(priorities, dtype=np.float64)
         assert np.min(priorities) > 0
