@@ -198,7 +198,7 @@ int ssac_get_overlap(void);
  * produced.  0 = plain stream-ordered launches.  Results are identical.  Default 1. */
 int ssac_set_pdl(int on);
 int ssac_get_pdl(void);
-/* impl 2, 2 x 256-class networks (H in 32..256 and a multiple of 16, first-layer width <= 32, O <= 16): the whole forward
+/* impl 2, 2 x 256-class networks (H in 32..256 and a multiple of 16, first-layer width <= 64, O <= 32): the whole forward
  * (three layers + head epilogue) runs as ONE kernel that keeps the activations in tensor / shared memory.  h1 / h2 are
  * then written only when keep_hidden != 0 (a backward pass will read them); with keep_hidden == 0 their contents are
  * unspecified after the call.  Other shapes use the layered path (one launch per layer), which always needs the

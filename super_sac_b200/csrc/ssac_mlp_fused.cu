@@ -1,24 +1,28 @@
 // Whole-MLP forward in ONE kernel on the 5th-generation tensor cores: fc1 -> ReLU -> fc2 -> ReLU -> output layer ->
 // head epilogue (tanh-Normal sample / deterministic head / critic loss seed), for the 2 x 256 networks of the
-// REDQ / SAC / SUNRISE configurations (H in 32..256 and a multiple of 16, first-layer width <= 32, O <= 16).
-// sm_100a only.
+// REDQ / SAC / SUNRISE configurations and the SAC-Discrete heads (H in 32..256 and a multiple of 16, first-layer width
+// <= 64, O <= 32).  sm_100a only.
 //
 // The layered path (ssac_mlp_tc.cu) spends most of each of its three launches on fixed cost (launch, TMEM allocation,
 // pipeline fill, epilogue, drain) and round-trips h1 / h2 through global memory.  Here a CLUSTER OF CS = 2 OR 4 CTAs
 // (4 while the grid still fits the 148 SMs) owns 128 batch rows of one net and keeps the activations on chip:
 //
-//   layer 1  : every CTA computes the full h1 accumulator [128 x H] in tensor memory (K <= 32: one k-chunk, cheap, and
-//              it saves exchanging h1 between the CTAs); x and W1 are staged through registers (their 92-byte pitch
-//              is not TMA-addressable); the accumulator is then read into registers ONCE, before layer 2 starts
-//              (a tcgen05.ld issued while MMAs are in flight only completes when they drain)
+//   layer 1  : every CTA computes the full h1 accumulator [128 x H] in tensor memory (K <= 64: one or two k-chunks,
+//              cheap, and it saves exchanging h1 between the CTAs); x and W1 are staged through registers (their 92-byte
+//              pitch is not TMA-addressable); a second chunk (D > 32) is staged into the same A regions once the MMAs
+//              of the first have read them and accumulates into the same columns; the accumulator is then read into
+//              registers ONCE, before layer 2 starts (a tcgen05.ld issued while MMAs are in flight only completes when
+//              they drain)
 //   layer 2  : CTA r computes output columns [r*Hn, r*Hn + n_cnt) (Hn = H/CS rounded up to 32).  The A operand is
 //              produced from the layer-1 accumulator 32 columns at a time (tcgen05.ld -> +bias -> ReLU -> 3xTF32
 //              hi / lo planes in the swizzled UMMA layout) while TMA streams the matching W2 chunk into the B planes
 //              of a 3-stage ring; the three B planes are free from the first cycle, so three chunks are prefetched
 //              while layer 1 is still being staged
-//   layer 3  : O <= 16 outputs: fp32 FMAs straight from the layer-2 accumulator (thread = batch row), partial sums over
+//   layer 3  : O <= 32 outputs: fp32 FMAs straight from the layer-2 accumulator (thread = batch row), partial sums over
 //              each CTA's columns, CTAs 1.. push their partials into CTA 0's shared memory (DSMEM, 16-byte stores), CTA 0
 //              runs the head epilogue.  No third GEMM pipeline, no per-chunk TMA latency.  (no_head: stop after h2.)
+//              O > 16 (discrete heads): the landing zone would not fit next to the 193 KB of stages, so the partials land
+//              in CTA 0's stage 0, which is idle once every CTA of the cluster has passed one more cluster barrier
 //   PDL      : everything up to the first read of x (TMEM allocation, barrier init, biases, W1 / W3 loads, the first
 //              three W2 chunks) precedes griddepcontrol.wait and overlaps the previous kernel of the stream
 //
@@ -61,14 +65,14 @@ __device__ long long* g_trace_fz = nullptr;
 constexpr int FM = 128;                         // batch rows per cluster (MMA M)
 constexpr int FK = 32;                          // k per chunk
 constexpr int kMaxH = 256;
-constexpr int kMaxO = 16;
+constexpr int kMaxO = 32;
+constexpr int kMaxD = 2 * FK;                   // first-layer width: up to two k-chunks
 constexpr int kPlane = FM * FK * 4;             // 16 KB: one hi or lo plane of 128 rows x 32 k
 constexpr int kStage = 4 * kPlane;              // A_hi, A_lo, B_hi, B_lo = 64 KB
 constexpr int kNumStages = 3;
 constexpr int kSmem = kNumStages * kStage + 1024;
 constexpr uint32_t kTmemCols = 512;
 constexpr uint32_t kD2Col = 256;
-constexpr int kYPitch = kMaxO + 1;
 
 struct FusedFwd {
   CUtensorMap tmW2, tmH1, tmH2;
@@ -116,11 +120,12 @@ __device__ __forceinline__ void emit_planes(const float (&v)[16], int row, int h
   }
 }
 
-// OC: compile-time bound on the number of outputs (1, 4, 8, 12 or 16 >= O; rows O..OC-1 of the W3 slice are zero), so
-// that the output-layer FMAs are straight-line code on register-resident accumulators
+// OC: compile-time bound on the number of outputs (1, 4, 8, 12, 16, 24 or 32 >= O; rows O..OC-1 of the W3 slice are
+// zero), so that the output-layer FMAs are straight-line code on register-resident accumulators
 // CS: CTAs per cluster (2 or 4) = number of column slices of layer 2; 4 halves the per-CTA main loop again and is used
 // while the grid still fits the 148 SMs (small ensembles: the target actor, the REDQ target subset, 10 critics)
-template <int OC, int CS>
+// K2: first-layer width > 32, i.e. a second k-chunk (compiled out of the kernels of the narrow inputs)
+template <int OC, int CS, bool K2>
 __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_constant__ FusedFwd q) {
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t bar_raw[kNumStages];    // TMA -> workers: W2 chunk landed (=> B planes were free)
@@ -128,18 +133,27 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
   __shared__ __align__(8) uint64_t bar_empty[kNumStages];  // tensor core -> TMA producer: MMAs reading the stage done
   __shared__ __align__(8) uint64_t bar_l1in, bar_l1, bar_l2;
   __shared__ uint32_t tmem_base_sh;
-  __shared__ float b1s[kMaxH], b2s[kMaxH], b3s[kMaxO];
-  __shared__ __align__(16) float W3s[kMaxO][FM];           // this CTA's column slice of the output layer
+  constexpr int OW = OC <= 16 ? 16 : OC;                  // rows of the W3 slice / registers of the head epilogue
+  constexpr int YP = OW + 1;                               // ypart row pitch (conflict-free per-row stores)
+  constexpr bool kYInStage = OC > 16;                      // DSMEM landing zone in stage 0 (see the header)
+  __shared__ float b1s[kMaxH], b2s[kMaxH], b3s[OW];
+  __shared__ __align__(16) float W3s[OW][FM];              // this CTA's column slice of the output layer
   constexpr int OCP = (OC + 3) & ~3;
-  __shared__ __align__(16) float yx[CS - 1][FM][OCP];      // CTA 0: partial outputs pushed by CTAs 1 .. CS-1 (DSMEM)
+  // CTA 0: partial outputs pushed by CTAs 1 .. CS-1 (DSMEM); a placeholder when they land in stage 0
+  __shared__ __align__(16) float yx_s[kYInStage ? 1 : CS - 1][kYInStage ? 1 : FM][kYInStage ? 4 : OCP];
   __shared__ float red[2][4];
 
   if (threadIdx.x == 0) FZ_TRACE(0);
   FZ_GTRACE(0);
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  // per-CTA partial outputs of the two column-group parities: lives in the B planes of stage 2 (32 KB), idle once
-  // layer 2 has finished (the kept-h2 boxes use the B planes of stages 0 and 1)
-  float (*ypart)[FM][kYPitch] = reinterpret_cast<float (*)[FM][kYPitch]>(smem + 2 * kStage + 2 * kPlane);
+  // per-CTA partial outputs of the two column-group parities: lives in the B planes of stage 2 (32 KB; from its A_lo
+  // plane on, 48 KB, for O > 16), idle once layer 2 has finished (only the MMAs read them; the h1 store reads A_hi
+  // planes, the kept-h2 boxes use the B planes of stages 0 and 1)
+  float (*ypart)[FM][YP] =
+      reinterpret_cast<float (*)[FM][YP]>(smem + 2 * kStage + (kYInStage ? kPlane : 2 * kPlane));
+  static_assert(2 * FM * YP * 4 <= (kYInStage ? 3 : 2) * kPlane, "ypart overflows stage 2");
+  float (*yx)[FM][OCP] = kYInStage ? reinterpret_cast<float (*)[FM][OCP]>(smem) : reinterpret_cast<float (*)[FM][OCP]>(yx_s);
+  static_assert(!kYInStage || (CS - 1) * FM * OCP * 4 <= kStage, "DSMEM landing zone overflows stage 0");
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int rank = (int)cluster_rank();
   const int g = blockIdx.y, m0 = ((int)blockIdx.x / CS) * FM;
@@ -178,17 +192,17 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
   if (t < kMaxH) {
     b1s[t] = t < H ? __ldg(q.b1 + (int64_t)wg * H + t) : 0.f;
     b2s[t] = t < H ? __ldg(q.b2 + (int64_t)wg * H + t) : 0.f;
-    // this CTA's column slice of W3, zero padded to [16][128]; all eight loads of a thread are in flight together
-    float w3r[kMaxO * FM / kWorkerThreads];
+    // this CTA's column slice of W3, zero padded to [OW][128]; all loads of a thread are in flight together
+    float w3r[OW * FM / kWorkerThreads];
 #pragma unroll
-    for (int u = 0; u < kMaxO * FM / kWorkerThreads; ++u) {
+    for (int u = 0; u < OW * FM / kWorkerThreads; ++u) {
       const int i = t + kWorkerThreads * u, o = i / FM, c = i % FM;
       w3r[u] = (o < O && c < n_cnt) ? __ldg(q.W3 + ((int64_t)wg * O + o) * H + n_lo + c) : 0.f;
     }
 #pragma unroll
-    for (int u = 0; u < kMaxO * FM / kWorkerThreads; ++u) (&W3s[0][0])[t + kWorkerThreads * u] = w3r[u];
+    for (int u = 0; u < OW * FM / kWorkerThreads; ++u) (&W3s[0][0])[t + kWorkerThreads * u] = w3r[u];
   }
-  if (t < kMaxO) b3s[t] = t < O ? __ldg(q.b3 + (int64_t)wg * O + t) : 0.f;
+  if (t < OW) b3s[t] = t < O ? __ldg(q.b3 + (int64_t)wg * O + t) : 0.f;
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
@@ -243,7 +257,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
       // layer 1: x planes in the A region of stage 0, W1 hi / lo in the A regions of stages 1 / 2 (32 KB each)
       const uint32_t a_hi = sbase, a_lo = sbase + kPlane, b_hi = sbase + kStage, b_lo = sbase + 2 * kStage;
       const uint32_t idesc = instr_desc(H, 0, 0);
-      const int ksteps = (D + 7) / 8;
+      const int ksteps = K2 ? FK / 8 : (D + 7) / 8;
       for (int j = 0; j < ksteps; ++j) {
         const uint64_t dah = smem_desc(a_hi + j * 32, 16, 1024, 2), dal = smem_desc(a_lo + j * 32, 16, 1024, 2);
         const uint64_t dbh = smem_desc(b_hi + j * 32, 16, 1024, 2), dbl = smem_desc(b_lo + j * 32, 16, 1024, 2);
@@ -254,6 +268,25 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
       mma_commit(&bar_l1);
     }
     __syncwarp();
+    if (K2) {
+      // second k-chunk of layer 1 (columns 32 .. D-1), staged into the same A regions: accumulate
+      mbar_wait(&bar_l1in, 1);
+      fence_after_sync();
+      if (elect_one()) {
+        const uint32_t a_hi = sbase, a_lo = sbase + kPlane, b_hi = sbase + kStage, b_lo = sbase + 2 * kStage;
+        const uint32_t idesc = instr_desc(H, 0, 0);
+        const int ksteps = (D - FK + 7) / 8;
+        for (int j = 0; j < ksteps; ++j) {
+          const uint64_t dah = smem_desc(a_hi + j * 32, 16, 1024, 2), dal = smem_desc(a_lo + j * 32, 16, 1024, 2);
+          const uint64_t dbh = smem_desc(b_hi + j * 32, 16, 1024, 2), dbl = smem_desc(b_lo + j * 32, 16, 1024, 2);
+          mma_tf32(tmem, dal, dbh, idesc, 1u);
+          mma_tf32(tmem, dah, dbl, idesc, 1u);
+          mma_tf32(tmem, dah, dbh, idesc, 1u);
+        }
+        mma_commit(&bar_l1);
+      }
+      __syncwarp();
+    }
     const uint32_t idesc2 = instr_desc(n_cnt, 0, 0);
     for (int qi = 0; qi < nk; ++qi) {
       const int s = qi % kNumStages;
@@ -285,13 +318,29 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
     if (H > 128) store_kmajor(smem + kStage + kPlane, smem + 2 * kStage + kPlane, vc);
     fence_async_smem();
     mbar_arrive(&bar_l1in);
+    if (K2) {
+      // second k-chunk: its loads run while the tensor core reads the first, which it overwrites afterwards
+      const float* W1 = q.W1 + (int64_t)wg * H * D;
+      const bool w_vec = ((D & 3) == 0) && ((((uintptr_t)W1) & 15) == 0);
+      const float* X = q.x + (int64_t)g * q.x_gs;
+      const bool x_vec = ((q.ldx & 3) == 0) && ((((uintptr_t)X) & 15) == 0);
+      load_kmajor(va, X, q.ldx, m0, B, FK, D, x_vec);
+      load_kmajor(vb, W1, D, 0, H, FK, D, w_vec);
+      if (H > 128) load_kmajor(vc, W1, D, 128, H, FK, D, w_vec);
+      mbar_wait(&bar_l1, 0);   // first chunk's MMAs done: the A regions are free
+      store_kmajor(smem, smem + kPlane, va);
+      store_kmajor(smem + kStage, smem + 2 * kStage, vb);
+      if (H > 128) store_kmajor(smem + kStage + kPlane, smem + 2 * kStage + kPlane, vc);
+      fence_async_smem();
+      mbar_arrive(&bar_l1in);
+    }
     if (t == 0) FZ_TRACE(2);
     {
       // ---- layer-1 accumulator -> registers, all of it, BEFORE the layer-2 MMAs start (a tcgen05.ld issued while MMAs
       // are in flight only completes when they drain, which would serialise producer and tensor core): this thread keeps
       // its row's columns [128*half, 128*half + 128)
       uint32_t hr[4][32];
-      mbar_wait(&bar_l1, 0);   // layer-1 accumulator complete, A regions (x, W1) free again
+      mbar_wait(&bar_l1, K2 ? 1u : 0u);   // layer-1 accumulator complete, A regions (x, W1) free again
       fence_after_sync();
       if (t == 0) FZ_TRACE(3);
 #pragma unroll
@@ -400,6 +449,9 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
     return;
   }
   // ---- combine the two column halves: CTA 1 pushes its partial outputs into CTA 0's shared memory -----------------
+  // (landing in stage 0: first every CTA of the cluster past layer 3, i.e. CTA 0's MMAs drained and its h1 / h2 TMA
+  // stores done reading shared memory)
+  if (kYInStage) cluster_sync_all();
   if (rank > 0 && warp < 4) {
     const int row = warp * 32 + lane;
     // one 16-byte remote store per four outputs (remote stores are paid per request, not per byte)
@@ -426,9 +478,9 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
   if (rank == 0 && warp < 4) {
     // ---- head epilogue: thread = batch row, all O outputs in registers ---------------------------------------
     const int row = warp * 32 + lane;
-    float out[kMaxO];
+    float out[OW];
 #pragma unroll
-    for (int o = 0; o < kMaxO; ++o)
+    for (int o = 0; o < OW; ++o)
     {
       float v = 0.f;
       if (o < OC) {
@@ -445,7 +497,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
     if (row_ok && q.y) {
       float* yp = q.y + ((int64_t)g * B + b) * O;
 #pragma unroll
-      for (int o = 0; o < kMaxO; ++o)
+      for (int o = 0; o < OW; ++o)
         if (o < O) yp[o] = out[o];
     }
     if (epi.kind == 1) {
@@ -454,11 +506,11 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
       if (row_ok) {
         float lp = 0.f;
 #pragma unroll
-        for (int j = 0; j < kMaxO / 2; ++j) {
+        for (int j = 0; j < OW / 2; ++j) {
           if (j < A) {
             float mu = 0.f, raw = 0.f;
 #pragma unroll
-            for (int o = 0; o < kMaxO; ++o) {   // register-resident select (no dynamic indexing)
+            for (int o = 0; o < OW; ++o) {   // register-resident select (no dynamic indexing)
               if (o == j) mu = out[o];
               if (o == A + j) raw = out[o];
             }
@@ -479,7 +531,7 @@ __global__ void __launch_bounds__(kThreads, 1) mlp3_forward_kernel(const __grid_
     } else if (epi.kind == 2) {
       if (row_ok) {
 #pragma unroll
-        for (int j = 0; j < kMaxO; ++j) {
+        for (int j = 0; j < OW; ++j) {
           if (j < epi.A) {
             const int64_t i = (int64_t)b * epi.A + j;
             const float th = tanhf(out[j]);
@@ -548,7 +600,7 @@ int launch_mlp3_fused(const float* W1, const float* b1, const float* W2, const f
                       cudaStream_t s, int no_head) {
   if (!g_fused_forward || !tc::tma_enabled()) return -1;
   if (no_head && !keep_hidden) return -1;
-  if (H < 32 || H > fz::kMaxH || (H % 16) != 0 || D < 1 || D > fz::FK || O < 1 || O > fz::kMaxO) return -1;
+  if (H < 32 || H > fz::kMaxH || (H % 16) != 0 || D < 1 || D > fz::kMaxD || O < 1 || O > fz::kMaxO) return -1;
   if (epi && epi->kind == 1 && 2 * epi->A != O) return -1;
   if (epi && epi->kind == 2 && epi->A != O) return -1;
   if (keep_hidden && (!h1 || !h2)) return -1;
@@ -560,6 +612,7 @@ int launch_mlp3_fused(const float* W1, const float* b1, const float* W2, const f
     if (!tc::make_map(h2, H, (int64_t)B * H, H, B, false, &q.tmH2, G)) return -1;
   }
   // column slices per 128-row tile: 4 while the grid fits the SMs (and the DSMEM landing zone fits: O <= 12), else 2
+  // (O > 16 always 2: one partner's partials, landed in CTA 0's stage 0)
   const int tiles = (B + fz::FM - 1) / fz::FM;
   const int cs = (O <= 12 && (int64_t)G * tiles * 4 <= kNumSMs && H >= 128) ? 4 : 2;
   q.x = x; q.ldx = ldx; q.x_gs = x_gs; q.W1 = W1; q.b1 = b1; q.b2 = b2; q.W3 = W3; q.b3 = b3; q.net_index = net_index; q.y = y;
@@ -567,19 +620,24 @@ int launch_mlp3_fused(const float* W1, const float* b1, const float* W2, const f
   if (epi) q.epi = *epi;
   dim3 grid(cs * tiles, G);   // clusters of cs CTAs per 128-row tile
   cudaError_t le;
-#define SSAC_FZ_LAUNCH(OC_, CS_)                                                                                         \
+#define SSAC_FZ_LAUNCH1(OC_, CS_, K2_)                                                                                   \
   do {                                                                                                                   \
     static bool attr_set = false;                                                                                        \
     if (!attr_set) {                                                                                                     \
-      cudaError_t e = cudaFuncSetAttribute(fz::mlp3_forward_kernel<OC_, CS_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                           fz::kSmem);                                                                   \
+      cudaError_t e = cudaFuncSetAttribute(fz::mlp3_forward_kernel<OC_, CS_, K2_>,                                       \
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, fz::kSmem);                      \
       if (e != cudaSuccess) {                                                                                            \
         set_error(std::string("fused mlp forward (smem attribute): ") + cudaGetErrorString(e));                          \
         return (int)e;                                                                                                   \
       }                                                                                                                  \
       attr_set = true;                                                                                                   \
     }                                                                                                                    \
-    le = launch_cluster_pdl(fz::mlp3_forward_kernel<OC_, CS_>, grid, dim3(tc::kThreads), fz::kSmem, s, CS_, q);          \
+    le = launch_cluster_pdl(fz::mlp3_forward_kernel<OC_, CS_, K2_>, grid, dim3(tc::kThreads), fz::kSmem, s, CS_, q);     \
+  } while (0)
+#define SSAC_FZ_LAUNCH(OC_, CS_)                     \
+  do {                                               \
+    if (D > fz::FK) SSAC_FZ_LAUNCH1(OC_, CS_, true);  \
+    else SSAC_FZ_LAUNCH1(OC_, CS_, false);            \
   } while (0)
   if (cs == 4) {
     if (O == 1) SSAC_FZ_LAUNCH(1, 4);
@@ -591,9 +649,12 @@ int launch_mlp3_fused(const float* W1, const float* b1, const float* W2, const f
     else if (O <= 4) SSAC_FZ_LAUNCH(4, 2);
     else if (O <= 8) SSAC_FZ_LAUNCH(8, 2);
     else if (O <= 12) SSAC_FZ_LAUNCH(12, 2);
-    else SSAC_FZ_LAUNCH(16, 2);
+    else if (O <= 16) SSAC_FZ_LAUNCH(16, 2);
+    else if (O <= 24) SSAC_FZ_LAUNCH(24, 2);
+    else SSAC_FZ_LAUNCH(32, 2);
   }
 #undef SSAC_FZ_LAUNCH
+#undef SSAC_FZ_LAUNCH1
   if (le != cudaSuccess) {
     set_error(std::string("fused mlp forward: ") + cudaGetErrorString(le));
     return (int)le;

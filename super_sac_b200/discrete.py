@@ -4,11 +4,15 @@
 Same flat arenas, grouped MLP launches (ssac_mlp_forward / ssac_mlp_backward with O = number of actions: every critic
 net emits its whole Q row), fused Adam and device-side logs as the continuous path in learning.py; the categorical
 arithmetic around the networks (softmax, expectation over actions, gather at the taken action and its scatter back into
-the dense output gradient) runs in the ssac_discrete_* kernels (csrc/ssac_discrete.cu).  This is the first correct path:
-eager launches, members in series, no CUDA-graph capture / cross-update pipelining yet.  The offline (AFBC) actor update
+the dense output gradient) runs in the ssac_discrete_* kernels (csrc/ssac_discrete.cu).  Members run in series.  Nothing
+here allocates by host state, reads back or decides on the host (except the logged member, ``random.choice``, frozen at
+capture as in the continuous path), so ``learning.critic_update`` / ``online_actor_update`` replay these functions as
+CUDA graphs under ``graphed.enable_auto_graphs()``; inside ``lu.pipelined_updates()`` the target side of a one-member
+critic update runs on the block's front stream (as in learning._critic_update_impl).  The offline (AFBC) actor update
 with the indirect advantage filter (adv_estimator.py:45-56) and the priority refresh are here too.  Not implemented
 (raise): softmax Bellman weights (they draw Categorical samples), the invariance regularisers, sharded ensembles.
 """
+import contextlib
 import random
 
 import torch
@@ -64,9 +68,14 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
         s1_rep = target_agent.encoder(o1)
     X1, ld1 = _rows(s1_rep)
     B, dev = X1.shape[0], X1.device
-    logits = _forward(aa, i, 1, X1, ld1, B)
+    # the subset is drawn before the actor forward: the single-kernel forward reads net_index ahead of its PDL wait,
+    # which needs the draw at least two launches back (ssac_mlp_fused.cu).  The actor forward draws nothing, so the
+    # random numbers are the same as in the reference's order (policy, then subset).
     subset = torch.empty(M, dtype=torch.int32, device=dev)
     _rng.source().subsets(subset, N, M)                                     # agent.py:29
+    logits = _forward(aa, i, 1, X1, ld1, B)
+    if lu.pipeline() is not None:
+        lu.pipeline().front_wait_polyak()   # the target critics' parameters: the only thing this side reads that Polyak writes
     qt = _forward(target_agent._critic_arena, i * N, M, X1, ld1, B, net_index=subset)   # [M,B,A]
     v = torch.empty(B, dtype=torch.float32, device=dev)
     ev, eslot = dlogs.slots(1)                                              # zero-initialised with the buffer
@@ -125,22 +134,49 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
     _check(agent)
     if encoder_lambda:
         raise NotImplementedError("encoder invariance regulariser (lambda = 0 in every shipped config) is out of scope")
-    lu.pipeline_barrier()
+    from .learning import _encoder_trainable
+
     ca = agent._critic_arena
     dev = ca.device
     L, stream = _lib.lib(), _lib.stream_ptr()
     E, N, B, A = agent.ensemble_size, agent.num_critics, batch_size, agent.act_space_size
-    logs = _logs.DeviceLogs(dev)
+    # Inside lu.pipelined_updates(): the target side (draws, gather, actor logits and target-critic subset on s1, state
+    # value, TD target) runs on the front stream, the online side on the caller's; the same eligibility as the continuous
+    # path (one member, uniform sampling, plain Bellman backups, no trainable encoder), else serial.  PopArt stays serial
+    # too: the next update's TD target rescales the PopArt layer this update's loss seed still reads.
+    pipe = lu.pipeline()
+    if pipe is not None and (E != 1 or per or update_priorities or weight_type is not None or _encoder_trainable(agent)
+                             or any(bool(p) for p in agent.popart) or lu.side_stream(dev) is None or pipe.device != dev):
+        pipe = None
+    if pipe is None:
+        lu.pipeline_barrier()
+    else:
+        main = torch.cuda.current_stream(dev)
+        pipe.front_wait_dep(main)
+    with (torch.cuda.stream(pipe.front) if pipe is not None else contextlib.nullcontext()):
+        logs = _logs.DeviceLogs(dev)   # (zeroed on the stream that writes it first)
+    if pipe is not None:
+        pipe.keep.append(logs)
     loss_all, loss_slot = logs.slots(2 * E)   # per member: {loss contribution, mean td error of its last net}
     opt = _arena.FlatAdam.attach(critic_optimizer, ca)
     enc_outs, replay_dicts = [], []
     for i in range(E):
         loss_v = loss_all[2 * i:2 * i + 2]
-        rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
-        td_target, (s1_rep, _) = lu.compute_td_targets(
-            logs=logs, replay_dict=rd, agent=agent, target_agent=target_agent, ensemble_idx=i,
-            ensemble_n=target_critic_ensemble_n, log_alphas=log_alphas, pop=pop, gamma=gamma, random_process=None,
-            noise_clip=None, discrete=True)
+        with (torch.cuda.stream(pipe.front) if pipe is not None else contextlib.nullcontext()):
+            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
+            if pipe is not None:
+                batch_ready = torch.cuda.Event()
+                batch_ready.record(pipe.front)
+            td_target, (s1_rep, _) = lu.compute_td_targets(
+                logs=logs, replay_dict=rd, agent=agent, target_agent=target_agent, ensemble_idx=i,
+                ensemble_n=target_critic_ensemble_n, log_alphas=log_alphas, pop=pop, gamma=gamma, random_process=None,
+                noise_clip=None, discrete=True)
+            if pipe is not None:
+                target_ready = torch.cuda.Event()
+                target_ready.record(pipe.front)
+                pipe.keep.append((rd, td_target, s1_rep))
+        if pipe is not None:
+            main.wait_event(batch_ready)
         w = lu.compute_backup_weights(logs=logs, replay_dict=rd, agent=agent, target_agent=target_agent,
                                       weight_type=weight_type, weight_temp=weighted_bellman_temp, batch_size=B, discrete=True)
         o, a, *_ = rd["primary_batch"]
@@ -153,6 +189,8 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
         popart = agent.popart[i]
         imp = rd["imp_weights"].float().contiguous() if per else None          # per=False: ones(1), i.e. no weighting
         dy = torch.empty((N, B, A), dtype=torch.float32, device=dev)
+        if pipe is not None:
+            main.wait_event(target_ready)
         L.discrete_critic_loss_seed(q.data_ptr(), N, B, A, act.data_ptr(), td_target.data_ptr(),
                                     w.data_ptr() if torch.is_tensor(w) else None, None if imp is None else imp.data_ptr(),
                                     popart.state_ptr() if popart else None, int(bool(pop)), E, 0, dy.data_ptr(),
@@ -191,6 +229,8 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
                 torch.nn.utils.clip_grad_norm_(agent.encoder.parameters(), encoder_clip)
             encoder_optimizer.step()
     member = random.choice(range(E))
+    if pipe is not None:
+        pipe.main_wait_polyak(main)   # a Polyak step on the block's auxiliary stream still reads the online parameters
     opt.step(stream, max_norm=critic_clip if critic_clip else None)   # (clipping rescales the stored gradients, as the reference's does)
     gslot = lu._member_grad_norm_slot(logs, ca, member * N, (member + 1) * N)
     logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)

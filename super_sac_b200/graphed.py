@@ -55,7 +55,7 @@ _auto = {"on": False, "cache": {}, "min_calls": 2, "lazy": False, "pipeline": Fa
 
 
 def enable_auto_graphs(on=True, lazy_logs=False, pipeline=False):
-    """After ``enable_auto_graphs()``, ``learning.critic_update`` / ``online_actor_update`` / ``alpha_update`` replay a
+    """After ``enable_auto_graphs()``, ``learning.critic_update`` / ``online_actor_update`` (continuous or discrete) replay a
     captured CUDA graph from the third call with identical arguments on (same objects, same hyper-parameters): the call
     a user makes stays ``learning.critic_update(...)``, the ~20 launches and their Python marshalling collapse into one
     ``cudaGraphLaunch`` + one device->host copy of the logged scalars.  ``lazy_logs``: the returned dict materialises its

@@ -58,11 +58,13 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
     args = (buffer, agent, target_agent, critic_optimizer, encoder_optimizer, log_alphas, batch_size, gamma, critic_clip,
             encoder_clip, target_critic_ensemble_n, weighted_bellman_temp, weight_type, pop, augmenter, encoder_lambda,
             random_process, noise_clip, aug_mix, discrete, per, update_priorities, dr3_coeff)
-    if not discrete and not encoder_lambda and _graphable(agent, random_process, per, update_priorities, encoder_optimizer):
+    # (a discrete critic update reads no random_process: the exploration process a training loop passes does not matter)
+    if not encoder_lambda and _graphable(agent, None if discrete else random_process, per, update_priorities,
+                                         encoder_optimizer):
         key = ("critic", id(buffer), id(agent), id(target_agent), _opt_sig(critic_optimizer), id(encoder_optimizer),
                id(random_process),
                tuple(id(l) for l in log_alphas), batch_size, gamma, critic_clip, encoder_clip, target_critic_ensemble_n,
-               weighted_bellman_temp, weight_type, pop, id(augmenter), noise_clip, aug_mix, dr3_coeff,
+               weighted_bellman_temp, weight_type, pop, id(augmenter), noise_clip, aug_mix, dr3_coeff, discrete,
                _lib.lib().default_mlp_impl())
         opt = _arena.FlatAdam.attach(critic_optimizer, agent._critic_arena)
 
@@ -77,7 +79,8 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
         refs = (buffer, agent, target_agent, critic_optimizer, encoder_optimizer, tuple(log_alphas), augmenter, random_process)
         # cross-call pipelining (graphed._Cross) covers what lu.pipelined_updates covers, minus PopArt (device state that
         # both sides of an update touch)
-        cross_ok = (agent.ensemble_size == 1 and weight_type is None and not any(bool(p) for p in agent.popart)
+        # (discrete updates: not yet, their captures launch one after the other)
+        cross_ok = (not discrete and agent.ensemble_size == 1 and weight_type is None and not any(bool(p) for p in agent.popart)
                     and lu.side_stream(agent._critic_arena.device) is not None and not enc_trained)
         return graphed.run_cached(key, lambda: _critic_update_impl(*args), on_replay, refs=refs, cross_ok=cross_ok)
     graphed.join()
@@ -406,11 +409,12 @@ def online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_s
     # Graph the actor update only over the STATIC buffers of a graph-captured critic update: eager critic updates hand
     # out fresh replay dicts every step (whose ids CPython recycles), and a graph captured over those would replay on
     # freed memory.
-    if (not discrete and not use_baseline and premade_replay_dicts is not None
+    if (not use_baseline and premade_replay_dicts is not None
             and all(graphed.is_static(rd) for rd in premade_replay_dicts)
-            and _graphable(agent, random_process, per, False)):
+            and _graphable(agent, None if discrete else random_process, per, False)):
         key = ("actor", id(agent), _opt_sig(actor_optimizer), tuple(id(l) for l in log_alphas), batch_size, clip, pop,
-               tuple(id(rd) for rd in premade_replay_dicts), _lib.lib().default_mlp_impl(), id(random_process), noise_clip)
+               tuple(id(rd) for rd in premade_replay_dicts), _lib.lib().default_mlp_impl(), id(random_process), noise_clip,
+               discrete)
         opt = _arena.FlatAdam.attach(actor_optimizer, agent._actor_arena)
         refs = (agent, actor_optimizer, tuple(log_alphas), tuple(premade_replay_dicts), random_process)
         return graphed.run_cached(key, lambda: _online_actor_update_impl(*args), opt.note_replayed_step, refs=refs)

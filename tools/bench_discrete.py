@@ -1,18 +1,27 @@
 #!/usr/bin/env python
-"""SAC-Discrete step (SURVEY 8f N4) timed on the device: critic_update(discrete=True) + Polyak + online_actor_update +
-alpha_update through the drop-in API, eager launches (this path is not graph-captured yet), CUDA events around K steps.
-Atari-like head sizes: 64 features, H = 256, 18 actions, 2 critics, B = 256.  With --ref the UNMODIFIED reference
-(baseline/_ref) runs the same step through PyTorch-CUDA on the same GPU, as a labelled comparison.
+"""SAC-Discrete step (SURVEY 8f N4) timed on the device: critic_update(discrete=True) + Polyak every second step +
+online_actor_update + alpha_update, CUDA events around K steps.  Atari-like head sizes: 64 features, H = 256, 18 actions,
+2 critics, B = 256.  One run, one shape, four execution models:
 
-    python tools/bench_discrete.py --steps 300 --warmup 20 --ref > gpurun_out/r2_27_bench_discrete.json
-    ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file gpurun_out/r2_27_discrete_launches.csv \
-        python tools/bench_discrete.py --steps 2 --warmup 2
+    eager      the drop-in calls, eager launches, logs read back every step
+    auto       the same calls under graphed.enable_auto_graphs() (critic and actor updates replay graphs), logs read back
+               every step
+    utd        a block of --utd critic updates + Polyak every second one inside lu.pipelined_updates(), captured as ONE
+               GraphedCall; time per update
+    step_graph the full step (critic + Polyak/2 + actor + alpha) as one GraphedCall (two steps per capture, one with the
+               Polyak step); time per step
+
+plus kernel launches per eager step (a separate torch.profiler run) and the card's name and power limit.  With --ref the
+UNMODIFIED reference (baseline/_ref) runs the eager step through PyTorch-CUDA on the same GPU, as a labelled comparison.
+
+    python tools/bench_discrete.py --steps 300 --warmup 20 > bench_discrete.json
 """
 import argparse
 import copy
 import json
 import math
 import os
+import subprocess
 import sys
 from itertools import chain
 
@@ -60,7 +69,7 @@ def build(pkg, device, ours):
     te = -math.log(1.0 / A) * 0.98
     L, lu = pkg.learning, pkg.learning_utils
 
-    def step(k):
+    def critic(k):
         logs, rds = L.critic_update(
             buffer=buf, agent=agent, target_agent=target, critic_optimizer=critic_opt, encoder_optimizer=enc_opt,
             log_alphas=[la], batch_size=B, gamma=0.99, critic_clip=None, encoder_clip=None, target_critic_ensemble_n=M,
@@ -69,14 +78,21 @@ def build(pkg, device, ours):
         if k % 2 == 0:
             for ac, tc in zip(agent.critics, target.critics):
                 lu.soft_update(tc, ac, 0.005)
+        return logs, rds
+
+    def step(k, read=True):
+        logs, rds = critic(k)
         alogs = L.online_actor_update(
             buffer=buf, agent=agent, pop=False, actor_optimizer=actor_opt, log_alphas=[la], batch_size=B, clip=None,
             random_process=None, noise_clip=None, augmenter=aug, aug_mix=0.0, premade_replay_dicts=rds, per=False,
             discrete=True, use_baseline=False)
         L.alpha_update(buffer=buf, agent=agent, optimizers=[alpha_opt], batch_size=B, log_alphas=[la], augmenter=aug,
                        aug_mix=0.0, target_entropy=te, premade_replay_dicts=rds, discrete=True)
-        return float(logs["losses/critic_overall_loss"]), float(alogs["losses/actor_pg_loss"])
+        if read:   # (not while a graph is being captured: the logs are read back after each replay)
+            return float(logs["losses/critic_overall_loss"]), float(alogs["losses/actor_pg_loss"])
+        return logs, alogs
 
+    step.critic = critic
     return step
 
 
@@ -93,19 +109,93 @@ def timed(step, steps, warmup):
     return e0.elapsed_time(e1) / steps, out
 
 
+def launches_per_step(step, steps=4):
+    """Kernel launches of `steps` eager steps, from torch.profiler (CUDA activities), per step."""
+    from torch.profiler import ProfilerActivity, profile
+
+    for k in range(2):
+        step(k)
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for k in range(steps):
+            step(k)
+        torch.cuda.synchronize()
+    kernels = [e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA
+               and not e.name.startswith(("Memcpy", "Memset", "[memory]"))]
+    return len(kernels) / steps
+
+
+def card():
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                           text=True, timeout=30).stdout.strip().splitlines()[0]
+    except Exception:   # noqa: BLE001 -- the card's name still comes from the runtime
+        q = f"{torch.cuda.get_device_name(0)}, power limit unknown"
+    return q
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=300)
     ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--utd", type=int, default=8)
     ap.add_argument("--ref", action="store_true")
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     import super_sac_b200 as ssb
+    from super_sac_b200 import graphed, learning_utils as lu
 
     ms, out = timed(build(ssb, dev, True), args.steps, args.warmup)
+
+    # (a) the same drop-in calls, replayed from graphs from the third call on
+    graphed.enable_auto_graphs(True)
+    try:
+        ms_auto, _ = timed(build(ssb, dev, True), args.steps, args.warmup)
+    finally:
+        graphed.enable_auto_graphs(False)
+
+    # (b) a UTD block of critic updates (+ Polyak every second) inside lu.pipelined_updates(), one graph
+    step = build(ssb, dev, True)
+
+    def utd_block():
+        with lu.pipelined_updates():
+            for k in range(args.utd):
+                logs, _ = step.critic(k)
+        return logs
+
+    g_utd = graphed.GraphedCall(utd_block, warmup=2)
+    ms_utd, _ = timed(lambda k: g_utd.replay(), max(1, args.steps // args.utd), 3)
+    ms_utd /= args.utd
+    utd_logs = g_utd.logs()
+
+    # (c) the full step as one graph (two steps: with and without the Polyak step)
+    step = build(ssb, dev, True)
+
+    def two_steps():
+        step(0, read=False)
+        return step(1, read=False)
+
+    g_step = graphed.GraphedCall(two_steps, warmup=2)
+    ms_graph, _ = timed(lambda k: g_step.replay(), max(1, args.steps // 2), 3)
+    ms_graph /= 2
+
+    try:
+        n_launch = launches_per_step(build(ssb, dev, True))
+    except Exception as e:   # noqa: BLE001 -- the timings above stand without the count
+        n_launch = f"not measured: {e!r}"
     line = {"metric": "sac_discrete_steps_per_sec", "unit": "steps/s", "value": 1e3 / ms, "ms_per_step": ms,
             "config": {"workload": f"SAC-Discrete step (critic + Polyak/2 + actor + alpha), S={S} H={H} A={A} N={N} B={B}",
                        "mode": "eager launches, logs read back every step"},
+            "auto_graphs": {"ms_per_step": ms_auto, "value": 1e3 / ms_auto,
+                            "mode": "drop-in calls under enable_auto_graphs(), logs read back every step"},
+            "utd_block": {"us_per_update": 1e3 * ms_utd, "updates_per_block": args.utd,
+                          "mode": "critic updates + Polyak/2 inside pipelined_updates(), one GraphedCall per block",
+                          "last_loss": float(utd_logs["losses/critic_overall_loss"])},
+            "step_graph": {"ms_per_step": ms_graph, "value": 1e3 / ms_graph,
+                           "mode": "critic + Polyak/2 + actor + alpha as one GraphedCall"},
+            "eager_kernel_launches_per_step": n_launch,
+            "fused_forward": bool(ssb._lib.lib().get_fused_forward()),
+            "card": card(),
             "steps": args.steps, "warmup": args.warmup, "dtype": "f32", "last_losses": out}
     if args.ref:
         from baseline import ref_import
