@@ -46,7 +46,7 @@ int ssac_polyak(float* target_dev, const float* source_dev, int64_t n, double ta
 int ssac_polyak_multi(const uint64_t* table_dev, int n_tensors, int64_t max_numel, double tau, void* stream);
 
 /* ---- optimiser: torch.optim.Adam as configured in main.py:188-239 (coupled L2, no amsgrad) -------- */
-/* ctl_dev: int32[2] (int32[8] when shared with ssac_mlp_backward_post_adam) = {step, blocks_done}; the kernel reads step, uses t = step+1 for the bias
+/* ctl_dev: int32[2] = {step, blocks_done}; the kernel reads step, uses t = step+1 for the bias
  * corrections and the last block to finish stores step+1 (graph replays advance it).
  * gnorm_sq_dev (nullable): if given with max_norm > 0, grads are scaled by
  * min(1, max_norm/(sqrt(*gnorm_sq_dev)+1e-6)) (torch.nn.utils.clip_grad_norm_, learning.py:122-128) and,
@@ -236,20 +236,6 @@ int ssac_mlp_backward_post(const float* W3, int G, int D, int H, const float* x_
                            const float* h1_dev, const float* h2_dev, const float* dq_dev, float* ws_dev, float* gW1,
                            float* gb1, float* gW2, float* gb2, float* gW3, float* gb3, int impl, void* stream);
 
-/* _post with the optimiser step folded into its two branches: the gW1 / gb1 / gW3 / gb3 reduction applies Adam to the
- * elements it has just produced (behind the gW2 GEMM, the last reader of W3), an Adam launch over W2 / b2 follows the gW2
- * GEMM on `stream` (behind the u GEMM of an asynchronous _pre, the last reader of W2); no separate pass over the arena
- * after the join, gradients still written.  The parameter / exp_avg / exp_avg_sq of a gradient element sit at float
- * offsets param_off / exp_avg_off / exp_avg_sq_off from the gradient's own address (twin arenas with one layout; W2 and
- * b2 adjacent).  ctl_dev: int32[8], [0] = step as in ssac_adam_step (the same counter; it advances once per call, when
- * both branches are done), [2..4] scratch counters, zero-initialised.  No gradient clipping (that needs the global norm
- * first: use _post + ssac_adam_step).  Same arithmetic per element as ssac_adam_step. */
-int ssac_mlp_backward_post_adam(const float* W3, int G, int D, int H, const float* x_dev, int64_t ldx, int64_t x_gs, int B,
-                                const float* h1_dev, const float* h2_dev, const float* dq_dev, float* ws_dev, float* gW1,
-                                float* gb1, float* gW2, float* gb2, float* gW3, float* gb3, int64_t param_off,
-                                int64_t exp_avg_off, int64_t exp_avg_sq_off, int32_t* ctl_dev, double lr, double beta1,
-                                double beta2, double eps, double weight_decay, int impl, void* stream);
-
 /* The actor update's pass through an ensemble of scalar-output critics (learning.py:400-418): from the seed dq [G,B]
  * (ssac_actor_loss_seed: non-zero on each row's arg-min net only) straight to the action gradient summed over the nets,
  * da[b][a] = sum_g dQ_g/dx[b][col0 + a] * dq[g][b], without materialising the per-net input gradients (replaces
@@ -287,22 +273,11 @@ int ssac_critic_forward_loss(const float* W1, const float* b1, const float* W2, 
  * One launch of ceil(B/8) clusters x 4 CTAs; every cluster walks the whole chain for 8 batch rows (layer slices per CTA,
  * activations exchanged over distributed shared memory).  H in 32..256 (multiple of 8), first-layer width <= 64, O <= 16;
  * ssac_rows_supported(D, H, O) tells.  No activations are kept (forward-only uses).
- *
- * ssac_target_chain: the TD-target path of one member (learning_utils.py:314-338, agent.py:22-40): a1, logp = pi(s1)
- * (policy head as in ssac_actor_forward_sample) written into the action columns x1[:, S:], then the M critics
- * net_index[m] (NULL: 0..M-1) of the given stack on (s1, a1): qt [M,B].  Replaces ssac_actor_forward_sample +
- * ssac_mlp_forward(net_index), two tensor-core launches whose 8- and 16-CTA grids are pure latency.
  * ssac_policy_rows: one actor with its head (acting path agent.py:204-327, forward-only policy samples); out_dev
  * (nullable) receives the raw output layer [B, 2A | A]. */
 int ssac_rows_supported(int D, int H, int O);
 /* 0: ssac_rows_supported answers 0 for every shape, i.e. callers keep the tensor-core launches (A/B switch).  Default 1. */
 int ssac_set_rows_enabled(int on);
-int ssac_target_chain(const float* aW1, const float* ab1, const float* aW2, const float* ab2, const float* aW3,
-                      const float* ab3, int S, int H, int A, int deterministic, const float* cW1, const float* cb1,
-                      const float* cW2, const float* cb2, const float* cW3, const float* cb3,
-                      const int32_t* net_index_dev, int M, float* x1_dev, int64_t ldx, int B, const float* eps_dev,
-                      const float* noise_dev, float sigma, float clip, float log_std_lo, float log_std_hi,
-                      float* logp_dev, float* qt_dev, void* stream);
 int ssac_policy_rows(const float* W1, const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
                      int D, int H, int A, int deterministic, const float* x_dev, int64_t ldx, int B, float* out_dev,
                      const float* eps_dev, const float* noise_dev, float sigma, float clip, float log_std_lo,
@@ -451,15 +426,15 @@ int ssac_peer_wait(const void* my_buf_dev, int64_t half_bytes, int64_t nbytes, c
  * ws_dev: caller-owned workspace of ssac_conv_encoder_ws_floats floats, ZERO-INITIALISED once by the caller (padding
  * channels / pixels are never written); it carries the activations from a forward with save = 1 to its backward.
  * save = 0: no backward will follow (target encoder, acting path): activations ping-pong between two buffers.
- * out_dev f32 [B,out_dim].  backward: dout_dev = dL/dout, out_dev = the forward's output, obs_dev = the forward's input (the
- * first layer's weight gradient re-reads the image patches instead of keeping an im2col copy); every gradient is WRITTEN
- * (not accumulated).  ssac_conv_encoder_ws_offsets (tests / tools): int64[32] = float offsets of {x0, y1..y4, dz1..dz4, wfc,
+ * out_dev f32 [B,out_dim].  backward: dout_dev = dL/dout, out_dev = the forward's output, obs_dev = the forward's input (not
+ * read: the first layer's weight gradient reads the space-to-depth copy of it that the forward left in ws_dev); every
+ * gradient is WRITTEN (not accumulated).  ssac_conv_encoder_ws_offsets (tests / tools): int64[32] = float offsets of {x0, y1..y4, dz1..dz4, wfc,
  * gwfc, fc partials, xhat, rstd, dfc, dl} followed by {rows R1..R4, pitches P1..P4 of the four layers' grids, kf, kf padded,
  * split size, splits, total}.  Layer l works on its INPUT grid R_l x P_l per image: y_l (l = 1..3) is stored compacted on
  * layer l+1's grid, y4 on layer 4's own grid (valid region R4-2 x P4-2), dz_l on layer l's grid. */
 /* debugging switch (results do not depend on it): bit 0 = halo tiles (one TMA box per tile instead of one per filter tap) in
- * the forward / data-gradient kernel, bit 1 = in the weight-gradient kernel, bit 2 = first layer built straight from the
- * observation (measured slower than the default space-to-depth copy); default 3.  Set before the first workspace is planned. */
+ * the forward / data-gradient kernel, bit 1 = in the weight-gradient kernel; a cleared bit forces the per-tap kernel, which
+ * otherwise only runs where the halo box does not fit.  mode 0..3, default 3. */
 int ssac_set_conv_halo(int mode);
 int ssac_conv_encoder_ws_floats(int B, int C, int H, int W, int out_dim, int save, int64_t* n_floats_out);
 int ssac_conv_encoder_ws_offsets(int B, int C, int H, int W, int out_dim, int save, int64_t* offsets_out);

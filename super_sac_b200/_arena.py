@@ -150,7 +150,7 @@ class FlatAdam:
         dev = arena.device
         self.m = torch.zeros_like(arena.flat)
         self.v = torch.zeros_like(arena.flat)
-        self.ctl = torch.zeros(8, dtype=torch.int32, device=dev)   # [0] step, [1] blocks done, [2..4] fused-epilogue counters
+        self.ctl = torch.zeros(2, dtype=torch.int32, device=dev)   # [0] step, [1] blocks done
         self.gnorm_sq = torch.zeros(1, dtype=torch.float32, device=dev)
         self.steps = 0
         self._step_tensor = torch.zeros((), dtype=torch.float32)
@@ -218,19 +218,6 @@ class FlatAdam:
             _lib.lib().adam_step(a.flat.data_ptr(), a.grad.data_ptr(), self.m.data_ptr(), self.v.data_ptr(), a.numel,
                                  self.ctl.data_ptr(), lr, b1, b2, eps, wd, gptr, float(max_norm or 0.0), 1, stream)
         if not torch.cuda.is_current_stream_capturing():   # a captured step executes (and is counted) at replay time
-            self.steps += 1
-            self._step_tensor.fill_(self.steps)
-
-    def fused_offsets(self):
-        """Float offsets from a gradient element to its parameter / exp_avg / exp_avg_sq (ssac_mlp_backward_post_adam)."""
-        g = self.arena.grad.data_ptr()
-        offs = tuple((t.data_ptr() - g) // 4 for t in (self.arena.flat, self.m, self.v))
-        assert all((t.data_ptr() - g) % 16 == 0 for t in (self.arena.flat, self.m, self.v))
-        return offs
-
-    def note_fused_step(self):
-        """The step was applied by the kernels that produced the gradients (device counter advanced by them)."""
-        if not torch.cuda.is_current_stream_capturing():
             self.steps += 1
             self._step_tensor.fill_(self.steps)
 

@@ -29,7 +29,7 @@ class FlatParamAdam:
         self.optimizer, self.net = optimizer, net
         self.flat, self.grad = net._flat, net._flat_grad
         self.m, self.v = torch.zeros_like(self.flat), torch.zeros_like(self.flat)
-        self.ctl = torch.zeros(8, dtype=torch.int32, device=self.flat.device)
+        self.ctl = torch.zeros(2, dtype=torch.int32, device=self.flat.device)
         self.gnorm_sq = torch.zeros(1, dtype=torch.float32, device=self.flat.device)
         self.steps = 0
         self._step_tensor = torch.zeros((), dtype=torch.float32)

@@ -94,7 +94,7 @@ class _Lib:
         if os.environ.get("SSAC_NO_TMA"):
             self.cdll.ssac_set_tma_enabled(0)
         if os.environ.get("SSAC_CONV_HALO"):
-            self.cdll.ssac_set_conv_halo(int(os.environ["SSAC_CONV_HALO"]))
+            self.set_conv_halo(int(os.environ["SSAC_CONV_HALO"]))
         if os.environ.get("SSAC_NO_FUSED"):
             self.cdll.ssac_set_fused_forward(0)
 

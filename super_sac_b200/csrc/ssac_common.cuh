@@ -8,13 +8,6 @@
 
 #include "../../include/ssac_b200.h"
 
-// (library-internal, shared between translation units: Adam over one contiguous range; fuse_n > 0 = one of fuse_n kernels
-// that share the optimiser step, see AdamFuse)
-extern "C" int ssac_internal_adam_launch(int polyak, float* p, float* g, float* m, float* v, float* tgt, int64_t n,
-                                         int32_t* ctl, double lr, double b1, double b2, double eps, double wd,
-                                         const float* gnorm_sq, double max_norm, int wb, double tau, void* stream,
-                                         int fuse_slot, int fuse_n);
-
 namespace ssac {
 
 void set_error(const std::string& msg);
@@ -84,9 +77,9 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 struct AdamScalars {
   float step_size, bc2_sqrt, clip_coef;
 };
-// Every operation is spelled out (no compiler-chosen FMA contraction): the stand-alone kernel and the fused epilogues
-// must round identically.  The contractions are the ones torch's CUDA kernels compile to: lerp = fma(w, end - start,
-// start), addcmul = fma(value * t1, t2, self), addcdiv = fma(value, t1 / t2, self).
+// Every operation is spelled out (no compiler-chosen FMA contraction).  The contractions are the ones torch's CUDA
+// kernels compile to: lerp = fma(w, end - start, start), addcmul = fma(value * t1, t2, self),
+// addcdiv = fma(value, t1 / t2, self).
 __device__ __forceinline__ void adam1(float& p, float& g, float& m, float& v, const AdamScalars& sc, float one_m_b1,
                                       float b2, float one_m_b2, float eps, float wd, bool clip) {
   if (clip) g = __fmul_rn(g, sc.clip_coef);
@@ -96,56 +89,6 @@ __device__ __forceinline__ void adam1(float& p, float& g, float& m, float& v, co
   v = __fmaf_rn(__fmul_rn(one_m_b2, ge), ge, __fmul_rn(v, b2));               // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1-beta2)
   const float denom = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), sc.bc2_sqrt), eps);  // exp_avg_sq.sqrt() / bc2_sqrt + eps
   p = __fmaf_rn(-sc.step_size, __fdiv_rn(m, denom), p);                       // param.addcdiv_(exp_avg, denom, value=-step_size)
-}
-
-// Adam applied by the kernel that PRODUCES a gradient, to the element it has just reduced (ssac_mlp_backward_post_adam):
-// the parameter, exp_avg and exp_avg_sq of a gradient element live at the same offset of three twin arrays, so they are
-// addressed relative to the gradient's own address.  Same arithmetic, element by element, as adam_kernel.
-//   ctl = int32[8]: [0] step (shared with adam_kernel), [2 + slot] blocks of kernel `slot` that have finished,
-//   [4] kernels that have finished.  Every block derives its bias corrections from ctl[0] before anything else; the step
-//   advances when the LAST block of the LAST of the n_kernels participating kernels is done, i.e. after every block of
-//   every participant has read it.
-struct AdamFuse {
-  int64_t dp, dm, dv;   // in floats
-  int32_t* ctl;
-  int slot, n_kernels;
-  double lr, b1, b2;
-  float eps, wd;
-  int on;
-};
-struct AdamFuseConsts {
-  AdamScalars sc;
-  float one_m_b1, b2, one_m_b2;
-};
-__device__ __forceinline__ AdamFuseConsts adam_fuse_consts(const AdamFuse& a) {
-  AdamFuseConsts c;
-  const int t = a.ctl[0] + 1;
-  c.sc.step_size = (float)(a.lr / (1.0 - pow(a.b1, (double)t)));
-  c.sc.bc2_sqrt = (float)sqrt(1.0 - pow(a.b2, (double)t));
-  c.sc.clip_coef = 1.f;
-  c.one_m_b1 = (float)(1.0 - a.b1);
-  c.b2 = (float)a.b2;
-  c.one_m_b2 = (float)(1.0 - a.b2);
-  return c;
-}
-__device__ __forceinline__ void adam_fuse1(float* gaddr, float g, const AdamFuse& a, const AdamFuseConsts& c) {
-  float pv = gaddr[a.dp], mv = gaddr[a.dm], vv = gaddr[a.dv];
-  adam1(pv, g, mv, vv, c.sc, c.one_m_b1, c.b2, c.one_m_b2, a.eps, a.wd, false);
-  gaddr[a.dp] = pv; gaddr[a.dm] = mv; gaddr[a.dv] = vv;
-}
-// ONE thread of every block, after a __threadfence() by every writer and a block-wide barrier
-__device__ __forceinline__ void adam_fuse_block_done(const AdamFuse& a, int nblocks) {
-  const int prev = atomicAdd(&a.ctl[2 + a.slot], 1);
-  if (prev == nblocks - 1) {
-    a.ctl[2 + a.slot] = 0;
-    __threadfence();
-    const int k = atomicAdd(&a.ctl[4], 1);
-    if (k == a.n_kernels - 1) {
-      a.ctl[4] = 0;
-      a.ctl[0] = a.ctl[0] + 1;
-      __threadfence();
-    }
-  }
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

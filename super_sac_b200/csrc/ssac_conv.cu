@@ -689,309 +689,12 @@ __global__ void __launch_bounds__(kWgThreads, 1) conv_wgrad_halo_kernel(const __
   if (warp == 0) tmem_dealloc(tmem_d, 256);
 }
 
-// ---- first layer, direct: the im2col tile is built by CUDA cores straight from the NCHW observation ------------------
-// K = 9C patch elements in the weight's own order k = (c, kh, kw) (81 for a 9-channel frame stack -> three 32-deep
-// k-blocks), so the MMA count per tile is a third of the space-to-depth formulation's, no intermediate image exists and
-// the obs/255 - 0.5 normalisation happens on the way into shared memory.  Pixel p of the flat gh x gw grid reads
-// obs[b][c][2gy+kh][2gx+kw]; grid positions whose patch leaves the image (the last row / column: not outputs of the
-// layer) read zeros.
-struct DirectGeo {
-  const float* obs;
-  int C, H, W, gw, pp, k_real;   // k_real = 9C
-  int64_t np;
-};
-struct PixelAt {
-  const float* base;   // &obs[b][0][2gy][2gx]
-  int vy, vx;          // rows / columns of the image left from there (0 for pixels beyond the tensor)
-};
-__device__ __forceinline__ PixelAt pixel_at(const DirectGeo& g, int64_t p) {
-  PixelAt a;
-  a.base = g.obs;
-  a.vy = a.vx = 0;
-  if (p < g.np) {
-    const int b = (int)(p / g.pp), rem = (int)(p - (int64_t)b * g.pp), gy = rem / g.gw, gx = rem - gy * g.gw;
-    a.base = g.obs + ((int64_t)b * g.C * g.H + 2 * gy) * g.W + 2 * gx;
-    a.vy = g.H - 2 * gy;
-    a.vx = g.W - 2 * gx;
-  }
-  return a;
-}
-// patch elements k0 .. k0+3 of one pixel, normalised (nets/cnns.py:58: two separately rounded fp32 operations)
-__device__ __forceinline__ float4 patch4(const DirectGeo& g, const PixelAt& a, int k0) {
-  float v[4];
-#pragma unroll
-  for (int e = 0; e < 4; ++e) {
-    const int k = k0 + e, c = k / 9, t9 = k - 9 * c, kh = t9 / 3, kw = t9 - 3 * kh;
-    v[e] = 0.f;
-    if (k < g.k_real && kh < a.vy && kw < a.vx)
-      v[e] = __fsub_rn(__fdiv_rn(__ldg(a.base + ((int64_t)c * g.H + kh) * g.W + kw), 255.0f), 0.5f);
-  }
-  return make_float4(v[0], v[1], v[2], v[3]);
-}
-
-struct Conv1P {
-  ConvP c;          // bias, wpack, out + destination grid, ntiles, mode = 0, np (the epilogue's view); ntb = number of k-blocks, ksteps[]
-  DirectGeo g;
-};
-constexpr int kDirThreads = 416;   // warps 0-3 epilogue, 4-11 tile builders, 12 MMA issuer
-constexpr int kDirSmem = 5 * 8192 + kConvStages * kConvStageBytes + 1024;
-__global__ void __launch_bounds__(kDirThreads, 1) conv1_direct_kernel(const __grid_constant__ Conv1P q) {
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t bar_full[kConvStages], bar_empty[kConvStages], bar_accf[2], bar_acce[2];
-  __shared__ uint32_t tmem_base_sh;
-  __shared__ float bias_sh[32];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint8_t* wsm = smem;
-  uint8_t* stg = smem + 5 * 8192;
-  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  const int nkb = q.c.ntb;
-
-  if (warp == 0) tmem_alloc(&tmem_base_sh, 128);
-  if (t == 0) {
-    for (int s = 0; s < kConvStages; ++s) {
-      mbar_init(&bar_full[s], 256);
-      mbar_init(&bar_empty[s], 1);
-    }
-    for (int b = 0; b < 2; ++b) {
-      mbar_init(&bar_accf[b], 1);
-      mbar_init(&bar_acce[b], 128);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  pdl_wait();
-  pdl_trigger();
-  {
-    const float4* src = reinterpret_cast<const float4*>(q.c.wpack);
-    float4* dst = reinterpret_cast<float4*>(wsm);
-    for (int i = t; i < nkb * 512; i += kDirThreads) dst[i] = __ldg(src + i);
-  }
-  if (t < 32) bias_sh[t] = q.c.bias ? __ldg(q.c.bias + t) : 0.f;
-  fence_async_smem();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
-  const uint32_t tmem_d = tmem_base_sh;
-  const int ntl = ((int)blockIdx.x < q.c.ntiles) ? (q.c.ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-
-  if (warp == 12) {
-    const uint32_t idesc64 = instr_desc(64, 0, 0), idesc32 = instr_desc(32, 0, 0);
-    const uint64_t dah0 = smem_desc(smem_u32(stg), 16u, 1024u, 2u), db0 = smem_desc(smem_u32(wsm), 16u, 1024u, 2u);
-    int it = 0;
-    for (int i = 0; i < ntl; ++i) {
-      const int buf = i & 1;
-      const uint32_t d = tmem_d + (uint32_t)(buf * 64);
-      if (i >= 2) {
-        mbar_wait(&bar_acce[buf], (uint32_t)(((i >> 1) - 1) & 1));
-        fence_after_sync();
-      }
-      for (int kb = 0; kb < nkb; ++kb, ++it) {
-        const int s = it % kConvStages, use = it / kConvStages;
-        mbar_wait(&bar_full[s], (uint32_t)(use & 1));
-        fence_after_sync();
-        if (elect_one()) {
-          const uint64_t dah = dah0 + (uint64_t)(s * (kConvStageBytes >> 4)), dal = dah + (16384u >> 4);
-          const uint64_t db = db0 + (uint64_t)(kb * (8192 >> 4));
-          mma_tf32(d, dah, db, idesc64, kb != 0);
-          mma_tf32(d, dal, db, idesc32, 1u);
-          const int ks = q.c.ksteps[kb];
-#pragma unroll
-          for (int j = 1; j < 4; ++j) {
-            if (j < ks) {
-              mma_tf32(d, dah + 2 * j, db + 2 * j, idesc64, 1u);
-              mma_tf32(d, dal + 2 * j, db + 2 * j, idesc32, 1u);
-            }
-          }
-          mma_commit(&bar_empty[s]);
-          if (kb == nkb - 1) mma_commit(&bar_accf[buf]);
-        }
-        __syncwarp();
-      }
-    }
-  } else if (warp >= 4) {
-    // ===== builders: thread = (pixel row r, 16 consecutive k of the block) -> four 16-byte chunks of the swizzled row =====
-    const int tl = t - 128, r = tl & 127, half = tl >> 7;
-    const uint32_t r7 = (uint32_t)(r & 7);
-    const uint32_t rowoff = (uint32_t)(r >> 3) * 1024u + r7 * 128u;
-    int it = 0;
-    for (int i = 0; i < ntl; ++i) {
-      const int tile = (int)blockIdx.x + i * (int)gridDim.x;
-      const PixelAt a = pixel_at(q.g, (int64_t)tile * 128 + r);
-      for (int kb = 0; kb < nkb; ++kb, ++it) {
-        const int s = it % kConvStages, use = it / kConvStages;
-        float4 v[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) v[j] = patch4(q.g, a, kb * 32 + half * 16 + 4 * j);    // loads fly before the wait
-        if (it >= kConvStages) mbar_wait(&bar_empty[s], (uint32_t)((use - 1) & 1));
-        uint8_t* hi = stg + s * kConvStageBytes + rowoff;
-        uint8_t* lo = hi + 16384;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const uint32_t co = (((uint32_t)(half * 4 + j)) ^ r7) << 4;
-          *reinterpret_cast<float4*>(hi + co) = v[j];
-          *reinterpret_cast<float4*>(lo + co) = lo4(v[j]);
-        }
-        fence_async_smem();
-        mbar_arrive(&bar_full[s]);
-      }
-    }
-  } else {
-    conv_epilogue(q.c, tmem_d, bar_accf, bar_acce, bias_sh, ntl);
-  }
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem_d, 128);
-}
-
-// First-layer weight gradient, direct: gW1[co][k] = sum_p dZ1[p][co] * patch[p][k].  A = the patch tile of 32 pixels as an
-// MN-major operand (M = 128 patch elements = four 32-column groups, built by CUDA cores), B = [dZ_hi | dZ_lo] by TMA.
-struct Wgrad1P {
-  CUtensorMap tmD;   // (32, pixels), box 32 x 32, SWIZZLE_128B_ATOM_32B
-  DirectGeo g;
-  float* part;       // [grid][128 k][32 co]
-  float* bpart;      // [grid][32]
-  int nstages, spc;
-};
-constexpr int kW1Stages = 4;
-constexpr int kW1Stage = 2 * 16384 + 8192;
-__global__ void __launch_bounds__(kWgThreads, 1) conv1_wgrad_direct_kernel(const __grid_constant__ Wgrad1P q) {
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t bar_raw[kW1Stages], bar_full[kW1Stages], bar_empty[kW1Stages], bar_done;
-  __shared__ uint32_t tmem_base_sh;
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-
-  if (warp == 0) tmem_alloc(&tmem_base_sh, 64);
-  if (t == 0) {
-    for (int s = 0; s < kW1Stages; ++s) {
-      mbar_init(&bar_raw[s], 1);
-      mbar_init(&bar_full[s], 256);
-      mbar_init(&bar_empty[s], 1);
-    }
-    mbar_init(&bar_done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  pdl_wait();
-  pdl_trigger();
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
-  const uint32_t tmem_d = tmem_base_sh;
-  const int st0 = (int)blockIdx.x * q.spc;
-  const int nst = max(0, min(q.spc, q.nstages - st0));
-
-  if (warp == 9) {
-    if (lane == 0) {
-      for (int i = 0; i < nst; ++i) {
-        const int s = i % kW1Stages, use = i / kW1Stages;
-        if (i >= kW1Stages) mbar_wait(&bar_empty[s], (uint32_t)((use - 1) & 1));
-        mbar_arrive_expect_tx(&bar_raw[s], 4096u);
-        tma_load_2d(smem_u32(smem) + (uint32_t)(s * kW1Stage + 32768), &q.tmD, &bar_raw[s], 0, (st0 + i) * 32);
-      }
-    }
-  } else if (warp == 8) {
-    const uint32_t idesc64 = instr_desc(64, 1, 1), idesc32 = instr_desc(32, 1, 1);
-    const uint64_t da0 = smem_desc(smem_u32(smem), 4096u, 512u, 1u);
-    const uint64_t db0 = smem_desc(smem_u32(smem) + 32768u, 4096u, 512u, 1u);
-    for (int i = 0; i < nst; ++i) {
-      const int s = i % kW1Stages, use = i / kW1Stages;
-      mbar_wait(&bar_full[s], (uint32_t)(use & 1));
-      fence_after_sync();
-      if (elect_one()) {
-        const uint64_t so = (uint64_t)(s * (kW1Stage >> 4));
-        const uint64_t dah = da0 + so, dal = dah + (16384u >> 4), db = db0 + so;
-        mma_tf32(tmem_d, dah, db, idesc64, i != 0);
-        mma_tf32(tmem_d, dal, db, idesc32, 1u);
-#pragma unroll
-        for (int j = 1; j < 4; ++j) {
-          mma_tf32(tmem_d, dah + 64 * j, db + 64 * j, idesc64, 1u);
-          mma_tf32(tmem_d, dal + 64 * j, db + 64 * j, idesc32, 1u);
-        }
-        mma_commit(&bar_empty[s]);
-        if (i == nst - 1) mma_commit(&bar_done);
-      }
-      __syncwarp();
-    }
-  } else {
-    // ===== builders (thread = pixel k row kr, 16 consecutive patch elements) + lo plane / column sums of dZ =============
-    float cs[4] = {0.f, 0.f, 0.f, 0.f};
-    const int kr = t & 31, h = t >> 5;               // h = 0..7: patch elements 16h .. 16h+15
-    // MN-major: addr(m, k) = (m/32)*4096 + k*128 + ((((m%32)/8) ^ (k%4))*32) + (m%8)*4
-    const uint32_t goff = (uint32_t)(h >> 1) * 4096u + (uint32_t)kr * 128u;
-    const uint32_t c0 = (((uint32_t)(2 * (h & 1))) ^ (uint32_t)(kr & 3)) << 5, c1 = (((uint32_t)(2 * (h & 1) + 1)) ^ (uint32_t)(kr & 3)) << 5;
-    for (int i = 0; i < nst; ++i) {
-      const int s = i % kW1Stages, use = i / kW1Stages;
-      const PixelAt a = pixel_at(q.g, (int64_t)(st0 + i) * 32 + kr);
-      float4 v[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) v[j] = patch4(q.g, a, 16 * h + 4 * j);
-      if (i >= kW1Stages) mbar_wait(&bar_empty[s], (uint32_t)((use - 1) & 1));
-      uint8_t* a_hi = smem + s * kW1Stage;
-      uint8_t* a_lo = a_hi + 16384;
-      *reinterpret_cast<float4*>(a_hi + goff + c0) = v[0];      *reinterpret_cast<float4*>(a_lo + goff + c0) = lo4(v[0]);
-      *reinterpret_cast<float4*>(a_hi + goff + c0 + 16) = v[1]; *reinterpret_cast<float4*>(a_lo + goff + c0 + 16) = lo4(v[1]);
-      *reinterpret_cast<float4*>(a_hi + goff + c1) = v[2];      *reinterpret_cast<float4*>(a_lo + goff + c1) = lo4(v[2]);
-      *reinterpret_cast<float4*>(a_hi + goff + c1 + 16) = v[3]; *reinterpret_cast<float4*>(a_lo + goff + c1 + 16) = lo4(v[3]);
-      mbar_wait(&bar_raw[s], (uint32_t)(use & 1));
-      {
-        uint8_t* d_hi = a_hi + 32768;
-        const float4 d = *reinterpret_cast<const float4*>(d_hi + t * 16);
-        *reinterpret_cast<float4*>(d_hi + 4096 + t * 16) = lo4(d);
-        cs[0] += d.x; cs[1] += d.y; cs[2] += d.z; cs[3] += d.w;
-      }
-      fence_async_smem();
-      mbar_arrive(&bar_full[s]);
-    }
-    if (nst > 0) mbar_wait(&bar_done, 0);
-    fence_after_sync();
-    float* scr = reinterpret_cast<float*>(smem);
-    {
-      const int krow = t >> 3;
-      const int col = 8 * (((t >> 1) & 3) ^ (krow & 3)) + 4 * (t & 1);
-#pragma unroll
-      for (int e = 0; e < 4; ++e) scr[krow * 32 + col + e] = cs[e];
-    }
-    asm volatile("bar.sync 1, 256;" ::: "memory");
-    if (t < 32) {
-      float tot = 0.f;
-      for (int k = 0; k < 32; ++k) tot += scr[k * 32 + t];
-      q.bpart[(int64_t)blockIdx.x * 32 + t] = tot;
-    }
-    if (warp < 4) {
-      float4 o[8];
-      if (nst > 0) {
-        uint32_t r0[32], r1[32];
-        const uint32_t ta = tmem_d + ((uint32_t)(warp * 32) << 16);
-        tmem_ld32_issue(ta, r0);
-        tmem_ld32_issue(ta + 32u, r1);
-        tmem_wait_ld();
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {
-          o[c].x = __uint_as_float(r0[4 * c + 0]) + __uint_as_float(r1[4 * c + 0]);
-          o[c].y = __uint_as_float(r0[4 * c + 1]) + __uint_as_float(r1[4 * c + 1]);
-          o[c].z = __uint_as_float(r0[4 * c + 2]) + __uint_as_float(r1[4 * c + 2]);
-          o[c].w = __uint_as_float(r0[4 * c + 3]) + __uint_as_float(r1[4 * c + 3]);
-        }
-      } else {
-#pragma unroll
-        for (int c = 0; c < 8; ++c) o[c] = make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-      float4* dst = reinterpret_cast<float4*>(q.part + ((int64_t)blockIdx.x * 128 + warp * 32 + lane) * 32);
-#pragma unroll
-      for (int c = 0; c < 8; ++c) dst[c] = o[c];
-    }
-  }
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc(tmem_d, 64);
-}
-
 // ---- small kernels -----------------------------------------------------------------------------------------------
 // Shared-memory images of the per-tap weight matrices: rows n = 0..31 hold B[n][k] as the tensor core sees it, rows
 // 32..63 the lo parts; K-major SWIZZLE_128B.
 //   mode 0 (forward 3x3, 32 in):  tb = kh*3+kw,           B[n=co][k=ci] = W[co][ci][kh][kw]
 //   mode 1 (data gradient):       tb = kh*3+kw,           B[n=ci][k=co] = W[co][ci][kh][kw]
 //   mode 2 (first layer, s2d):    tb = (dh*2+dw)*2 + cb,  B[n=co][k] = W[co][c][2dh+ph][2dw+pw], s2d channel cb*32+k = (ph*2+pw)*C + c
-//   mode 3 (first layer, direct): tb = k-block,           B[n=co][k] = W[co][tb*32+k] (flat (c,kh,kw) index, zero beyond 9C)
 __global__ void conv_pack_kernel(const float* __restrict__ W, float* __restrict__ pack, int mode, int C, int ntb) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= ntb * 2048) return;
@@ -1001,9 +704,6 @@ __global__ void conv_pack_kernel(const float* __restrict__ W, float* __restrict_
     w = W[(nn * 32 + k) * 9 + tb];
   } else if (mode == 1) {
     w = W[(k * 32 + nn) * 9 + tb];
-  } else if (mode == 3) {   // first layer, direct: tb = k-block, B[n=co][k] = W[co][tb*32 + k] in the weight's own (c, kh, kw) order
-    const int kg = tb * 32 + k;
-    if (kg < 9 * C) w = W[nn * 9 * C + kg];
   } else {
     const int cb = tb & 1, tap = tb >> 1, dh = tap >> 1, dw = tap & 1, sc = cb * 32 + k;
     if (sc < 4 * C) {
@@ -1088,11 +788,7 @@ __global__ void wgrad_reduce_kernel(const float* __restrict__ part, const float*
   const int per = (nparts + 3) / 4, p0 = sl * per, p1 = min(nparts, p0 + per);
   float tot = 0.f;
   int out = -1;
-  if (idx < nW && mode == 3) {   // direct first layer: part[p][k][co] with k the flat (c,kh,kw) index
-    const int co = idx & 31, k = idx >> 5;
-    for (int p = p0; p < p1; ++p) tot += part[((int64_t)p * 128 + k) * 32 + co];
-    out = co * 9 * C + k;
-  } else if (idx < nW) {
+  if (idx < nW) {
     int co, tb, k;
     if (mode == 0) {
       co = idx & 31; k = (idx >> 5) & 31; tb = idx >> 10;   // k = ci
@@ -1232,7 +928,7 @@ __global__ void fc_colred_kernel(const float* __restrict__ dl, const float* __re
 // ---- host ----------------------------------------------------------------------------------------------------------
 namespace {
 
-// bit 0: halo tiles in the forward / data-gradient kernel, bit 1: in the weight-gradient kernel, bit 2: direct first layer
+// bit 0: halo tiles in the forward / data-gradient kernel, bit 1: in the weight-gradient kernel
 int g_conv_halo = 3;
 
 struct EncPlan {
@@ -1244,7 +940,7 @@ struct EncPlan {
   int64_t npl[5];
   int vh[5], vw[5];
   int64_t kf, kfp;
-  int ks, nsplit, direct;
+  int ks, nsplit;
   int64_t x0, y[5], d[5], wfc, gwfc, part_fc, xhat, rstd, dfc, dl, pack_f[5], pack_d[5], wpart, bpart, total;
 };
 
@@ -1273,8 +969,7 @@ int make_plan(int B, int C, int H, int W, int O, int save, EncPlan* p) {
   const int64_t pad = p->ks + 256;     // zero tail behind every activation buffer (the last split-K group reads past kf)
   int64_t o = 0;
   auto take = [&](int64_t n) { const int64_t at = o; o += up256(n); return at; };
-  p->direct = (g_conv_halo & 4) && 9 * C <= 128;     // first layer straight from the NCHW observation: no s2d image
-  p->x0 = p->direct ? -1 : take(p->npl[1] * 64 + pad);
+  p->x0 = take(p->npl[1] * 64 + pad);
   // y[l]: output of layer l -- compacted onto layer l+1's grid (l = 1..3), on layer 4's own grid for l = 4
   const int64_t ysz[5] = {0, p->npl[2] * 32 + pad, p->npl[3] * 32 + pad, p->npl[4] * 32 + pad, p->npl[4] * 32 + pad};
   p->d[0] = -1;
@@ -1305,8 +1000,6 @@ bool g_conv_attr = false;
 int conv_attrs() {
   if (g_conv_attr) return 0;
   cudaError_t e = cudaFuncSetAttribute(cv::conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cv::kConvSmem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(cv::conv1_direct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cv::kDirSmem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(cv::conv1_wgrad_direct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cv::kW1Stages * cv::kW1Stage + 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(cv::conv_wgrad_halo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 231424);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(cv::conv_halo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 231424);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(cv::conv_wgrad_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * (6 * 16384 + 8192) + 1024);
@@ -1429,45 +1122,6 @@ int launch_wgrad(const EncPlan& pl, int layer, const float* x, int x_ch, const f
   return 0;
 }
 
-cv::DirectGeo direct_geo(const EncPlan& pl, const float* obs) {
-  cv::DirectGeo g;
-  g.obs = obs; g.C = pl.C; g.H = pl.H; g.W = pl.W; g.gw = pl.gw; g.pp = pl.gh * pl.gw; g.k_real = 9 * pl.C; g.np = pl.npl[1];
-  return g;
-}
-
-int launch_conv1_direct(const EncPlan& pl, const float* obs, float* out, const float* wpack, const float* bias, cudaStream_t s) {
-  cv::Conv1P q;
-  memset(&q, 0, sizeof(q));
-  q.c.wpack = wpack; q.c.bias = bias; q.c.out = out;
-  q.c.pp = pl.gh * pl.gw; q.c.pw = pl.gw;
-  q.c.out_vh = pl.vh[1]; q.c.out_vw = pl.vw[1]; q.c.dst_pp = pl.vh[1] * pl.vw[1]; q.c.dst_pw = pl.vw[1];
-  q.c.ntb = (9 * pl.C + 31) / 32;
-  for (int kb = 0; kb < q.c.ntb; ++kb) q.c.ksteps[kb] = std::min(4, (9 * pl.C - 32 * kb + 7) / 8);
-  q.c.ntiles = (int)((pl.npl[1] + 127) / 128);
-  q.c.mode = 0;
-  q.c.np = pl.npl[1];
-  q.g = direct_geo(pl, obs);
-  cv::conv1_direct_kernel<<<std::min(q.c.ntiles, kNumSMs), cv::kDirThreads, cv::kDirSmem, s>>>(q);
-  SSAC_CHECK_LAUNCH("conv1_direct_kernel");
-  return 0;
-}
-
-int launch_wgrad1_direct(const EncPlan& pl, const float* obs, const float* dz, float* ws, float* gW, float* gb, cudaStream_t s) {
-  cv::Wgrad1P q;
-  memset(&q, 0, sizeof(q));
-  if (!tc::make_map2d(dz, 32, 32, pl.npl[1], 32, true, &q.tmD)) return fail(SSAC_E_UNSUPPORTED, "conv encoder: tensor map");
-  q.g = direct_geo(pl, obs);
-  q.part = ws + pl.wpart; q.bpart = ws + pl.bpart;
-  q.nstages = (int)((pl.npl[1] + 31) / 32);
-  const int grid = std::min(q.nstages, kNumSMs);
-  q.spc = (q.nstages + grid - 1) / grid;
-  cv::conv1_wgrad_direct_kernel<<<grid, cv::kWgThreads, cv::kW1Stages * cv::kW1Stage + 1024, s>>>(q);
-  SSAC_CHECK_LAUNCH("conv1_wgrad_direct_kernel");
-  cv::wgrad_reduce_kernel<<<(9 * 32 * pl.C + 32 + 63) / 64, 256, 0, s>>>(q.part, q.bpart, grid, 3, pl.C, gW, gb);
-  SSAC_CHECK_LAUNCH("wgrad_reduce_kernel");
-  return 0;
-}
-
 GemmP zero_gemm() {
   GemmP g;
   memset(&g, 0, sizeof(g));
@@ -1480,6 +1134,7 @@ GemmP zero_gemm() {
 using namespace ssac;
 
 extern "C" int ssac_set_conv_halo(int mode) {
+  SSAC_REQUIRE(mode >= 0 && mode <= 3, "ssac_set_conv_halo: mode must be 0..3");
   g_conv_halo = mode;
   return 0;
 }
@@ -1511,16 +1166,11 @@ extern "C" int ssac_conv_encoder_forward(const float* obs_dev, int B, int C, int
   SSAC_REQUIRE(obs_dev && params && ws_dev && out_dev, "conv encoder: null pointer");
   cudaStream_t s = (cudaStream_t)stream;
   float* ws = ws_dev;
-  if (!pl.direct) {
-    int rp = std::max(1, std::min(pl.gh, (int)(40960 / ((size_t)pl.gw * 4 * C * sizeof(float)))));   // <= 40 KB of smem
-    while (pl.gh % rp) --rp;
-    cv::s2d_norm_kernel<<<B * (pl.gh / rp), 512, (size_t)rp * pl.gw * 4 * C * sizeof(float), s>>>(obs_dev, ws + pl.x0, C, H, W, rp);
-    SSAC_CHECK_LAUNCH("s2d_norm_kernel");
-    cv::conv_pack_kernel<<<(8 * 2048 + 255) / 256, 256, 0, s>>>(params[0], ws + pl.pack_f[1], 2, C, 8);
-  } else {
-    const int nkb = (9 * C + 31) / 32;
-    cv::conv_pack_kernel<<<(nkb * 2048 + 255) / 256, 256, 0, s>>>(params[0], ws + pl.pack_f[1], 3, C, nkb);
-  }
+  int rp = std::max(1, std::min(pl.gh, (int)(40960 / ((size_t)pl.gw * 4 * C * sizeof(float)))));   // <= 40 KB of smem
+  while (pl.gh % rp) --rp;
+  cv::s2d_norm_kernel<<<B * (pl.gh / rp), 512, (size_t)rp * pl.gw * 4 * C * sizeof(float), s>>>(obs_dev, ws + pl.x0, C, H, W, rp);
+  SSAC_CHECK_LAUNCH("s2d_norm_kernel");
+  cv::conv_pack_kernel<<<(8 * 2048 + 255) / 256, 256, 0, s>>>(params[0], ws + pl.pack_f[1], 2, C, 8);
   SSAC_CHECK_LAUNCH("conv_pack_kernel");
   for (int l = 2; l <= 4; ++l) {
     cv::conv_pack_kernel<<<(9 * 2048 + 255) / 256, 256, 0, s>>>(params[2 * (l - 1)], ws + pl.pack_f[l], 0, C, 9);
@@ -1530,11 +1180,7 @@ extern "C" int ssac_conv_encoder_forward(const float* obs_dev, int B, int C, int
     cv::fc_pack_kernel<<<out_dim * pl.vh[4], 256, (size_t)32 * (pl.vw[4] + 1) * sizeof(float), s>>>(params[8], ws + pl.wfc, out_dim, pl.vh[4], pl.vw[4], pl.P[4], pl.kfp, 0);
     SSAC_CHECK_LAUNCH("fc_pack_kernel");
   }
-  if (pl.direct) {
-    if (int rc = launch_conv1_direct(pl, obs_dev, ws + pl.y[1], ws + pl.pack_f[1], params[1], s)) return rc;
-  } else {
-    if (int rc = launch_conv(pl, 1, false, ws + pl.x0, 64, ws + pl.y[1], ws + pl.pack_f[1], params[1], nullptr, s)) return rc;
-  }
+  if (int rc = launch_conv(pl, 1, false, ws + pl.x0, 64, ws + pl.y[1], ws + pl.pack_f[1], params[1], nullptr, s)) return rc;
   for (int l = 2; l <= 4; ++l)
     if (int rc = launch_conv(pl, l, false, ws + pl.y[l - 1], 32, ws + pl.y[l], ws + pl.pack_f[l], params[2 * (l - 1) + 1], nullptr, s)) return rc;
   // FC: split-K as groups of the grouped GEMM
@@ -1590,6 +1236,5 @@ extern "C" int ssac_conv_encoder_backward(const float* dout_dev, const float* ou
     SSAC_CHECK_LAUNCH("conv_pack_kernel");
     if (int rc = launch_conv(pl, l, true, ws + pl.d[l], 32, ws + pl.d[l - 1], ws + pl.pack_d[l], nullptr, ws + pl.y[l - 1], s)) return rc;
   }
-  if (pl.direct) return launch_wgrad1_direct(pl, obs_dev, ws + pl.d[1], ws, grads[0], grads[1], s);
   return launch_wgrad(pl, 1, ws + pl.x0, 64, ws + pl.d[1], ws, grads[0], grads[1], s);
 }

@@ -88,7 +88,7 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, float*
                                                    float* __restrict__ v, float* __restrict__ tgt, int64_t n,
                                                    int32_t* __restrict__ ctl, double lr, double b1d, double b2d, float eps,
                                                    float wd, const float* __restrict__ gnorm_sq, float max_norm,
-                                                   int write_back, float c1, float c2, int fuse_slot, int fuse_n) {
+                                                   int write_back, float c1, float c2) {
   __shared__ AdamScalars sc;
   if (threadIdx.x == 0) {
     // the step counter is only ever written by this optimiser's own previous launch: the (double-precision) bias
@@ -158,18 +158,11 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, float*
   __threadfence();
   __syncthreads();
   if (threadIdx.x == 0) {
-    if (fuse_n > 0) {
-      // one of several kernels that share this step (ssac_mlp_backward_post_adam): the last of them advances it
-      AdamFuse a;
-      a.ctl = ctl; a.slot = fuse_slot; a.n_kernels = fuse_n;
-      adam_fuse_block_done(a, (int)gridDim.x);
-    } else {
-      const int prev = atomicAdd(&ctl[1], 1);
-      if (prev == (int)gridDim.x - 1) {
-        ctl[0] = ctl[0] + 1;
-        ctl[1] = 0;
-        __threadfence();
-      }
+    const int prev = atomicAdd(&ctl[1], 1);
+    if (prev == (int)gridDim.x - 1) {
+      ctl[0] = ctl[0] + 1;
+      ctl[1] = 0;
+      __threadfence();
     }
   }
 }
@@ -665,9 +658,9 @@ int ssac_polyak_multi(const uint64_t* table_dev, int n_tensors, int64_t max_nume
   return 0;
 }
 
-int ssac_internal_adam_launch(int polyak, float* p, float* g, float* m, float* v, float* tgt, int64_t n, int32_t* ctl,
-                double lr, double b1, double b2, double eps, double wd, const float* gnorm_sq, double max_norm,
-                int wb, double tau, void* stream, int fuse_slot, int fuse_n) {
+static int adam_launch(int polyak, float* p, float* g, float* m, float* v, float* tgt, int64_t n, int32_t* ctl,
+                       double lr, double b1, double b2, double eps, double wd, const float* gnorm_sq, double max_norm,
+                       int wb, double tau, void* stream) {
   if (n <= 0) return 0;
   SSAC_REQUIRE(p && g && m && v && ctl, "ssac_adam_step: null pointer");
   const int grid = grid_for((n + 3) / 4, 256, 8);
@@ -675,10 +668,10 @@ int ssac_internal_adam_launch(int polyak, float* p, float* g, float* m, float* v
   if (polyak) {
     SSAC_REQUIRE(tgt, "ssac_adam_polyak_step: null target");
     launch_pdl(adam_kernel<true>, dim3(grid), dim3(256), 0, (cudaStream_t)stream, p, g, m, v, tgt, n, ctl, lr, b1, b2, (float)eps,
-               (float)wd, gnorm_sq, (float)max_norm, wb, c1, c2, fuse_slot, fuse_n);
+               (float)wd, gnorm_sq, (float)max_norm, wb, c1, c2);
   } else {
     launch_pdl(adam_kernel<false>, dim3(grid), dim3(256), 0, (cudaStream_t)stream, p, g, m, v, (float*)nullptr, n, ctl, lr, b1, b2,
-               (float)eps, (float)wd, gnorm_sq, (float)max_norm, wb, 0.f, 0.f, fuse_slot, fuse_n);
+               (float)eps, (float)wd, gnorm_sq, (float)max_norm, wb, 0.f, 0.f);
   }
   SSAC_CHECK_LAUNCH("ssac_adam_step");
   return 0;
@@ -687,15 +680,15 @@ int ssac_internal_adam_launch(int polyak, float* p, float* g, float* m, float* v
 int ssac_adam_step(float* p, float* g, float* m, float* v, int64_t n, int32_t* ctl, double lr, double beta1,
                    double beta2, double eps, double weight_decay, const float* gnorm_sq_dev, double max_norm,
                    int write_back_grad, void* stream) {
-  return ssac_internal_adam_launch(0, p, g, m, v, nullptr, n, ctl, lr, beta1, beta2, eps, weight_decay, gnorm_sq_dev, max_norm,
-                     write_back_grad, 0.0, stream, 0, 0);
+  return adam_launch(0, p, g, m, v, nullptr, n, ctl, lr, beta1, beta2, eps, weight_decay, gnorm_sq_dev, max_norm,
+                     write_back_grad, 0.0, stream);
 }
 
 int ssac_adam_polyak_step(float* p, float* g, float* m, float* v, float* target, int64_t n, int32_t* ctl, double lr,
                           double beta1, double beta2, double eps, double weight_decay, const float* gnorm_sq_dev,
                           double max_norm, int write_back_grad, double tau, void* stream) {
-  return ssac_internal_adam_launch(1, p, g, m, v, target, n, ctl, lr, beta1, beta2, eps, weight_decay, gnorm_sq_dev, max_norm,
-                     write_back_grad, tau, stream, 0, 0);
+  return adam_launch(1, p, g, m, v, target, n, ctl, lr, beta1, beta2, eps, weight_decay, gnorm_sq_dev, max_norm,
+                     write_back_grad, tau, stream);
 }
 
 // x[i] *= *scale_dev: a factor that lives in device memory (the annealed TD3 noise scale), so that a captured graph

@@ -17,7 +17,7 @@ int mlp_backward_pre(const float* W2, const float* W3, int G, int H, int B, cons
                      cudaStream_t s, int impl);
 int mlp_backward_post(const float* W3, int G, int D, int H, const float* x, int64_t ldx, int64_t x_gs, int B, const float* h1,
                       const float* h2, const float* dq, float* ws, float* gW1, float* gb1, float* gW2, float* gb2,
-                      float* gW3, float* gb3, cudaStream_t s, int impl, const AdamFuse* adam = nullptr);
+                      float* gW3, float* gb3, cudaStream_t s, int impl);
 int mlp_backward_dact(const float* W1, const float* W2, const float* W3, int G, int D, int H, int col0, int A, int B,
                       const float* h1, const float* h2, const float* dq, float* da, float* ws, cudaStream_t s, int impl);
 void set_overlap(int on);
@@ -146,26 +146,6 @@ int ssac_mlp_backward_post(const float* W3, int G, int D, int H, const float* x_
   if (impl != 2) return fail(SSAC_E_UNSUPPORTED, "ssac_mlp_backward_post: the split backward exists for impl 2 (tcgen05) only");
   return mlp_backward_post(W3, G, D, H, x_dev, ldx, x_gs, B, h1_dev, h2_dev, dq_dev, ws_dev, gW1, gb1, gW2, gb2, gW3, gb3,
                            (cudaStream_t)stream, impl);
-}
-
-int ssac_mlp_backward_post_adam(const float* W3, int G, int D, int H, const float* x_dev, int64_t ldx, int64_t x_gs, int B,
-                                const float* h1_dev, const float* h2_dev, const float* dq_dev, float* ws_dev, float* gW1,
-                                float* gb1, float* gW2, float* gb2, float* gW3, float* gb3, int64_t param_off,
-                                int64_t exp_avg_off, int64_t exp_avg_sq_off, int32_t* ctl_dev, double lr, double beta1,
-                                double beta2, double eps, double weight_decay, int impl, void* stream) {
-  SSAC_REQUIRE(W3 && x_dev && h1_dev && h2_dev && dq_dev && ws_dev && gW1 && gb1 && gW2 && gb2 && gW3 && gb3 && ctl_dev,
-               "ssac_mlp_backward_post_adam: null pointer");
-  SSAC_REQUIRE(G > 0 && D > 0 && H > 0 && B > 0 && ldx >= D, "ssac_mlp_backward_post_adam: bad sizes");
-  SSAC_REQUIRE((param_off & 3) == 0 && (exp_avg_off & 3) == 0 && (exp_avg_sq_off & 3) == 0,
-               "ssac_mlp_backward_post_adam: the twin arrays must keep the gradient's 16-byte alignment");
-  if (impl == 0) impl = ssac_default_mlp_impl();
-  if (impl != 2) return fail(SSAC_E_UNSUPPORTED, "ssac_mlp_backward_post_adam: the split backward exists for impl 2 (tcgen05) only");
-  AdamFuse a;
-  memset(&a, 0, sizeof(a));
-  a.dp = param_off; a.dm = exp_avg_off; a.dv = exp_avg_sq_off; a.ctl = ctl_dev;
-  a.lr = lr; a.b1 = beta1; a.b2 = beta2; a.eps = (float)eps; a.wd = (float)weight_decay;
-  return mlp_backward_post(W3, G, D, H, x_dev, ldx, x_gs, B, h1_dev, h2_dev, dq_dev, ws_dev, gW1, gb1, gW2, gb2, gW3, gb3,
-                           (cudaStream_t)stream, impl, &a);
 }
 
 int ssac_mlp_backward_dact(const float* W1, const float* W2, const float* W3, int G, int D, int H, int col0, int A, int B,

@@ -1,23 +1,23 @@
-// Row-local MLP chains on the CUDA cores, exact fp32: the latency-bound single-net forwards of the update step.
+// Row-local MLP forwards on the CUDA cores, exact fp32, for small batches whose activations are not kept.
 //
-// The TD-target path of one member -- a1, logp = pi(s1), then the M target critics of the REDQ subset on (s1, a1)
-// (learning_utils.py:314-338, agent.py:22-40) -- is 0.11 GFLOP on B = 256 rows: as two tensor-core launches its grids are
-// 8 and 16 CTAs and each launch pays ~15 us of serial latency (TMEM allocation, a K = 256 pipeline of eight chunks,
-// epilogue).  Every step of that chain is ROW-LOCAL, so here ONE launch of ceil(B/16) clusters x 4 CTAs (64 CTAs for
-// B = 256) walks the whole chain for 16 batch rows per cluster:
+// Their purpose is the acting path (Agent.forward / sample_action at B = num_envs: agent.py:204-327): one actor and its
+// policy head (ssac_policy_rows).  As a tensor-core launch that forward runs on a grid of a few CTAs and pays ~15 us of
+// serial latency (TMEM allocation, a K = 256 pipeline of eight chunks, epilogue).  Every step of it is ROW-LOCAL, so here
+// ONE launch of ceil(B/16) clusters x 4 CTAs walks the whole network for 16 batch rows per cluster.  The same kernel also
+// runs G nets one after another on a shared batch (impl 3 of ssac_mlp_forward):
 //
 //   per net  : CTA r of the cluster owns hidden units [r*H/4, (r+1)*H/4) of both hidden layers
 //     layer 1: K = D <= 64, weights slice staged in shared memory, thread = (unit, row group)
-//              -> the 8 x H/4 activations are broadcast into all four CTAs' shared memory (DSMEM, 16-byte stores)
+//              -> the 16 x H/4 activations are broadcast into all four CTAs' shared memory (DSMEM, 16-byte stores)
 //     layer 2: thread = (unit pair, k split): its 2 x 32 weights come straight from L2 into registers (sixteen 16-byte
-//              loads in flight per thread, each weight is used for all 8 rows), activations are warp-broadcast 16-byte
-//              shared-memory reads: 64 FMAs per 8 reads; k-split partials are summed in a fixed order (bit-reproducible)
+//              loads in flight per thread, each weight is used for 8 rows at a time), activations are warp-broadcast
+//              16-byte shared-memory reads: 64 FMAs per 8 reads; k-split partials are summed in a fixed order
+//              (bit-reproducible)
 //     layer 3: O <= 16 outputs from the CTA's own units, partial sums exchanged over DSMEM, every CTA sums the four
 //              partials in rank order (identical results in all four)
-//   head     : tanh-Normal sample + log-prob / deterministic head + TD3 noise, written into the next net's input row
+//   head     : (actor) tanh-Normal sample + log-prob / deterministic head + TD3 noise
 //
-// The same kernel serves the acting path (Agent.forward / sample_action at B = num_envs: agent.py:204-327) and any
-// forward that does not keep activations.  sm_100a (thread-block clusters, DSMEM, PDL).
+// sm_100a (thread-block clusters, DSMEM, PDL).
 #include <cstring>
 
 #include "ssac_mlp.cuh"
@@ -25,8 +25,7 @@
 namespace ssac {
 namespace rows {
 
-constexpr int R = 16;       // batch rows per cluster (B = 256: 16 clusters x 4 = 64 CTAs, the other SMs stay free for the
-                            // online critics' tensor-core launches that run next to this kernel)
+constexpr int R = 16;       // batch rows per cluster
 constexpr int CS = 4;       // CTAs per cluster = slices of the hidden layers
 constexpr int T = 256;      // threads per CTA
 constexpr int kMaxH = 256, kMaxO = 16, kMaxD = 64;
@@ -38,22 +37,14 @@ struct Net {
 };
 
 struct Args {
-  Net actor; int has_actor, det, A, S;
+  Net actor; int has_actor, det, A;
   const float *eps, *noise; float sigma, clip, lo, hi;
   float *logp, *tanh_out, *actor_out;   // nullable outputs: log-prob [B], tanh(out) [B,A] (det), raw head input [B,O]
-  float* a_out; int64_t lda;            // sampled action [B,A] (row stride lda), e.g. the action columns of x
+  float* a_out; int64_t lda;            // sampled action [B,A] (row stride lda)
   Net critic; const int32_t* net_index; int M;
   float* y;                             // [M,B,O] critic outputs
   const float* x; int64_t ldx; int B, H;
 };
-
-#ifdef SSAC_TRACE
-__device__ long long* g_trace_rows = nullptr;
-__device__ int g_trace_slot = 0;
-#define RT(slot) do { if (g_trace_rows && blockIdx.x == 0 && threadIdx.x == 0) g_trace_rows[slot] = clock64(); } while (0)
-#else
-#define RT(slot) do {} while (0)
-#endif
 
 #define SSAC_LOG2F 0.6931471805599453f
 #define SSAC_LOG_SQRT_2PIF 0.9189385332046727f
@@ -87,7 +78,7 @@ struct Ops {                        // the small operands of one net, this CTA's
 };
 
 struct Smem {
-  float xs[R][kXP];                 // input rows of the current net: [s | a]
+  float xs[R][kXP];                 // input rows
   float hfull[R][kMaxH];            // layer-1 activations of all units (every CTA's slice, via DSMEM)
   float hloc[R][kMaxH / CS + 4];    // this CTA's layer-1 slice (before the broadcast) / layer-2 slice
   float red[2 * R * T];             // layer-2 k-split partials: [j][r][ks][pair]
@@ -169,8 +160,7 @@ __device__ __forceinline__ void load_ops(Ops& op, const Net& n, int g, const Geo
 // ``op`` hold this net's layer-2 weights / small operands (visible: a barrier separates the load from this call); on exit
 // they hold those of (next, next_g) when ``next`` is given, loaded behind this net's layer-2 arithmetic.
 __device__ void run_net(Smem& sm, int buf, float4 (&w)[2][8], const Net& n, const Net* next, int next_g, const Geo& G, int rank,
-                        int t, int tb = 0) {
-  RT(tb + 0);
+                        int t) {
   const int D = n.D, O = n.O, HC = G.HC, NP = G.NP, KS = G.KS;
   const Ops& op = sm.ops[buf];
   // ---- layer 1: thread = (unit c, row group of R / (T / HC) rows); one weight read feeds all rows of the group ------
@@ -196,7 +186,6 @@ __device__ void run_net(Smem& sm, int buf, float4 (&w)[2][8], const Net& n, cons
     }
   }
   __syncthreads();
-  RT(tb + 2);
   // broadcast the slice into every CTA's hfull (16-byte remote stores when the slice is a multiple of 4 units wide)
   if ((HC & 3) == 0) {
     const int q = HC / 4;
@@ -213,9 +202,7 @@ __device__ void run_net(Smem& sm, int buf, float4 (&w)[2][8], const Net& n, cons
       for (int d = 0; d < CS; ++d) st_remote_f1(&sm.hfull[r][G.n_lo + c], (uint32_t)d, sm.hloc[r][c]);
     }
   }
-  RT(tb + 3);
   cluster_sync_all();
-  RT(tb + 4);
   // ---- layer 2: thread = (unit pair, k split) ----------------------------------------------------------------------
   if (G.l2_active) {
 #pragma unroll
@@ -243,7 +230,6 @@ __device__ void run_net(Smem& sm, int buf, float4 (&w)[2][8], const Net& n, cons
     }
   }
   __syncthreads();
-  RT(tb + 5);
   // the registers are free again: the next net's layer-2 weights fly behind the rest of this net
   if (next) load_w2(w, *next, next_g, G);
   for (int o = t; o < R * HC; o += T) {
@@ -256,7 +242,6 @@ __device__ void run_net(Smem& sm, int buf, float4 (&w)[2][8], const Net& n, cons
     sm.hloc[r][c] = fmaxf(s, 0.f);
   }
   __syncthreads();
-  RT(tb + 6);
   // ---- layer 3: partial outputs over this CTA's units (thread = output), exchanged over DSMEM ------------------------
   for (int o = t; o < R * O; o += T) {
     const int oo = o % O, r = o / O;
@@ -271,9 +256,7 @@ __device__ void run_net(Smem& sm, int buf, float4 (&w)[2][8], const Net& n, cons
 #pragma unroll
     for (int d = 0; d < CS; ++d) st_remote_f1(&sm.yp[rank][r][oo], (uint32_t)d, acc);
   }
-  RT(tb + 7);
   cluster_sync_all();
-  RT(tb + 8);
   for (int o = t; o < R * O; o += T) {
     const int oo = o % O, r = o / O;
     float s = op.b3s[oo];
@@ -283,7 +266,6 @@ __device__ void run_net(Smem& sm, int buf, float4 (&w)[2][8], const Net& n, cons
   }
   if (next) load_ops(sm.ops[buf ^ 1], *next, next_g, G, t);
   __syncthreads();
-  RT(tb + 9);
 }
 
 __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(T, 1) mlp_rows_kernel(const __grid_constant__ Args q) {
@@ -294,7 +276,6 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(T, 1) mlp_rows_kern
   const int m0 = ((int)blockIdx.x / CS) * R;
   const int B = q.B;
   const Geo G(q.H, rank, t);
-  RT(0);
   // parameters first (nobody upstream writes them: Adam / Polyak never trigger early), so that under PDL their latency
   // overlaps the tail of the previous kernel; the REDQ subset was drawn at least two launches ago
   float4 w[2][8];
@@ -305,20 +286,15 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(T, 1) mlp_rows_kern
   for (int i = t; i < R * kXP; i += T) (&sm.xs[0][0])[i] = 0.f;
   pdl_wait();      // the batch (x, eps, noise) is the previous kernels' business
   pdl_trigger();
-  RT(1);
   __syncthreads();
-  const int Dload = q.has_actor ? q.S : q.critic.D;
-  for (int i = t; i < R * Dload; i += T) {
-    const int r = i / Dload, k = i - r * Dload;
+  for (int i = t; i < R * first.D; i += T) {
+    const int r = i / first.D, k = i - r * first.D;
     if (m0 + r < B) sm.xs[r][k] = q.x[(int64_t)(m0 + r) * q.ldx + k];
   }
   __syncthreads();
 
-  int buf = 0;
   if (q.has_actor) {
-    const int g_next = q.M > 0 ? (q.net_index ? q.net_index[0] : 0) : 0;
-    run_net(sm, buf, w, q.actor, q.M > 0 ? &q.critic : nullptr, g_next, G, rank, t, 10);
-    buf ^= 1;
+    run_net(sm, 0, w, q.actor, nullptr, 0, G, rank, t);
     // ---- policy head: thread = row (all four CTAs compute it, rank 0 writes the global outputs) -----------------------
     if (t < R) {
       const int r = t, b = m0 + r;
@@ -340,7 +316,6 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(T, 1) mlp_rows_kern
           const float ladj = 2.f * (SSAC_LOG2F - xv - softplus_th(-2.f * xv));
           const float dxm = xv - mu;
           lp += (0.f - ladj) + (-(dxm * dxm) / (2.f * (sd * sd)) - logf(sd) - SSAC_LOG_SQRT_2PIF);
-          sm.xs[r][q.S + j] = av;
           if (wr && q.a_out) q.a_out[(int64_t)b * q.lda + j] = av;
         }
         if (wr && q.logp) q.logp[b] = lp;
@@ -358,27 +333,24 @@ __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(T, 1) mlp_rows_kern
             v2 = __fadd_rn(v2, nz);
             v2 = fminf(fmaxf(v2, __fadd_rn(-1.f, 1e-6f)), __fadd_rn(1.f, -1e-6f));
           }
-          sm.xs[r][q.S + j] = v2;
           if (wr && q.a_out) q.a_out[(int64_t)b * q.lda + j] = v2;
         }
       }
     }
-    __syncthreads();
-  }
-  for (int m = 0; m < q.M; ++m) {
-    const int g_next = m + 1 < q.M ? (q.net_index ? q.net_index[m + 1] : m + 1) : 0;
-    run_net(sm, buf, w, q.critic, m + 1 < q.M ? &q.critic : nullptr, g_next, G, rank, t, 20 + 10 * m);
-    buf ^= 1;
-    const int O = q.critic.O;
-    if (rank == 0)
-      for (int o = t; o < R * O; o += T) {
-        const int oo = o % O, r = o / O;
-        if (m0 + r < B) q.y[((int64_t)m * B + m0 + r) * O + oo] = sm.out[r][oo];
-      }
-    __syncthreads();
+  } else {
+    for (int m = 0; m < q.M; ++m) {
+      const int g_next = m + 1 < q.M ? (q.net_index ? q.net_index[m + 1] : m + 1) : 0;
+      run_net(sm, m & 1, w, q.critic, m + 1 < q.M ? &q.critic : nullptr, g_next, G, rank, t);
+      const int O = q.critic.O;
+      if (rank == 0)
+        for (int o = t; o < R * O; o += T) {
+          const int oo = o % O, r = o / O;
+          if (m0 + r < B) q.y[((int64_t)m * B + m0 + r) * O + oo] = sm.out[r][oo];
+        }
+      __syncthreads();
+    }
   }
   cluster_sync_all();   // nobody leaves while a neighbour may still write into its shared memory
-  RT(2);
 }
 
 static int launch(const Args& a, cudaStream_t s) {
@@ -420,10 +392,6 @@ using namespace ssac;
 
 extern "C" {
 
-#ifdef SSAC_TRACE
-int ssac_debug_set_trace_rows(long long* dev_ptr) { return (int)cudaMemcpyToSymbol(rows::g_trace_rows, &dev_ptr, sizeof(dev_ptr)); }
-#endif
-
 int ssac_policy_rows(const float* W1, const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
                      int D, int H, int A, int deterministic, const float* x_dev, int64_t ldx, int B, float* out_dev,
                      const float* eps_dev, const float* noise_dev, float sigma, float clip, float log_std_lo,
@@ -436,33 +404,10 @@ int ssac_policy_rows(const float* W1, const float* b1, const float* W2, const fl
   rows::Args a;
   memset(&a, 0, sizeof(a));
   a.actor = rows::Net{W1, b1, W2, b2, W3, b3, D, O};
-  a.has_actor = 1; a.det = deterministic; a.A = A; a.S = D;
+  a.has_actor = 1; a.det = deterministic; a.A = A;
   a.eps = eps_dev; a.noise = noise_dev; a.sigma = sigma; a.clip = clip; a.lo = log_std_lo; a.hi = log_std_hi;
   a.logp = logp_dev; a.tanh_out = tanh_out_dev; a.actor_out = out_dev; a.a_out = a_dev; a.lda = lda;
   a.M = 0; a.x = x_dev; a.ldx = ldx; a.B = B; a.H = H;
-  return rows::launch(a, (cudaStream_t)stream);
-}
-
-int ssac_target_chain(const float* aW1, const float* ab1, const float* aW2, const float* ab2, const float* aW3,
-                      const float* ab3, int S, int H, int A, int deterministic, const float* cW1, const float* cb1,
-                      const float* cW2, const float* cb2, const float* cW3, const float* cb3,
-                      const int32_t* net_index_dev, int M, float* x1_dev, int64_t ldx, int B, const float* eps_dev,
-                      const float* noise_dev, float sigma, float clip, float log_std_lo, float log_std_hi,
-                      float* logp_dev, float* qt_dev, void* stream) {
-  SSAC_REQUIRE(aW1 && ab1 && aW2 && ab2 && aW3 && ab3 && cW1 && cb1 && cW2 && cb2 && cW3 && cb3 && x1_dev && qt_dev,
-               "ssac_target_chain: null pointer");
-  SSAC_REQUIRE(S > 0 && A > 0 && A <= 8 && M > 0 && B > 0 && ldx >= S + A, "ssac_target_chain: bad sizes");
-  SSAC_REQUIRE(deterministic || (eps_dev && logp_dev), "ssac_target_chain: a stochastic actor needs eps and logp");
-  const int O = deterministic ? A : 2 * A;
-  if (!rows::shape_ok(S + A, H, O)) return fail(SSAC_E_UNSUPPORTED, "ssac_target_chain: shape outside the rows kernel");
-  rows::Args a;
-  memset(&a, 0, sizeof(a));
-  a.actor = rows::Net{aW1, ab1, aW2, ab2, aW3, ab3, S, O};
-  a.has_actor = 1; a.det = deterministic; a.A = A; a.S = S;
-  a.eps = eps_dev; a.noise = noise_dev; a.sigma = sigma; a.clip = clip; a.lo = log_std_lo; a.hi = log_std_hi;
-  a.logp = logp_dev; a.a_out = x1_dev + S; a.lda = ldx;
-  a.critic = rows::Net{cW1, cb1, cW2, cb2, cW3, cb3, S + A, 1};
-  a.net_index = net_index_dev; a.M = M; a.y = qt_dev; a.x = x1_dev; a.ldx = ldx; a.B = B; a.H = H;
   return rows::launch(a, (cudaStream_t)stream);
 }
 

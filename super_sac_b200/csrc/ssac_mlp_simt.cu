@@ -402,7 +402,7 @@ __global__ void __launch_bounds__(kWgThreads) first_layer_wgrad_kernel(const flo
                                                                       float* __restrict__ gW1, float* __restrict__ gb1,
                                                                       int accumulate, const float* __restrict__ row_scale,
                                                                       const float* __restrict__ h2, float* __restrict__ gW3,
-                                                                      float* __restrict__ gb3, const AdamFuse adam) {
+                                                                      float* __restrict__ gb3) {
   constexpr int kRows = 256;                    // batch rows staged per pass
   // h2 / gW3 / gb3 (optional, scalar-output critics with row_scale = dq): the output-layer weight gradients
   // gW3[g][h] = sum_b dq[b] h2[b][h], gb3[g] = sum_b dq[b] ride along (same rows, same lanes: one more load and FMA per row)
@@ -410,12 +410,8 @@ __global__ void __launch_bounds__(kWgThreads) first_layer_wgrad_kernel(const flo
   __shared__ __align__(16) float shbuf[kPartFloats > kXFloats ? kPartFloats : kXFloats];   // x rows, then the partials
   float (*xs)[DP] = reinterpret_cast<float (*)[DP]>(shbuf);
   float (*part)[32][DP + 3] = reinterpret_cast<float (*)[32][DP + 3]>(shbuf);
-  __shared__ AdamFuseConsts adam_sh;
-  // (the step counter is only written by this optimiser's own previous kernels: the double-precision bias corrections can
-  // be evaluated while the producer of the operands is still running)
-  if (adam.on && threadIdx.x == 0) adam_sh = adam_fuse_consts(adam);
   pdl_wait();
-  if (!adam.on) pdl_trigger();   // a kernel that writes parameters never triggers early: later kernels prefetch them
+  pdl_trigger();
   const int g = blockIdx.y, h0 = blockIdx.x * 32, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int h = h0 + lane;
   const float* dz = dz1 + (int64_t)g * B * H + (h < H ? h : 0);
@@ -506,28 +502,17 @@ __global__ void __launch_bounds__(kWgThreads) first_layer_wgrad_kernel(const flo
     float* out = d < DP ? gW1 + ((int64_t)g * H + h0 + hl) * D + d
                  : d == DP ? gb1 + (int64_t)g * H + h0 + hl
                  : d == DP + 1 ? gW3 + (int64_t)g * H + h0 + hl : gb3 + g;
-    const float val = accumulate ? *out + tot : tot;
-    *out = val;
-    if (adam.on) adam_fuse1(out, val, adam, adam_sh);
-  }
-  if (adam.on) {
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) adam_fuse_block_done(adam, (int)(gridDim.x * gridDim.y));
+    *out = accumulate ? *out + tot : tot;
   }
 }
 
 static int first_layer_wgrad(const float* dz1, const float* x, int64_t ldx, int64_t x_gs, int G, int B, int H, int D,
                              float* gW1, float* gb1, int accumulate, cudaStream_t s, const float* row_scale = nullptr,
-                             const float* h2 = nullptr, float* gW3 = nullptr, float* gb3 = nullptr,
-                             const AdamFuse* adam = nullptr) {
+                             const float* h2 = nullptr, float* gW3 = nullptr, float* gb3 = nullptr) {
   dim3 grid((H + 31) / 32, G);
-  AdamFuse af;
-  memset(&af, 0, sizeof(af));
-  if (adam) af = *adam;
 #define SSAC_FLW(DP)                                                                                                   \
   launch_pdl(first_layer_wgrad_kernel<DP>, grid, dim3(kWgThreads), 0, s, dz1, x, ldx, x_gs, B, H, D, gW1, gb1, accumulate, row_scale, \
-             h2, gW3, gb3, af)
+             h2, gW3, gb3)
   if (D <= 8) SSAC_FLW(8);
   else if (D <= 16) SSAC_FLW(16);
   else if (D <= 24) SSAC_FLW(24);
@@ -556,9 +541,7 @@ static int launch_gemm(int layout, const GemmP& p, int G, cudaStream_t s, const 
 static int g_overlap = 1;
 struct Side {
   cudaStream_t s = nullptr;
-  cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  int u_pending = 0;   // asynchronous mlp_backward_pre calls whose _post is still to come (ev[5] sits behind their u GEMM; on the
-                       // in-order second stream its latest record covers the earlier ones)
+  cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
 };
 static Side* side_of_current_device() {
   static Side sides[64];
@@ -817,17 +800,12 @@ int mlp_backward_pre(const float* W2, const float* W3, int G, int H, int B, cons
     p.A = v; p.a_gate = nullptr;
     rc = launch_gemm(L_NN, p, G, s, "mlp_backward_pre u");
   }
-  if (rc) return rc;
-  if (sd) {   // the last reader of W2 in this update: a fused optimiser step of _post waits for it
-    if (cudaEventRecord(sd->ev[5], s) != cudaSuccess) return fail((int)cudaErrorUnknown, "mlp_backward_pre: event record");
-    sd->u_pending++;
-  }
-  return 0;
+  return rc;
 }
 
 int mlp_backward_post(const float* W3, int G, int D, int H, const float* x, int64_t ldx, int64_t x_gs, int B, const float* h1,
                       const float* h2, const float* dq, float* ws, float* gW1, float* gb1, float* gW2, float* gb2,
-                      float* gW3, float* gb3, cudaStream_t s, int impl, const AdamFuse* adam) {
+                      float* gW3, float* gb3, cudaStream_t s, int impl) {
   g_impl = impl;
   SSAC_REQUIRE(D <= 32, "ssac_mlp_backward_post: first-layer width must be <= 32");
   float* v = ws;
@@ -838,10 +816,8 @@ int mlp_backward_post(const float* W3, int G, int D, int H, const float* x, int6
   if (sd && (rc = order_after(s, w, sd->ev[0]))) return rc;   // fork
   // the short reductions go to the side stream (behind the u GEMM of an asynchronous _pre); the gW2 GEMM stays on the
   // caller's stream, where its set-up overlaps the loss kernel (programmatic dependent launch)
-  if (!adam) {
-    rc = first_layer_wgrad(u, x, ldx, x_gs, G, B, H, D, gW1, gb1, 0, w, dq, h2, gW3, gb3);   // gW1, gb1, gW3, gb3
-    if (rc) return rc;
-  }
+  rc = first_layer_wgrad(u, x, ldx, x_gs, G, B, H, D, gW1, gb1, 0, w, dq, h2, gW3, gb3);   // gW1, gb1, gW3, gb3
+  if (rc) return rc;
   // gW2 = (dq .* v)^T h1 with v generated from h2 while the A tiles are staged
   GemmP q = blank();
   q.A = h2; q.lda = H; q.a_gs = (int64_t)B * H; q.a_gate = W3; q.a_gate_gs = H;
@@ -856,32 +832,6 @@ int mlp_backward_post(const float* W3, int G, int D, int H, const float* x, int6
     rc = launch_gemm(L_TN, q, G, s, "mlp_backward_post gW2");
   }
   if (rc) return rc;
-  // Fused optimiser step (ssac_mlp_backward_post_adam).  Who may write what, and when:
-  //   W1, b1, W3, b3  by the gW1 reduction itself, element by element as it produces their gradients -- once the gW2 GEMM,
-  //                   the last reader of W3 (its gate), is done: the second stream waits for it first;
-  //   W2, b2          by an Adam launch over that range behind the gW2 GEMM on the caller's stream -- once the u GEMM of an
-  //                   asynchronous _pre, the last reader of W2, is done.
-  // The two share the step counter (AdamFuse): it advances when both have finished.
-  AdamFuse a1;
-  if (adam) {
-    a1 = *adam; a1.slot = 0; a1.n_kernels = 2; a1.on = 1;
-    if (sd && (rc = order_after(s, w, sd->ev[1]))) return rc;
-  }
-  if (adam) {
-    rc = first_layer_wgrad(u, x, ldx, x_gs, G, B, H, D, gW1, gb1, 0, w, dq, h2, gW3, gb3, &a1);   // gW1, gb1, gW3, gb3 + Adam
-    if (rc) return rc;
-  }
-  if (sd && sd->u_pending > 0) {
-    if (adam && cudaStreamWaitEvent(s, sd->ev[5], 0) != cudaSuccess) return fail((int)cudaErrorUnknown, "mlp_backward_post: event wait");
-    sd->u_pending--;
-  }
-  if (adam) {
-    SSAC_REQUIRE(gb2 > gW2 && (gb2 - gW2) < (int64_t)G * H * H + 1024, "ssac_mlp_backward_post_adam: W2 / b2 gradients must be adjacent arrays of one arena");
-    const int64_t n = (gb2 - gW2) + (int64_t)G * H;
-    rc = ssac_internal_adam_launch(0, gW2 + adam->dp, gW2, gW2 + adam->dm, gW2 + adam->dv, nullptr, n, adam->ctl, adam->lr, adam->b1,
-                                   adam->b2, (double)adam->eps, (double)adam->wd, nullptr, 0.0, 0, 0.0, (void*)s, 1, 2);
-    if (rc) return rc;
-  }
   if (sd && (rc = order_after(w, s, sd->ev[3]))) return rc;   // join
   return 0;
 }

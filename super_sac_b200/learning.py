@@ -16,10 +16,6 @@ from . import _arena, _encoder_opt, _lib, _logs, _ops, _rng, discrete as _discre
 from . import learning_utils as lu
 
 
-# Adam folded into the branches of the split backward (ssac_mlp_backward_post_adam): correct and tested, but MEASURED slower
-# inside the pipelined REDQ block (55.6 vs 49.4 us per update on B200): the gW1 reduction then has to wait for the gW2
-# GEMM (the last reader of W3) and the extra optimiser launch competes with the next update's forward.  Opt-in.
-_FUSE_ADAM = bool(os.environ.get("SSAC_FUSED_ADAM"))
 _U_ASYNC = 0 if os.environ.get("SSAC_NO_UASYNC") else 1   # A/B switch: v / u of the split backward on the second stream
 
 
@@ -171,7 +167,6 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
                                             _idx=draws["idx"])
             presampled.append((draws, rd))
     replay_dicts = [None] * E
-    adam_done = []
 
     def member_step(i, draws, rd, lane, batch_ready=None):
         loss_v = loss_all[2 * i:2 * i + 2]
@@ -197,9 +192,6 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         # three weight-gradient reductions remain.
         split_bwd = side is not None and ca.O == 1 and ca.D <= 32 and not dr3_coeff and L.default_mlp_impl() == 2
         bws = _ops._bwd_ws(N, B, ca.H, dev) if split_bwd else None
-        # one member, no global-norm clipping (that needs every gradient first): the optimiser step rides in the epilogues
-        fuse_adam = (split_bwd and _FUSE_ADAM and E == 1 and not critic_clip and not parallel.is_sharded()
-                     and not parallel.members_sharded())
         if side is not None:
             main = torch.cuda.current_stream(dev)
             if piped:
@@ -268,19 +260,8 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
             extra, extra_scale, f1 = h2b, dr3_coeff / (E * Ng) / (Ng * B), (X1, h1b, h2b)
         dxg = torch.empty((N, B, S + A), dtype=torch.float32, device=dev) if need_ds else None
         if pipe is not None:
-            pipe.join_deferred(torch.cuda.current_stream(dev))   # the previous update's logged gradient norm reads what follows overwrites
             pipe.cross_before_grads(torch.cuda.current_stream(dev))
-        if split_bwd and fuse_adam:
-            # Adam applied by the two weight-gradient reductions themselves (no optimiser pass on the chain)
-            if pipe is not None:
-                pipe.main_wait_polyak(torch.cuda.current_stream(dev))   # a Polyak step still reads the online parameters
-            gW1, gb1, gW2, gb2, gW3, gb3 = ca.ptrs(i * N, grad=True)
-            lr, b1, b2, eps, wd = opt.hyper()
-            L.mlp_backward_post_adam(W3, N, ca.D, ca.H, X.data_ptr(), S + A, 0, B, h1.data_ptr(), h2.data_ptr(),
-                                     dq.data_ptr(), bws.data_ptr(), gW1, gb1, gW2, gb2, gW3, gb3, *opt.fused_offsets(),
-                                     opt.ctl.data_ptr(), lr, b1, b2, eps, wd, 0, _lib.stream_ptr())
-            adam_done.append(True)
-        elif split_bwd:
+        if split_bwd:
             gW1, gb1, gW2, gb2, gW3, gb3 = ca.ptrs(i * N, grad=True)
             L.mlp_backward_post(W3, N, ca.D, ca.H, X.data_ptr(), S + A, 0, B, h1.data_ptr(), h2.data_ptr(), dq.data_ptr(),
                                 bws.data_ptr(), gW1, gb1, gW2, gb2, gW3, gb3, 0, _lib.stream_ptr())
@@ -359,19 +340,13 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         # Adam on the second stream instead of behind it
         with torch.cuda.stream(side):
             parallel.all_reduce_sum_(loss_all[0:1], site="critic_loss")
-    if adam_done:
-        opt.note_fused_step()
-    else:
-        if pipe is not None:
-            pipe.main_wait_polyak(torch.cuda.current_stream(dev))   # a Polyak step on the auxiliary stream still reads these
-        opt.step(stream, max_norm=critic_clip if critic_clip else None)
+    if pipe is not None:
+        pipe.main_wait_polyak(torch.cuda.current_stream(dev))   # a Polyak step on the auxiliary stream still reads these
+    opt.step(stream, max_norm=critic_clip if critic_clip else None)
     if pipe is not None:
         pipe.cross_after_adam(torch.cuda.current_stream(dev))
     if side is not None:
-        if pipe is not None and adam_done:
-            pipe.defer_join(side)   # nothing on the caller's stream needs the logged norm before the next backward
-        else:
-            main.wait_stream(side)
+        main.wait_stream(side)
     else:
         gslot = lu._member_grad_norm_slot(logs, ca, member * N, (member + 1) * N)
         if parallel.is_sharded():

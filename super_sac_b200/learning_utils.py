@@ -237,7 +237,6 @@ class _Pipeline:
         self.polyak = None       # event of the latest Polyak step (the target critics' parameters), for the front stream
         self.polyak_main = None  # the same event, for the caller's stream (its next Adam step)
         self.aux = None          # stream the Polyak steps run on
-        self.deferred = []       # streams with log-only work the caller's stream has not joined yet
         self.cross = graphed.cross_capturing()   # (state, slot): this block is ONE update captured for cross-call pipelining
         self.keep = []           # front-allocated tensors that main-stream kernels read: alive until the block ends
         self.needs_order = False  # a barrier happened: the front's next work goes behind the caller's stream as it is then
@@ -300,16 +299,6 @@ class _Pipeline:
         self.polyak = ev
         self.polyak_main = ev
 
-    def defer_join(self, stream):
-        """A log-only reduction over the gradients runs on `stream`: the caller's stream joins it only before the next
-        backward overwrites the gradient arrays (or when the block ends), not before the next forward."""
-        self.deferred.append(stream)
-
-    def join_deferred(self, main):
-        for st in self.deferred:
-            main.wait_stream(st)
-        self.deferred.clear()
-
     def main_wait_polyak(self, main):
         """Before the caller's stream overwrites the online parameters (Adam) a Polyak step still reads."""
         if self.polyak_main is not None:
@@ -365,7 +354,6 @@ def pipelined_updates(device=None):
         main.wait_stream(p.front)
         if p.aux is not None:
             main.wait_stream(p.aux)
-        p.join_deferred(main)
         p.keep.clear()
 
 
@@ -381,7 +369,6 @@ def pipeline_barrier():
         if p.aux is not None:
             main.wait_stream(p.aux)
             p.polyak_main = None
-        p.join_deferred(main)
         p.needs_order = True
 
 
@@ -577,38 +564,29 @@ def _actor_forward(agent, i, X, B, S, A, keep=False):
     return out, h1, h2
 
 
-TARGET_CHAIN = False
-
-
 def _rows_ok(D, H, O):
     """The row-local CUDA-core kernel (ssac_mlp_rows.cu) covers this shape and is switched on."""
     return bool(_lib.lib().rows_supported(int(D), int(H), int(O)))
 
 
-def _policy_sample(agent, i, X, B, S, A, random_process, noise_clip, rsample=False, eps=None, noise=None, keep=None,
-                   chain=None):
+def _policy_sample(agent, i, X, B, S, A, random_process, noise_clip, rsample=False, eps=None, noise=None, keep=None):
     """a ~ pi_i(.|s) written into X[:, S:], with log-prob [B] (None when a noise process replaces the entropy term):
     actor MLP + policy head in one entry point (the head is fused into the output-layer kernel).  ``eps`` / ``noise``:
     pre-drawn N(0,1) tensors (drawn here otherwise).  Returns dict(out, h1, h2, eps, logp, tanh_out); h1 / h2 are only
-    valid when ``keep`` (default: rsample, i.e. a backward pass follows).
-
-    ``chain = (critic_arena, g0, net_index, M)`` (forward-only): the M critics net_index[m] of that arena (relative to
-    net g0) are evaluated on (s, a) in the SAME launch (ssac_target_chain); their values come back as ``qt`` [M,B,1]."""
+    valid when ``keep`` (default: rsample, i.e. a backward pass follows)."""
     dev = X.device
     keep = rsample if keep is None else keep
     arena = agent._actor_arena
     det = agent.deterministic
     use_rows = (not keep and _lib.lib().default_mlp_impl() == 2 and _rows_ok(S + A, arena.H, arena.O) and A <= 8
-                and (B <= 64 or chain is not None))   # the acting path (B = num_envs); large batches keep the tensor cores
-    if chain is not None and not (use_rows and chain[0].H == arena.H and chain[0].O == 1 and chain[0].D == S + A):
-        chain = None
+                and B <= 64)   # the acting path (B = num_envs); large batches keep the tensor cores
     h1 = h2 = out = None
     if not use_rows:
         h1 = torch.empty((1, B, arena.H), dtype=torch.float32, device=dev)
         h2 = torch.empty_like(h1)
         out = torch.empty((1, B, arena.O), dtype=torch.float32, device=dev)
     a_dst = X[:, S:]
-    res = dict(out=out, h1=h1, h2=h2, eps=None, logp=None, tanh_out=None, qt=None)
+    res = dict(out=out, h1=h1, h2=h2, eps=None, logp=None, tanh_out=None)
     sigma, clip, tanh_out, logp = 0.0, 0.0, None, None
     if det:
         if rsample and eps is None:  # Normal(loc, 1e-4).rsample() of the reference's deterministic "distribution"
@@ -641,15 +619,7 @@ def _policy_sample(agent, i, X, B, S, A, random_process, noise_clip, rsample=Fal
         logp = torch.empty((B,), dtype=torch.float32, device=dev)
     W1, b1, W2, b2, W3, b3 = arena.ptrs(i)
     L = _lib.lib()
-    if chain is not None:
-        c_arena, g0, net_index, M = chain
-        qt = torch.empty((M, B, 1), dtype=torch.float32, device=dev)
-        cW1, cb1, cW2, cb2, cW3, cb3 = c_arena.ptrs(g0)
-        L.target_chain(W1, b1, W2, b2, W3, b3, S, arena.H, A, int(det), cW1, cb1, cW2, cb2, cW3, cb3, _ops._p(net_index), M,
-                       X.data_ptr(), S + A, B, _ops._p(eps), _ops._p(noise), sigma, clip, float(agent.log_std_low),
-                       float(agent.log_std_high), _ops._p(logp), qt.data_ptr(), _lib.stream_ptr())
-        res["qt"] = qt
-    elif use_rows:
+    if use_rows:
         L.policy_rows(W1, b1, W2, b2, W3, b3, arena.D, arena.H, A, int(det), X.data_ptr(), S + A, B, None, _ops._p(eps),
                       _ops._p(noise), sigma, clip, float(agent.log_std_low), float(agent.log_std_high), a_dst.data_ptr(),
                       S + A, _ops._p(logp), _ops._p(tanh_out), _lib.stream_ptr())
@@ -735,33 +705,19 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
     # REDQ subset: drawn over the GLOBAL ensemble when the critics are sharded over ranks (replicated Philox state)
     pool = parallel.n_global() if parallel.is_sharded() else N
     assert 0 < ensemble_n <= pool
-    # ssac_target_chain (actor + target-critic subset + action write-back in ONE row-local CUDA-core launch) is exact fp32
-    # but measured SLOWER than the two tensor-core launches it replaces at B = 256 (35 vs 31 us back to back, and it takes
-    # SMs away from the online critics' branch): off unless TARGET_CHAIN is set (kept for small batches / A-B runs)
-    want_chain = TARGET_CHAIN and not parallel.is_sharded()
-    if want_chain and _pipeline is not None:
-        _pipeline.front_wait_polyak()
     if _draws is not None:   # critic_update drew indices, policy noise and the subset in ONE launch
         net_index = _draws["subset"]
         pol = _policy_sample(agent, i, X1, B, S, A, random_process, noise_clip,
                              eps=None if agent.deterministic else _draws["normal"],
-                             noise=_draws["normal"] if agent.deterministic else None,
-                             chain=(target_agent._critic_arena, i * N, net_index, ensemble_n) if want_chain else None)
+                             noise=_draws["normal"] if agent.deterministic else None)
     else:
         net_index = torch.empty(ensemble_n, dtype=torch.int32, device=X1.device)
         # (the reference draws the policy sample first, the subset second: learning_utils.py:321, agent.py:29)
-        if want_chain and isinstance(_rng.source(), _rng.PhiloxSource):
-            _rng.source().subsets(net_index, pool, ensemble_n)   # independent Philox draws: the order is immaterial
-            pol = _policy_sample(agent, i, X1, B, S, A, random_process, noise_clip,
-                                 chain=(target_agent._critic_arena, i * N, net_index, ensemble_n))
-        else:
-            pol = _policy_sample(agent, i, X1, B, S, A, random_process, noise_clip)
-            _rng.source().subsets(net_index, pool, ensemble_n)
+        pol = _policy_sample(agent, i, X1, B, S, A, random_process, noise_clip)
+        _rng.source().subsets(net_index, pool, ensemble_n)
     if _pipeline is not None:
         _pipeline.front_wait_polyak()   # the target critics' parameters: the only thing this side reads that Polyak writes
-    if pol.get("qt") is not None:
-        q_t = pol["qt"]
-    elif parallel.is_sharded():
+    if parallel.is_sharded():
         # every rank evaluates its own target critics and all-gathers the [N_global, B] values; the subset-min is then
         # identical on every rank
         q_t = parallel.all_gather_q(_critic_values(target_agent, i * N, N, X1, B), site="target_q", select=net_index)

@@ -45,7 +45,7 @@ def test_workspace_plan_cpu():
     kf, kfp, ks, nsplit, total = [off[i] for i in range(24, 29)]
     assert rows == pitch == [42, 41, 39, 37]      # layer l works on its input grid: s2d 42, then the valid outputs 41 / 39 / 37
     assert kf == 37 * 37 * 32 and kfp == ks * nsplit >= kf and ks % 32 == 0
-    assert total == n.value and all(off[i] % 256 == 0 or off[i] == -1 for i in range(16))
+    assert total == n.value and all(off[i] % 256 == 0 for i in range(16))
     with pytest.raises(_lib.SsacError):
         lib.conv_encoder_ws_floats(4, 17, 84, 84, 50, 1, ctypes.byref(n))   # 4C must fit 64 channels
     with pytest.raises(_lib.SsacError):
@@ -302,11 +302,24 @@ def test_fused_encoder_optimizer_step_matches_torch():
     assert _encoder_opt.eligible(a, oa) is a.net
 
 
+@pytest.fixture
+def conv_halo(request):
+    """ssac_set_conv_halo(mode) for the duration of one test, then the default (3) again."""
+    from super_sac_b200 import _lib
+
+    _lib.lib().set_conv_halo(request.param)
+    yield request.param
+    _lib.lib().set_conv_halo(3)
+
+
 @pytest.mark.gpu
+@pytest.mark.parametrize("conv_halo", [3, 0], ids=["halo", "per-tap"], indirect=True)
 @pytest.mark.parametrize("B,C,H,W,O", [(1, 9, 84, 84, 50), (2, 1, 16, 16, 8), (3, 16, 20, 28, 64), (7, 4, 32, 18, 33)])
-def test_encoder_edge_geometries_against_oracle(B, C, H, W, O):
+def test_encoder_edge_geometries_against_oracle(B, C, H, W, O, conv_halo):
     """Batch of one (the acting path), one channel, the widest channel count (4C = 64), non-square images, the smallest
-    image (a single valid output pixel in the last layer), an odd output width."""
+    image (a single valid output pixel in the last layer), an odd output width.  Each with the default kernel choice
+    (halo tiles wherever the halo box fits, as it does at these sizes) and with the per-tap kernels forced (mode 0: the
+    fallback for images whose halo box does not fit)."""
     from super_sac_b200.nets import cnns
 
     rng = np.random.default_rng(B * 1000 + C)

@@ -518,59 +518,6 @@ def test_split_critic_backward_matches_oracle(G, D, H, B, u_async):
         gu.assert_close(ar.g[n].cpu().numpy(), split[n].numpy(), 1e-4, 2e-6 * float(split[n].abs().max()), f"split vs one-call {n}")
 
 
-@pytest.mark.parametrize("wd", [0.0, 1e-3])
-@pytest.mark.parametrize("G,D,H,B", [(10, 23, 256, 256), (2, 4, 64, 200), (3, 32, 128, 300)])
-def test_split_backward_with_fused_adam_equals_separate_adam(G, D, H, B, wd):
-    """ssac_mlp_backward_post_adam (Adam applied by the two weight-gradient kernels to the elements they produce) ==
-    ssac_mlp_backward_post followed by ssac_adam_step over the arena: same gradients, bit-identical parameters and
-    moments over three steps, step counter advanced once per call."""
-    gen = torch.Generator().manual_seed(G * 7 + H + B)
-    st = uo.MLPStack(G, D, H, 1).random_init(gen)
-    ars = [_arena_from(st), _arena_from(st)]
-    ms = [torch.zeros_like(a.flat) for a in ars]
-    vs = [torch.zeros_like(a.flat) for a in ars]
-    ctls = [torch.zeros(8, dtype=torch.int32, device=DEV) for _ in ars]
-    ws = torch.empty(L().mlp_backward_ws(G, B, H), dtype=torch.float32, device=DEV)
-    lr, b1, b2, eps = 3e-4, 0.9, 0.999, 1e-8
-    for step in range(3):
-        x = torch.randn(B, D, generator=gen).to(DEV)
-        dq = (torch.randn(G, B, 1, generator=gen) / B).to(DEV)
-        h1 = torch.empty(G, B, H, device=DEV)
-        h2 = torch.empty(G, B, H, device=DEV)
-        q = torch.empty(G, B, 1, device=DEV)
-        for k, ar in enumerate(ars):
-            from super_sac_b200 import _ops
-            _ops.mlp_forward(ar, 0, G, x, B, h1, h2, q, keep_hidden=True)
-            W1, _, W2, _, W3, _ = ar.ptrs(0)
-            gW1, gb1, gW2, gb2, gW3, gb3 = ar.ptrs(0, grad=True)
-            ar.grad.zero_()
-            L().mlp_backward_pre(W2, W3, G, H, B, h1.data_ptr(), h2.data_ptr(), ws.data_ptr(), 1, 2, None)
-            if k == 0:
-                L().mlp_backward_post(W3, G, D, H, x.data_ptr(), D, 0, B, h1.data_ptr(), h2.data_ptr(), dq.data_ptr(), ws.data_ptr(),
-                                      gW1, gb1, gW2, gb2, gW3, gb3, 2, None)
-                # Adam over every array of the arena (the alignment gaps between the arrays hold no parameters)
-                for off, n in ar.range_table(0, G):
-                    c = torch.zeros(8, dtype=torch.int32, device=DEV)
-                    c[0] = step
-                    L().adam_step(ar.flat.data_ptr() + 4 * off, ar.grad.data_ptr() + 4 * off, ms[k].data_ptr() + 4 * off,
-                                  vs[k].data_ptr() + 4 * off, n, c.data_ptr(), lr, b1, b2, eps, wd, None, 0.0, 0, None)
-            else:
-                g0 = ar.grad.data_ptr()
-                offs = [(t.data_ptr() - g0) // 4 for t in (ar.flat, ms[k], vs[k])]
-                L().mlp_backward_post_adam(W3, G, D, H, x.data_ptr(), D, 0, B, h1.data_ptr(), h2.data_ptr(), dq.data_ptr(),
-                                           ws.data_ptr(), gW1, gb1, gW2, gb2, gW3, gb3, *offs, ctls[k].data_ptr(), lr, b1, b2, eps,
-                                           wd, 2, None)
-        torch.cuda.synchronize()
-        assert ctls[1].tolist()[:5] == [step + 1, 0, 0, 0, 0]
-        for n in uo.PARAM_NAMES:
-            assert torch.equal(ars[0].g[n], ars[1].g[n]), f"step {step}: grad {n}"
-            assert torch.equal(ars[0].p[n], ars[1].p[n]), f"step {step}: param {n}"
-        for name in uo.PARAM_NAMES:
-            off, n = ars[0].offsets[name], G * ars[0].net_stride[name]
-            assert torch.equal(ms[0][off:off + n], ms[1][off:off + n]), f"step {step}: exp_avg {name}"
-            assert torch.equal(vs[0][off:off + n], vs[1][off:off + n]), f"step {step}: exp_avg_sq {name}"
-
-
 @pytest.mark.parametrize("G,S,A,H,B", [(10, 17, 6, 256, 256), (2, 3, 1, 64, 100), (3, 11, 12, 128, 130)])
 def test_action_gradient_through_critics(G, S, A, H, B):
     """ssac_mlp_backward_dact == input-gradient pass of ssac_mlp_backward summed over the nets (and the oracle)."""
@@ -785,7 +732,7 @@ def test_advantage_estimator_mean_and_max(method):
     gu.assert_close(got.cpu().numpy(), want.numpy(), 1e-4, 2e-5, f"advantage ({method})")
 
 
-# ------------------------------------------------------------------------------------------------ row-local CUDA-core chains
+# ------------------------------------------------------------------------------------------------ row-local CUDA-core forwards
 def _rand_stack(G, D, H, O, seed):
     return uo.MLPStack(G, D, H, O).random_init(torch.Generator().manual_seed(seed))
 
@@ -803,42 +750,6 @@ def test_rows_forward_matches_oracle(G, D, H, O, B):
                     p["b3"].data_ptr(), None, G, D, H, O, xd.data_ptr(), D + 3, 0, B, None, None, 0, y.data_ptr(), 3, S())
     want = torch.stack([uo.mlp_forward(st, g, x[:, :D])[0] for g in range(G)], 0)
     gu.assert_close(y.cpu().numpy(), want.numpy(), 1e-5, 2e-6, "rows forward")
-
-
-@pytest.mark.parametrize("det", [False, True])
-@pytest.mark.parametrize("B", [256, 13])
-def test_target_chain_matches_oracle(det, B):
-    """ssac_target_chain: a1, logp = pi(s1) (tanh-Normal sample / deterministic head + TD3 noise), written into the action
-    columns, then the REDQ subset of target critics on (s1, a1) -- one launch -- against the oracle's per-net loops."""
-    S_, A, H, N, M = 17, 6, 256, 10, 2
-    actor = _rand_stack(1, S_, H, A if det else 2 * A, seed=1)
-    critics = _rand_stack(N, S_ + A, H, 1, seed=2)
-    g = torch.Generator().manual_seed(B)
-    s1 = torch.randn(B, S_, generator=g)
-    eps, noise = torch.randn(B, A, generator=g), torch.randn(B, A, generator=g)
-    subset = [7, 2]
-    X1 = torch.zeros(B, S_ + A)
-    X1[:, :S_] = s1
-    xd = X1.to(DEV)
-    pa = {n: getattr(actor, n).to(DEV).contiguous() for n in uo.PARAM_NAMES}
-    pc = {n: getattr(critics, n).to(DEV).contiguous() for n in uo.PARAM_NAMES}
-    ni = dev(np.array(subset, dtype=np.int32))
-    logp = torch.empty(B, device=DEV)
-    qt = torch.empty(M, B, 1, device=DEV)
-    ed, nd = eps.to(DEV), noise.to(DEV)
-    L().target_chain(*(pa[n].data_ptr() for n in uo.PARAM_NAMES), S_, H, A, int(det), *(pc[n].data_ptr() for n in uo.PARAM_NAMES),
-                     ni.data_ptr(), M, xd.data_ptr(), S_ + A, B, None if det else ed.data_ptr(), nd.data_ptr() if det else None,
-                     0.6, 0.3, -5.0, 2.0, None if det else logp.data_ptr(), qt.data_ptr(), S())
-    out = uo.mlp_forward(actor, 0, s1)[0]
-    if det:
-        a1 = uo.gaussian_noise_clamp(torch.tanh(out), noise, 0.6, 0.3, -1.0, 1.0)
-    else:
-        a1, lp, _ = uo.tanh_normal_sample(out, eps, -5.0, 2.0)
-        gu.assert_close(logp.cpu().numpy(), lp.squeeze(1).numpy(), 1e-4, 1e-4, "chain logp")
-    gu.assert_close(xd[:, S_:].cpu().numpy(), a1.numpy(), 1e-5, 1e-6, "chain action")
-    assert torch.equal(xd[:, :S_].cpu(), s1)
-    want = torch.stack([uo.mlp_forward(critics, k, torch.cat((s1, a1), -1))[0] for k in subset], 0)
-    gu.assert_close(qt.cpu().numpy(), want.numpy(), 1e-4, 1e-5, "chain target Q")
 
 
 @pytest.mark.parametrize("envs", [1, 5])

@@ -1,30 +1,19 @@
 #!/usr/bin/env python
-"""Timing of the row-local chain kernel against the two tensor-core launches it replaces (one JSON line each)."""
+"""Timing of the row-local forward (impl 3 of ssac_mlp_forward) against the tensor-core forward (one JSON line each)."""
 import json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tools"))
 import torch
 import benchlib as bl
 import super_sac_b200 as ssb
-from super_sac_b200 import _lib, learning_utils as lu
+from super_sac_b200 import _lib
 
 dev = torch.device("cuda", 0)
 W = bl.Workload(ssb, "redq", dev, buffer_size=10000)
-agent, target = W.agent, W.target
-S, A, B, N, M = 17, 6, 256, 10, 2
+target = W.target
+S, A, B = 17, 6, 256
 X1 = torch.randn(B, S + A, device=dev)
-eps = torch.randn(B, A, device=dev)
-ni = torch.tensor([3, 7], dtype=torch.int32, device=dev)
 L = _lib.lib()
-for on in (1, 0):
-    L.set_rows_enabled(on)
-    def chain():
-        pol = lu._policy_sample(agent, 0, X1, B, S, A, None, None, eps=eps, chain=(target._critic_arena, 0, ni, M))
-        if pol["qt"] is None:
-            lu._critic_values(target, 0, M, X1, B, net_index=ni)
-    ms = bl.graph_time(chain, per=10, iters=20)
-    print(json.dumps({"what": "target path (actor + 2 target critics), B=256", "rows_kernel": bool(on), "us": ms * 1e3}), flush=True)
-L.set_rows_enabled(1)
 for G in (1, 2, 3, 10):
     q = torch.empty(G, B, 1, device=dev)
     ca = target._critic_arena
