@@ -11,13 +11,16 @@ CUDA graphs under ``graphed.enable_auto_graphs()``; inside ``lu.pipelined_update
 critic update runs on the block's front stream (as in learning._critic_update_impl).  The offline (AFBC) actor update
 with the indirect advantage filter (adv_estimator.py:45-56) and the priority refresh are here too.  Not implemented
 (raise): softmax Bellman weights (they draw Categorical samples), the invariance regularisers, sharded ensembles.
+
+Only the member bodies are this module's own.  The skeleton around them -- pipeline eligibility, member batches, the
+member loop, the encoder step, the logged gradient norms and the temperature step -- is learning_utils' "shared pieces
+of the updates", which learning.py uses as well.
 """
 import contextlib
-import random
 
 import torch
 
-from . import _arena, _encoder_opt, _lib, _logs, _ops, _rng, parallel
+from . import _arena, _lib, _logs, _ops, _rng, parallel
 from . import learning_utils as lu
 
 
@@ -134,23 +137,14 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
     _check(agent)
     if encoder_lambda:
         raise NotImplementedError("encoder invariance regulariser (lambda = 0 in every shipped config) is out of scope")
-    from .learning import _encoder_trainable
-
     ca = agent._critic_arena
     dev = ca.device
     L, stream = _lib.lib(), _lib.stream_ptr()
     E, N, B, A = agent.ensemble_size, agent.num_critics, batch_size, agent.act_space_size
     # Inside lu.pipelined_updates(): the target side (draws, gather, actor logits and target-critic subset on s1, state
-    # value, TD target) runs on the front stream, the online side on the caller's; the same eligibility as the continuous
-    # path (one member, uniform sampling, plain Bellman backups, no trainable encoder), else serial.  PopArt stays serial
-    # too: the next update's TD target rescales the PopArt layer this update's loss seed still reads.
-    pipe = lu.pipeline()
-    if pipe is not None and (E != 1 or per or update_priorities or weight_type is not None or _encoder_trainable(agent)
-                             or any(bool(p) for p in agent.popart) or lu.side_stream(dev) is None or pipe.device != dev):
-        pipe = None
-    if pipe is None:
-        lu.pipeline_barrier()
-    else:
+    # value, TD target) runs on the front stream, the online side on the caller's (eligibility: lu._critic_pipeline).
+    pipe = lu._critic_pipeline(agent, per, update_priorities, weight_type)
+    if pipe is not None:
         main = torch.cuda.current_stream(dev)
         pipe.front_wait_dep(main)
     with (torch.cuda.stream(pipe.front) if pipe is not None else contextlib.nullcontext()):
@@ -159,8 +153,9 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
         pipe.keep.append(logs)
     loss_all, loss_slot = logs.slots(2 * E)   # per member: {loss contribution, mean td error of its last net}
     opt = _arena.FlatAdam.attach(critic_optimizer, ca)
-    enc_outs, replay_dicts = [], []
-    for i in range(E):
+    enc_outs = []
+
+    def member_step(i):
         loss_v = loss_all[2 * i:2 * i + 2]
         with (torch.cuda.stream(pipe.front) if pipe is not None else contextlib.nullcontext()):
             rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
@@ -214,39 +209,21 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
                               want_dw=True, accumulate=True)
         if need_ds:
             enc_outs.append((s_rep, dxg.sum(0)))
-        replay_dicts.append(rd)
+        return rd
 
-    encoder_optimizer.zero_grad()
-    if enc_outs:
-        torch.autograd.backward([s for s, _ in enc_outs], [g for _, g in enc_outs])
+    replay_dicts = lu._run_members(E, dev, False, member_step)
+    logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)
+    logs.defer("losses/critic_overall_loss", [loss_slot + 2 * i for i in range(E)])
+    enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
     if critic_clip:
         opt.grad_norm_sq(stream)
-    enc_net = None
-    if enc_outs:
-        enc_net = _encoder_opt.fused_step(agent.encoder, encoder_optimizer, encoder_clip)
-        if enc_net is None:
-            if encoder_clip:
-                torch.nn.utils.clip_grad_norm_(agent.encoder.parameters(), encoder_clip)
-            encoder_optimizer.step()
-    member = random.choice(range(E))
     if pipe is not None:
         pipe.main_wait_polyak(main)   # a Polyak step on the block's auxiliary stream still reads the online parameters
     opt.step(stream, max_norm=critic_clip if critic_clip else None)   # (clipping rescales the stored gradients, as the reference's does)
-    gslot = lu._member_grad_norm_slot(logs, ca, member * N, (member + 1) * N)
-    logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)
-    logs.defer("losses/critic_overall_loss", [loss_slot + 2 * i for i in range(E)])
-    logs.defer("gradients/critic_random_grad", gslot, transform=lambda v: v**0.5)
-    if enc_net is not None:
-        v, eslot = logs.slots(1)
-        _encoder_opt.grad_norm_sq_into(enc_net, v)
-        logs.defer("gradients/encoder_criticloss_grad_norm", eslot, transform=lambda v: v**0.5)
-    elif enc_outs:
-        gn = torch.linalg.vector_norm(torch.stack([p.grad.norm() for p in agent.encoder.parameters() if p.grad is not None]))
-        logs.put_tensor("gradients/encoder_criticloss_grad_norm", gn)
-    else:
-        logs["gradients/encoder_criticloss_grad_norm"] = 0.0
+    lu._log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad")
+    lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_criticloss_grad_norm")
     if update_priorities:
-        lu.adjust_priorities(logs, rd, agent, buffer)
+        lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)
     return logs.finalize(), replay_dicts
 
 
@@ -263,11 +240,9 @@ def online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_s
     logs = _logs.DeviceLogs(dev)
     loss_all, loss_slot = logs.slots(E)
     opt = _arena.FlatAdam.attach(actor_optimizer, aa)
-    for i in range(E):
-        if premade_replay_dicts is not None:
-            rd = premade_replay_dicts[i]
-        else:
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
+
+    def member_step(i):
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per)
         o, *_ = rd["primary_batch"]
         with torch.no_grad():  # actor gradients do not train the encoder (learning.py:378-380)
             s_rep = agent.encoder(o)
@@ -280,18 +255,18 @@ def online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_s
                               popart.state_ptr() if popart else None, int(bool(pop)), E, dlogits.data_ptr(),
                               loss_all[i:i + 1].data_ptr(), stream)
         _ops.mlp_backward(aa, i, 1, X, B, h1, h2, dlogits, ldx=ld, want_dw=True, accumulate=False)
+
+    lu._run_members(E, dev, False, member_step)
     if clip:
         opt.grad_norm_sq(stream)
     opt.step(stream, max_norm=clip if clip else None)
-    member = random.choice(range(E))
-    gslot = lu._member_grad_norm_slot(logs, aa, member, member + 1)
-    logs.defer("gradients/random_actor_online_grad", gslot, transform=lambda v: v**0.5)
+    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/random_actor_online_grad")
     logs.defer("losses/actor_pg_loss", [loss_slot + i for i in range(E)])
     return logs.finalize()
 
 
 def alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, aug_mix, target_entropy,
-                 premade_replay_dicts, alpha_state_cls):
+                 premade_replay_dicts):
     """learning.py:222-263 with discrete=True: logp = sum_a p log p (the policy's negative entropy, :252-253)."""
     _check(agent)
     lu.pipeline_barrier()
@@ -300,11 +275,9 @@ def alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, a
     L, stream = _lib.lib(), _lib.stream_ptr()
     E, B, A = agent.ensemble_size, batch_size, agent.act_space_size
     logs = _logs.DeviceLogs(dev)
-    for i in range(E):
-        if premade_replay_dicts is not None:
-            rd = premade_replay_dicts[i]
-        else:
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, per=False, aug_mix=aug_mix)
+
+    def member_step(i):
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, False)
         o, *_ = rd["primary_batch"]
         with torch.no_grad():
             s_rep = agent.encoder(o)
@@ -312,16 +285,9 @@ def alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, a
         logits = _forward(aa, i, 1, X, ld, B)
         plogp = torch.empty(B, dtype=torch.float32, device=dev)
         L.discrete_neg_entropy(logits.data_ptr(), B, A, plogp.data_ptr(), stream)
-        pg = optimizers[i].param_groups[0]
-        st = alpha_state_cls.attach(optimizers[i], log_alphas[i])
-        lv, slot = logs.slots(2)
-        L.alpha_step(log_alphas[i].data_ptr(), plogp.data_ptr(), B, float(target_entropy), st.state.data_ptr(),
-                     st.ctl.data_ptr(), float(pg["lr"]), float(pg["betas"][0]), float(pg["betas"][1]), float(pg["eps"]),
-                     lv.data_ptr(), stream)
-        st.steps += 1
-        st._step_tensor.fill_(st.steps)
-        logs.defer(f"losses/alpha_loss_{i}", slot)
-        logs.defer(f"alphas/alpha_{i}", slot + 1)
+        lu._alpha_step(logs, i, optimizers[i], log_alphas[i], plogp, B, target_entropy)
+
+    lu._run_members(E, dev, False, member_step)
     return logs.finalize()
 
 
@@ -365,11 +331,9 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
     loss_all, loss_slot = logs.slots(E)
     opt = _arena.FlatAdam.attach(actor_optimizer, aa)
     enc_outs = []
-    for i in range(E):
-        if premade_replay_dicts is not None:
-            rd = premade_replay_dicts[i]
-        else:
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
+
+    def member_step(i):
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per)
         o, a, *_ = rd["primary_batch"]
         mask = None
         if filter_:
@@ -393,28 +357,16 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
         _ops.mlp_backward(aa, i, 1, X, B, h1, h2, dlogits, ldx=ld, want_dw=True, accumulate=False, dx=dxg, lddx=S)
         if need_ds:
             enc_outs.append((s_rep, dxg[0]))
-    encoder_optimizer.zero_grad()
-    if enc_outs:
-        torch.autograd.backward([s for s, _ in enc_outs], [g for _, g in enc_outs])
+        return rd
+
+    replay_dicts = lu._run_members(E, dev, False, member_step)
+    enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
     if actor_clip:
         opt.grad_norm_sq(stream)
-    enc_net = None
-    if update_encoder and enc_outs:
-        enc_net = _encoder_opt.fused_step(agent.encoder, encoder_optimizer, encoder_clip)
-    if enc_net is None and encoder_clip and enc_outs:
-        torch.nn.utils.clip_grad_norm_(agent.encoder.parameters(), encoder_clip)
     opt.step(stream, max_norm=actor_clip if actor_clip else None)
-    if enc_net is None and update_encoder and enc_outs:
-        encoder_optimizer.step()
     logs.defer("losses/filtered_bc_overall_loss", [loss_slot + i for i in range(E)], transform=lambda v: v / E)
-    member = random.choice(range(E))
-    gslot = lu._member_grad_norm_slot(logs, aa, member, member + 1)
-    logs.defer("gradients/actor_offline_grad_norm", gslot, transform=lambda v: v**0.5)
-    if enc_outs:
-        gn = torch.linalg.vector_norm(torch.stack([p.grad.norm() for p in agent.encoder.parameters() if p.grad is not None]))
-        logs.put_tensor("gradients/encoder_offline_actorloss_grad_norm", gn)
-    else:
-        logs["gradients/encoder_offline_actorloss_grad_norm"] = 0.0
+    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/actor_offline_grad_norm")
+    lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_offline_actorloss_grad_norm")
     if per:
-        lu.adjust_priorities(logs, rd, agent, buffer)
+        lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)
     return logs.finalize()

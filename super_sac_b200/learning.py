@@ -5,18 +5,17 @@ Same signatures, same returned log keys, same arithmetic (fp32) -- but every mem
 launch, the backward is explicit (no autograd tape on the ensemble), Adam is one fused pass over the flat parameter
 arena, and the logged scalars come back with a single device->host copy.  The caller still owns the optimizer
 objects, ``log_alphas`` and the target agent exactly as main.py:188-244 / :321 builds them.
+
+This module holds the continuous member bodies and routes ``discrete=True`` to discrete.py.  The skeleton around the
+bodies -- pipeline eligibility, member batches, member stream lanes, the encoder step, the logged gradient norms and
+the temperature step -- is shared with discrete.py and lives in learning_utils ("shared pieces of the updates").
 """
 import contextlib
-import os
-import random
 
 import torch
 
 from . import _arena, _encoder_opt, _lib, _logs, _ops, _rng, discrete as _discrete, graphed, parallel
 from . import learning_utils as lu
-
-
-_U_ASYNC = 0 if os.environ.get("SSAC_NO_UASYNC") else 1   # A/B switch: v / u of the split backward on the second stream
 
 
 def _encoder_has_grad_path(s_rep):
@@ -28,13 +27,6 @@ def _opt_sig(opt):
     return (id(opt), pg["lr"], tuple(pg["betas"]), pg["eps"], pg["weight_decay"])
 
 
-def _encoder_trainable(agent):
-    ps = agent.__dict__.get("_ssac_encoder_params")
-    if ps is None:   # walking the module tree on every update call costs more than the check itself
-        ps = agent.__dict__["_ssac_encoder_params"] = [p for p in agent.encoder.parameters() if p.numel() > 2]
-    return any(p.requires_grad for p in ps)
-
-
 def _graphable(agent, random_process, per, update_priorities, encoder_optimizer=None):
     """Static shapes, device-side randomness (incl. the exploration-noise scale, GaussianExplorationNoise.scale_dev), no
     PyTorch autograd hand-off -- a parameterised encoder only if it is the native pixel encoder with its fused optimiser
@@ -42,7 +34,7 @@ def _graphable(agent, random_process, per, update_priorities, encoder_optimizer=
     return (graphed.auto_graphs_enabled() and isinstance(_rng.source(), _rng.PhiloxSource) and not per and
             not update_priorities and (random_process is None or hasattr(random_process, "scale_dev")) and
             not parallel.is_sharded() and not parallel.members_sharded() and
-            (not _encoder_trainable(agent) or _encoder_opt.structurally_eligible(agent.encoder, encoder_optimizer)))
+            (not lu._encoder_trainable(agent) or _encoder_opt.structurally_eligible(agent.encoder, encoder_optimizer)))
 
 
 def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimizer, log_alphas, batch_size, gamma,
@@ -64,7 +56,7 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
                _lib.lib().default_mlp_impl())
         opt = _arena.FlatAdam.attach(critic_optimizer, agent._critic_arena)
 
-        enc_trained = _encoder_trainable(agent)
+        enc_trained = lu._encoder_trainable(agent)
 
         def on_replay():
             opt.note_replayed_step()
@@ -102,17 +94,12 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
     S, A = lu._dims(agent)
     # Software pipelining across consecutive updates (lu.pipelined_updates): the target side of this update runs on the
     # front stream, which is NOT joined at the end of the update -- the next update's target side starts next to this
-    # update's backward / Adam.  One member, plain Bellman weights, uniform sampling, no trainable encoder.
-    pipe = lu.pipeline()
+    # update's backward / Adam.
     # Critics sharded over ranks: the exchange of the target values (put + wait, parallel.all_gather_q) belongs to the target
     # side and moves to the front stream with it -- its round trip over NVLink then runs under the previous update's
     # backward.  Both halves of an exchange site stay safe: put(k+2) follows wait(k+1) on the front stream, and a peer's
-    # put(k+1) follows ITS wait(k), so nobody still reads the half that put(k+2) overwrites.  (NCCL fallback: serial.)
-    if pipe is not None and (E != 1 or per or update_priorities or weight_type is not None or _encoder_trainable(agent) or
-                             (parallel.is_sharded() and not parallel.peer_exchange_ready()) or parallel.members_sharded() or
-                             lu.side_stream(dev) is None or pipe.device != dev):
-        lu.pipeline_barrier()
-        pipe = None
+    # put(k+1) follows ITS wait(k), so nobody still reads the half that put(k+2) overwrites.
+    pipe = lu._critic_pipeline(agent, per, update_priorities, weight_type)
     # (the log buffer is cleared by the first member's draw kernel, i.e. on the front stream when pipelined: it then has to
     # come from that stream's allocator pool -- a block recycled from the caller's stream could still be in use by the
     # previous update's backward -- and must not be recycled before the block ends)
@@ -133,21 +120,22 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
     lu._mark("start")
     En = parallel.members_global(E)   # loss normalisation: the global ensemble size when members are sharded over ranks
     presampled, q_weights = None, None
+
+    def draw_member():
+        draws = lu.draw_for_critic_member(buffer, agent, B, target_critic_ensemble_n, random_process, per,
+                                          zero=logs.take_unzeroed())
+        lu._mark("draws (indices, eps, subset)")
+        return draws, lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix,
+                                                 per=per, _idx=draws["idx"])
+
     if parallel.members_sharded() and weight_type is not None and weighted_bellman_temp is not None and En > 1:
         if weight_type != "sunrise":
             raise NotImplementedError("member-sharded ensembles exchange the sunrise weights only")
         # every local member samples first; then ONE exchange: all batches to all ranks, every rank's target critics on
         # every batch, the values back (parallel.py)
-        presampled = []
-        for i in range(E):
-            draws = lu.draw_for_critic_member(buffer, agent, B, target_critic_ensemble_n, random_process, per,
-                                              zero=logs.take_unzeroed())
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per,
-                                            _idx=draws["idx"])
-            pk = lu._packed_of(rd)
-            if pk is None:
-                raise NotImplementedError("member-sharded sunrise weights need state observations (packed batches)")
-            presampled.append((draws, rd))
+        presampled = [draw_member() for _ in range(E)]
+        if any(lu._packed_of(rd) is None for _, rd in presampled):
+            raise NotImplementedError("member-sharded sunrise weights need state observations (packed batches)")
         x_all = parallel.all_gather_members(torch.stack([lu._packed_of(rd)["XA"] for _, rd in presampled]))   # [En,B,S+A]
         q_loc = torch.stack([lu._critic_values(target_agent, 0, E * N, x_all[e].contiguous(), B).reshape(E * N, B)
                              for e in range(En)], dim=1)                                                    # [E*N,En,B]
@@ -156,17 +144,10 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
     # Members are independent once their batches are drawn (the draws share one device-side Philox offset and stay in
     # order): with more than one member each runs on its own stream lane, forked from / joined into the caller's stream.
     # (softmax weights draw policy samples inside the member's work: those stay serial, in the reference's draw order)
-    concurrent = (E > 1 and not per and lu.side_stream(dev) is not None and not _encoder_trainable(agent)
+    concurrent = (E > 1 and not per and lu.side_stream(dev) is not None and not lu._encoder_trainable(agent)
                   and weight_type != "softmax")
     if concurrent and presampled is None:
-        presampled = []
-        for i in range(E):
-            draws = lu.draw_for_critic_member(buffer, agent, B, target_critic_ensemble_n, random_process, per,
-                                              zero=logs.take_unzeroed())
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per,
-                                            _idx=draws["idx"])
-            presampled.append((draws, rd))
-    replay_dicts = [None] * E
+        presampled = [draw_member() for _ in range(E)]
 
     def member_step(i, draws, rd, lane, batch_ready=None):
         loss_v = loss_all[2 * i:2 * i + 2]
@@ -207,7 +188,7 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
                                   h2.data_ptr(), None, None, None, None, None, 0, En, 0, None, None, 1,
                                   None, 0, None, None, None, None, 0.0, None, None, 0, online.cuda_stream)
             if split_bwd:
-                L.mlp_backward_pre(W2, W3, N, ca.H, B, h1.data_ptr(), h2.data_ptr(), bws.data_ptr(), _U_ASYNC, 0, online.cuda_stream)
+                L.mlp_backward_pre(W2, W3, N, ca.H, B, h1.data_ptr(), h2.data_ptr(), bws.data_ptr(), 1, 0, online.cuda_stream)
         with (torch.cuda.stream(pipe.front) if piped else contextlib.nullcontext()):
             td_target, (s1, a1) = lu.compute_td_targets(
                 logs=logs, replay_dict=rd, agent=agent, target_agent=target_agent, log_alphas=log_alphas, ensemble_idx=i,
@@ -274,81 +255,52 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
                               want_dw=True, accumulate=True)
         if need_ds:
             enc_outs.append((s_rep, dxg.sum(0)[:, :S]))
-        replay_dicts[i] = rd
         lu._mark("ensemble backward")
+        return rd
 
-
-    caller = torch.cuda.current_stream(dev)
-    lanes = []
-    for i in range(E):
+    def run_member(i):
         if presampled is not None:
             draws, rd = presampled[i]
         elif pipe is not None:
             with torch.cuda.stream(pipe.front):
-                draws = lu.draw_for_critic_member(buffer, agent, B, target_critic_ensemble_n, random_process, per,
-                                                  zero=logs.take_unzeroed())
-                rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per,
-                                                _idx=draws["idx"])
+                draws, rd = draw_member()
                 pipe.cross_after_gather()
                 batch_ready = torch.cuda.Event()
                 batch_ready.record(pipe.front)
-            member_step(i, draws, rd, 0, batch_ready)
-            continue
+            return member_step(i, draws, rd, 0, batch_ready)
         else:
-            draws = lu.draw_for_critic_member(buffer, agent, B, target_critic_ensemble_n, random_process, per,
-                                              zero=logs.take_unzeroed())
-            lu._mark("draws (indices, eps, subset)")
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per,
-                                            _idx=draws["idx"])
-        if concurrent:
-            lane = i % lu.MEMBER_LANES
-            st = lu.member_stream(dev, lane)
-            if st not in lanes:
-                lanes.append(st)
-                st.wait_stream(caller)
-            with torch.cuda.stream(st):
-                member_step(i, draws, rd, lane)
-        else:
-            member_step(i, draws, rd, 0)
-    for st in lanes:
-        caller.wait_stream(st)
+            draws, rd = draw_member()
+        return member_step(i, draws, rd, i % lu.MEMBER_LANES if concurrent else 0)
 
-    encoder_optimizer.zero_grad()
-    if enc_outs:
-        torch.autograd.backward([s for s, _ in enc_outs], [g for _, g in enc_outs])
+    replay_dicts = lu._run_members(E, dev, concurrent, run_member)
+    logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)
+    logs.defer("losses/critic_overall_loss", [loss_slot + 2 * i for i in range(E)])
+
+    enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
     if critic_clip:
         opt.grad_norm_sq(stream)
         if parallel.is_sharded():   # the global norm runs over every rank's critics (SURVEY 8e (3)): one float per rank
             parallel.all_reduce_sum_(opt.gnorm_sq, site="critic_gnorm")
-    enc_net = None
-    if enc_outs:
-        # a native pixel encoder whose gradients sit in its flat buffer: clip + Adam as two launches (_encoder_opt.py)
-        enc_net = _encoder_opt.fused_step(agent.encoder, encoder_optimizer, encoder_clip)
-        if enc_net is None:
-            if encoder_clip:
-                torch.nn.utils.clip_grad_norm_(agent.encoder.parameters(), encoder_clip)
-            encoder_optimizer.step()
-    member = random.choice(range(E))
+    main = torch.cuda.current_stream(dev)
     side = None if critic_clip else lu.side_stream(dev)   # clipping rescales the gradients that get logged
     if side is not None:
         # logged gradient norm next to Adam (which only reads the gradients)
-        main = torch.cuda.current_stream(dev)
         side.wait_stream(main)
-        gslot = lu._member_grad_norm_slot(logs, ca, member * N, (member + 1) * N, stream=side)
-    if parallel.is_sharded() and side is not None:
-        # each rank summed its own critics: the logged loss is the global sum -- a log value, so its exchange runs next to
-        # Adam on the second stream instead of behind it
-        with torch.cuda.stream(side):
-            parallel.all_reduce_sum_(loss_all[0:1], site="critic_loss")
+        lu._log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad", stream=side)
+        if parallel.is_sharded():
+            # each rank summed its own critics: the logged loss is the global sum -- a log value, so its exchange runs
+            # next to Adam on the second stream instead of behind it
+            with torch.cuda.stream(side):
+                parallel.all_reduce_sum_(loss_all[0:1], site="critic_loss")
     if pipe is not None:
-        pipe.main_wait_polyak(torch.cuda.current_stream(dev))   # a Polyak step on the auxiliary stream still reads these
+        pipe.main_wait_polyak(main)   # a Polyak step on the auxiliary stream still reads these
     opt.step(stream, max_norm=critic_clip if critic_clip else None)
     if pipe is not None:
-        pipe.cross_after_adam(torch.cuda.current_stream(dev))
+        pipe.cross_after_adam(main)
     if side is not None:
         main.wait_stream(side)
     else:
-        gslot = lu._member_grad_norm_slot(logs, ca, member * N, (member + 1) * N)
+        lu._log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad")
         if parallel.is_sharded():
             parallel.all_reduce_sum_(loss_all[0:1], site="critic_loss")
     lu._mark("Adam (+ logged grad norm)")
@@ -358,20 +310,9 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         parallel.all_reduce_members_(tot)
         loss_all[0:2 * E:2].zero_()
         loss_all[0:1].copy_(tot)
-    logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)
-    logs.defer("losses/critic_overall_loss", [loss_slot + 2 * i for i in range(E)])
-    logs.defer("gradients/critic_random_grad", gslot, transform=lambda v: v**0.5)
-    if enc_net is not None:
-        v, eslot = logs.slots(1)
-        _encoder_opt.grad_norm_sq_into(enc_net, v)
-        logs.defer("gradients/encoder_criticloss_grad_norm", eslot, transform=lambda v: v**0.5)
-    elif enc_outs:
-        gn = torch.linalg.vector_norm(torch.stack([p.grad.norm() for p in agent.encoder.parameters() if p.grad is not None]))
-        logs.put_tensor("gradients/encoder_criticloss_grad_norm", gn)
-    else:
-        logs["gradients/encoder_criticloss_grad_norm"] = 0.0
+    lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_criticloss_grad_norm")
     if update_priorities:
-        lu.adjust_priorities(logs, rd, agent, buffer)
+        lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)
     return logs.finalize(), replay_dicts
 
 
@@ -431,7 +372,9 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
 
     predrawn = [draw_member() for _ in range(E)] if concurrent else None
 
-    def member_step(i, rd, eps, noise):
+    def member_step(i):
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per)
+        eps, noise = predrawn[i] if concurrent else (None, None)
         loss_v = loss_all[i:i + 1]
         o, *_ = rd["primary_batch"]
         packed = lu._packed_of(rd)
@@ -481,70 +424,22 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
                                    log_alphas[i].data_ptr(), dout.data_ptr(), _lib.stream_ptr())
         _ops.mlp_backward(aa, i, 1, XPI, B, pol["h1"], pol["h2"], dout, ldx=S + A, want_dw=True, accumulate=False)
 
-    caller = torch.cuda.current_stream(dev)
-    lanes = []
-    for i in range(E):
-        if premade_replay_dicts is not None:
-            rd = premade_replay_dicts[i]
-        else:
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
-        if concurrent:
-            st = lu.member_stream(dev, i % lu.MEMBER_LANES)
-            if st not in lanes:
-                lanes.append(st)
-                st.wait_stream(caller)
-            with torch.cuda.stream(st):
-                member_step(i, rd, *predrawn[i])
-        else:
-            member_step(i, rd, None, None)
-    for st in lanes:
-        caller.wait_stream(st)
+    lu._run_members(E, dev, concurrent, member_step)
     if clip:
         opt.grad_norm_sq(stream)
     opt.step(stream, max_norm=clip if clip else None)
-    member = random.choice(range(E))
-    gslot = lu._member_grad_norm_slot(logs, aa, member, member + 1)
-    logs.defer("gradients/random_actor_online_grad", gslot, transform=lambda v: v**0.5)
+    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/random_actor_online_grad")
     logs.defer("losses/actor_pg_loss", [loss_slot + i for i in range(E)])
     return logs.finalize()
-
-
-class _AlphaState:
-    """Adam state of one 1-element ``log_alpha`` optimiser (main.py:230-239), kept on the device."""
-
-    def __init__(self, optimizer, log_alpha):
-        self.state = torch.zeros(2, dtype=torch.float32, device=log_alpha.device)
-        self.ctl = torch.zeros(2, dtype=torch.int32, device=log_alpha.device)
-        st = optimizer.state[log_alpha]
-        self._step_tensor = torch.zeros((), dtype=torch.float32)
-        self.steps = 0
-        if "exp_avg" in st:   # resuming from a loaded optimizer state (optimizer.load_state_dict)
-            self.state[0:1].copy_(st["exp_avg"].reshape(1))
-            self.state[1:2].copy_(st["exp_avg_sq"].reshape(1))
-            self.steps = int(st["step"])
-            self.ctl[0] = self.steps
-            self._step_tensor.fill_(self.steps)
-        st["step"], st["exp_avg"], st["exp_avg_sq"] = self._step_tensor, self.state[0:1], self.state[1:2]
-
-    @classmethod
-    def attach(cls, optimizer, log_alpha):
-        cur = getattr(optimizer, "_ssac_alpha_state", None)
-        st = optimizer.state.get(log_alpha)
-        aliased = st is not None and "exp_avg" in st and cur is not None and st["exp_avg"].data_ptr() == cur.state.data_ptr()
-        if cur is None or cur.state.device != log_alpha.device or not aliased:   # not aliased: load_state_dict replaced the state
-            cur = cls(optimizer, log_alpha)
-            optimizer._ssac_alpha_state = cur
-        return cur
 
 
 def alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, aug_mix, target_entropy,
                  premade_replay_dicts, discrete):
     if discrete:   # learning.py:252-253
         return _discrete.alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, aug_mix, target_entropy,
-                                      premade_replay_dicts, _AlphaState)
+                                      premade_replay_dicts)
     lu.pipeline_barrier()
     dev = agent._actor_arena.device
-    L, stream = _lib.lib(), _lib.stream_ptr()
     E, B = agent.ensemble_size, batch_size
     S, A = lu._dims(agent)
     logs = _logs.DeviceLogs(dev)
@@ -558,42 +453,17 @@ def alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, a
             _rng.source().normal(eps)
             predrawn.append(eps)
 
-    def member_step(i, rd, eps):
+    def member_step(i):
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, False)
         o, *_ = rd["primary_batch"]
         with torch.no_grad():
             s_rep = agent.encoder(o)
         X = torch.empty((B, S + A), dtype=torch.float32, device=dev)
         X[:, :S].copy_(s_rep)
-        pol = lu._policy_sample(agent, i, X, B, S, A, None, None, eps=eps)
-        pg = optimizers[i].param_groups[0]
-        st = _AlphaState.attach(optimizers[i], log_alphas[i])
-        lv, slot = logs.slots(2)
-        L.alpha_step(log_alphas[i].data_ptr(), pol["logp"].data_ptr(), B, float(target_entropy), st.state.data_ptr(),
-                     st.ctl.data_ptr(), float(pg["lr"]), float(pg["betas"][0]), float(pg["betas"][1]), float(pg["eps"]),
-                     lv.data_ptr(), _lib.stream_ptr())
-        st.steps += 1
-        st._step_tensor.fill_(st.steps)
-        logs.defer(f"losses/alpha_loss_{i}", slot)
-        logs.defer(f"alphas/alpha_{i}", slot + 1)
+        pol = lu._policy_sample(agent, i, X, B, S, A, None, None, eps=predrawn[i] if predrawn is not None else None)
+        lu._alpha_step(logs, i, optimizers[i], log_alphas[i], pol["logp"], B, target_entropy)
 
-    caller = torch.cuda.current_stream(dev)
-    lanes = []
-    for i in range(E):
-        if premade_replay_dicts is not None:
-            rd = premade_replay_dicts[i]
-        else:
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, per=False, aug_mix=aug_mix)
-        if concurrent:
-            lane = lu.member_stream(dev, i % lu.MEMBER_LANES)
-            if lane not in lanes:
-                lanes.append(lane)
-                lane.wait_stream(caller)
-            with torch.cuda.stream(lane):
-                member_step(i, rd, predrawn[i] if predrawn is not None else None)
-        else:
-            member_step(i, rd, None)
-    for lane in lanes:
-        caller.wait_stream(lane)
+    lu._run_members(E, dev, concurrent, member_step)
     return logs.finalize()
 
 
@@ -620,11 +490,9 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
     opt = _arena.FlatAdam.attach(actor_optimizer, aa)
     total = torch.zeros(1, dtype=torch.float32, device=dev)
     enc_outs = []
-    for i in range(E):
-        if premade_replay_dicts is not None:
-            rd = premade_replay_dicts[i]
-        else:
-            rd = lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
+
+    def member_step(i):
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per)
         o, a, *_ = rd["primary_batch"]
         if filter_:
             _, mask, _ = lu._advantage(agent, rd, i)
@@ -648,35 +516,24 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
                               float(agent.log_std_high), logp.data_ptr(), dlogp.data_ptr(), dout.data_ptr(), stream)
         member_loss = -(logp * mask).mean()
         logs.put_tensor(f"losses/filterd_bc_loss_{i}", member_loss)
-        total += member_loss / E
+        total.add_(member_loss / E)
         dxg = torch.empty((1, B, S + A), dtype=torch.float32, device=dev) if need_ds else None
         _ops.mlp_backward(aa, i, 1, X, B, h1, h2, dout, ldx=S + A, want_dw=True, accumulate=False, dx=dxg, lddx=S + A)
         if need_ds:
             enc_outs.append((s_rep, dxg[0, :, :S]))
-    encoder_optimizer.zero_grad()
-    if enc_outs:
-        torch.autograd.backward([s for s, _ in enc_outs], [g for _, g in enc_outs])
+        return rd
+
+    replay_dicts = lu._run_members(E, dev, False, member_step)
+    # (s_rep carries gradient only with update_encoder: the same fused clip + Adam as in critic_update)
+    enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
     if actor_clip:
         opt.grad_norm_sq(stream)
-    enc_net = None
-    if update_encoder and enc_outs:   # (the same fused clip + Adam as in critic_update: one optimiser, one kind of state)
-        enc_net = _encoder_opt.fused_step(agent.encoder, encoder_optimizer, encoder_clip)
-    if enc_net is None and encoder_clip and enc_outs:
-        torch.nn.utils.clip_grad_norm_(agent.encoder.parameters(), encoder_clip)
     opt.step(stream, max_norm=actor_clip if actor_clip else None)
-    if enc_net is None and update_encoder and enc_outs:
-        encoder_optimizer.step()
     logs.put_tensor("losses/filtered_bc_overall_loss", total)
-    member = random.choice(range(E))
-    gslot = lu._member_grad_norm_slot(logs, aa, member, member + 1)
-    logs.defer("gradients/actor_offline_grad_norm", gslot, transform=lambda v: v**0.5)
-    if enc_outs:
-        gn = torch.linalg.vector_norm(torch.stack([p.grad.norm() for p in agent.encoder.parameters() if p.grad is not None]))
-        logs.put_tensor("gradients/encoder_offline_actorloss_grad_norm", gn)
-    else:
-        logs["gradients/encoder_offline_actorloss_grad_norm"] = 0.0
+    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/actor_offline_grad_norm")
+    lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_offline_actorloss_grad_norm")
     if per:
-        lu.adjust_priorities(logs, rd, agent, buffer)
+        lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)
     return logs.finalize()
 
 

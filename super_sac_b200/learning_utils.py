@@ -12,7 +12,8 @@ import random
 import numpy as np
 import torch
 
-from . import _lib, _logs, _ops, _rng, augmentations, graphed, parallel
+# (discrete.py imports this module as well: the two use each other only inside functions, never at import time)
+from . import _encoder_opt, _lib, _logs, _ops, _rng, augmentations, discrete as _discrete, graphed, parallel
 from ._arena import MLPArena
 
 LOG_SQRT_2PI = math.log(math.sqrt(2 * math.pi))
@@ -240,6 +241,9 @@ class _Pipeline:
         self.cross = graphed.cross_capturing()   # (state, slot): this block is ONE update captured for cross-call pipelining
         self.keep = []           # front-allocated tensors that main-stream kernels read: alive until the block ends
         self.needs_order = False  # a barrier happened: the front's next work goes behind the caller's stream as it is then
+        # the front has waited on the caller's stream once: before that it holds no work of this block, and under capture
+        # waiting on it would be a dependency on work outside the graph (a block whose critic updates all run serially)
+        self.forked = False
 
     def order_front_after_main(self, main):
         ev = torch.cuda.Event()
@@ -253,6 +257,7 @@ class _Pipeline:
         if self.dep is not None:
             self.front.wait_event(self.dep)
             self.dep = None
+            self.forked = True
             if self.cross is not None:   # one Philox stream, one set of ring readers: behind the other capture's target side
                 X, i = self.cross
                 self.front.wait_event(X.gather_done[1 - i])
@@ -351,7 +356,8 @@ def pipelined_updates(device=None):
     finally:
         _pipeline = None
         main = torch.cuda.current_stream(device)
-        main.wait_stream(p.front)
+        if p.forked:
+            main.wait_stream(p.front)
         if p.aux is not None:
             main.wait_stream(p.aux)
         p.keep.clear()
@@ -365,7 +371,8 @@ def pipeline_barrier():
         graphed.join()
     if p is not None:
         main = torch.cuda.current_stream(p.device)
-        main.wait_stream(p.front)
+        if p.forked:
+            main.wait_stream(p.front)
         if p.aux is not None:
             main.wait_stream(p.aux)
             p.polyak_main = None
@@ -660,6 +667,133 @@ def _dims(agent):
     return agent._actor_arena.D, agent.act_space_size
 
 
+def _encoder_trainable(agent):
+    ps = agent.__dict__.get("_ssac_encoder_params")
+    if ps is None:   # walking the module tree on every update call costs more than the check itself
+        ps = agent.__dict__["_ssac_encoder_params"] = [p for p in agent.encoder.parameters() if p.numel() > 2]
+    return any(p.requires_grad for p in ps)
+
+
+def _critic_pipeline(agent, per, update_priorities, weight_type):
+    """The active ``pipelined_updates()`` block if this critic update may run its target side on the block's front stream
+    (one member, uniform sampling, plain Bellman backups, no trainable encoder, no PopArt), else None after joining the
+    front stream.  PopArt stays serial: the next update's TD target rescales the PopArt layer this update's loss seed
+    still reads.  Critics sharded over ranks pipeline only over the peer exchange (the NCCL fallback stays serial)."""
+    p, dev = _pipeline, agent._critic_arena.device
+    if (p is None or agent.ensemble_size != 1 or per or update_priorities or weight_type is not None
+            or _encoder_trainable(agent) or any(bool(pa) for pa in agent.popart)
+            or (parallel.is_sharded() and not parallel.peer_exchange_ready()) or parallel.members_sharded()
+            or side_stream(dev) is None or p.device != dev):
+        pipeline_barrier()
+        return None
+    return p
+
+
+def _member_replay_dict(premade_replay_dicts, i, buffer, batch_size, augmenter, aug_mix, per):
+    """Member i's batch: the one the caller made (the critic update's replay dicts) or a fresh sample."""
+    if premade_replay_dicts is not None:
+        return premade_replay_dicts[i]
+    return sample_move_and_augment(buffer=buffer, batch_size=batch_size, augmenter=augmenter, aug_mix=aug_mix, per=per)
+
+
+def _run_members(E, device, concurrent, member_step):
+    """[member_step(i) for every member i], in order.  ``concurrent``: member i runs on stream lane i % MEMBER_LANES,
+    forked from the caller's stream, and every lane used is joined back into it afterwards."""
+    if not concurrent:
+        return [member_step(i) for i in range(E)]
+    caller = torch.cuda.current_stream(device)
+    lanes, out = [], []
+    for i in range(E):
+        st = member_stream(device, i % MEMBER_LANES)
+        if st not in lanes:
+            lanes.append(st)
+            st.wait_stream(caller)
+        with torch.cuda.stream(st):
+            out.append(member_step(i))
+    for st in lanes:
+        caller.wait_stream(st)
+    return out
+
+
+def _encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs):
+    """Hand the members' input gradients ``enc_outs`` [(s_rep, ds)] to autograd and clip + step the encoder (learning.py:
+    117-131).  A native pixel encoder whose gradients sit in its flat buffer takes the fused sumsq + Adam launches
+    (_encoder_opt.py); that net is returned, else None."""
+    encoder_optimizer.zero_grad()
+    if not enc_outs:
+        return None
+    torch.autograd.backward([s for s, _ in enc_outs], [g for _, g in enc_outs])
+    net = _encoder_opt.fused_step(agent.encoder, encoder_optimizer, encoder_clip)
+    if net is None:
+        if encoder_clip:
+            torch.nn.utils.clip_grad_norm_(agent.encoder.parameters(), encoder_clip)
+        encoder_optimizer.step()
+    return net
+
+
+def _log_member_grad_norm(logs, arena, E, nets_per_member, key, stream=None):
+    """Log the gradient norm of one member picked by ``random.choice`` (the reference's draw: it precedes the one in
+    adjust_priorities)."""
+    member = random.choice(range(E))
+    slot = _member_grad_norm_slot(logs, arena, member * nets_per_member, (member + 1) * nets_per_member, stream=stream)
+    logs.defer(key, slot, transform=lambda v: v**0.5)
+
+
+def _log_encoder_grad_norm(logs, agent, enc_net, enc_outs, key):
+    """Log the encoder's (post-clip) gradient norm, 0.0 when no gradient reached it."""
+    if enc_net is not None:
+        v, slot = logs.slots(1)
+        _encoder_opt.grad_norm_sq_into(enc_net, v)
+        logs.defer(key, slot, transform=lambda v: v**0.5)
+    elif enc_outs:
+        gn = torch.linalg.vector_norm(torch.stack([p.grad.norm() for p in agent.encoder.parameters() if p.grad is not None]))
+        logs.put_tensor(key, gn)
+    else:
+        logs[key] = 0.0
+
+
+class _AlphaState:
+    """Adam state of one 1-element ``log_alpha`` optimiser (main.py:230-239), kept on the device."""
+
+    def __init__(self, optimizer, log_alpha):
+        self.state = torch.zeros(2, dtype=torch.float32, device=log_alpha.device)
+        self.ctl = torch.zeros(2, dtype=torch.int32, device=log_alpha.device)
+        st = optimizer.state[log_alpha]
+        self._step_tensor = torch.zeros((), dtype=torch.float32)
+        self.steps = 0
+        if "exp_avg" in st:   # resuming from a loaded optimizer state (optimizer.load_state_dict)
+            self.state[0:1].copy_(st["exp_avg"].reshape(1))
+            self.state[1:2].copy_(st["exp_avg_sq"].reshape(1))
+            self.steps = int(st["step"])
+            self.ctl[0] = self.steps
+            self._step_tensor.fill_(self.steps)
+        st["step"], st["exp_avg"], st["exp_avg_sq"] = self._step_tensor, self.state[0:1], self.state[1:2]
+
+    @classmethod
+    def attach(cls, optimizer, log_alpha):
+        cur = getattr(optimizer, "_ssac_alpha_state", None)
+        st = optimizer.state.get(log_alpha)
+        aliased = st is not None and "exp_avg" in st and cur is not None and st["exp_avg"].data_ptr() == cur.state.data_ptr()
+        if cur is None or cur.state.device != log_alpha.device or not aliased:   # not aliased: load_state_dict replaced the state
+            cur = cls(optimizer, log_alpha)
+            optimizer._ssac_alpha_state = cur
+        return cur
+
+
+def _alpha_step(logs, i, optimizer, log_alpha, logp, B, target_entropy):
+    """Member i's temperature step (learning.py:246-262) on ``logp`` [B]: loss, scalar Adam and logs in one launch."""
+    pg = optimizer.param_groups[0]
+    st = _AlphaState.attach(optimizer, log_alpha)
+    lv, slot = logs.slots(2)
+    _lib.lib().alpha_step(log_alpha.data_ptr(), logp.data_ptr(), B, float(target_entropy), st.state.data_ptr(),
+                          st.ctl.data_ptr(), float(pg["lr"]), float(pg["betas"][0]), float(pg["betas"][1]),
+                          float(pg["eps"]), lv.data_ptr(), _lib.stream_ptr())
+    st.steps += 1
+    st._step_tensor.fill_(st.steps)
+    logs.defer(f"losses/alpha_loss_{i}", slot)
+    logs.defer(f"alphas/alpha_{i}", slot + 1)
+
+
 def draw_for_critic_member(buffer, agent, B, ensemble_n, random_process, per, zero=None):
     """Every random draw one member's critic update consumes up front -- replay indices (replay.py:122), the policy's
     N(0,1) draw or the TD3 noise (learning_utils.py:49,330), the REDQ target subset (agent.py:29) -- in ONE launch."""
@@ -683,12 +817,8 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
     reduction is left to the critic loss kernel -- the returned tensor is filled by that launch and carries the operands
     as ``_ssac_pending``."""
     if discrete:   # learning_utils.py:322-328
-        from . import discrete as _discrete
-
         return _discrete.compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ensemble_n, log_alphas, pop,
                                             gamma)
-    if discrete:
-        raise NotImplementedError("discrete actions are out of scope")
     dlogs, user_logs = _logs.as_device_logs(logs, agent._critic_arena.device)
     o, a, r, o1, d = replay_dict["primary_batch"]
     i = ensemble_idx
@@ -757,8 +887,6 @@ def compute_backup_weights(logs, replay_dict, agent, target_agent, weight_type, 
     if weight_type is None or weight_temp is None or parallel.members_global(agent.ensemble_size) == 1:
         return 1.0
     if discrete:   # learning_utils.py:373-376
-        from . import discrete as _discrete
-
         return _discrete.compute_backup_weights(logs, replay_dict, agent, target_agent, weight_type, weight_temp, batch_size)
     dlogs, user_logs = _logs.as_device_logs(logs, agent._critic_arena.device)
     o, a, _, o1, _ = replay_dict["primary_batch"]
@@ -802,8 +930,6 @@ def _advantage(agent, replay_dict, ensemble_idx, n=4, want_priority=False):
     """A(s,a) = Q(s,a) - mean_n Q(s, a'~pi) with min-over-N critics and PopArt (reference adv_estimator.py:58-79).
     Returns (adv [B], mask [B], priority float64 [B] or None)."""
     if agent.discrete:   # adv_estimator.py:45-56 ('indirect')
-        from . import discrete as _discrete
-
         return _discrete._advantage(agent, replay_dict, ensemble_idx, want_priority=want_priority)
     o, a, *_ = replay_dict["primary_batch"]
     i = ensemble_idx

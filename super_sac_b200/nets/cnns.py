@@ -48,7 +48,7 @@ class _EncoderFn(torch.autograd.Function):
         O = module.embedding_dim
         save = 1 if any(ctx.needs_input_grad[2:]) else 0
         # (one workspace per shape: every update path that may run encoders on several streams at once -- member lanes,
-        # pipelined blocks -- excludes agents with a parameterised encoder, learning._encoder_trainable)
+        # pipelined blocks -- excludes agents with a parameterised encoder, learning_utils._encoder_trainable)
         key = (B, C, H, W, save, obs.device)
         n = ctypes.c_int64()
         lib.conv_encoder_ws_floats(B, C, H, W, O, save, ctypes.byref(n))

@@ -488,11 +488,14 @@ def test_cross_call_pipelined_updates_equal_eager(shape):
             gu.assert_close(float(y[key]), float(x[key]), 1e-5, 1e-7, f"step {k} log {key}")
 
 
-@pytest.mark.parametrize("captured", [False, True], ids=["eager", "graph"])
-def test_pipelined_update_block_equals_sequential(captured):
+@pytest.mark.parametrize("captured,pop", [(False, False), (True, False), (False, True), (True, True)],
+                         ids=["eager", "graph", "eager-popart", "graph-popart"])
+def test_pipelined_update_block_equals_sequential(captured, pop):
     """lu.pipelined_updates(): the target side of update k+1 runs next to update k's backward / Adam on its own stream.
     Same kernels, same draw order, event-ordered where data flows => a block of UTD updates (+ Polyak every 2nd, + one
-    actor and one temperature update, as main.py:380-543 runs them) must reproduce the sequential schedule bit for bit."""
+    actor and one temperature update, as main.py:380-543 runs them) must reproduce the sequential schedule bit for bit.
+    With PopArt the critic updates take the serial schedule inside the block (the next TD target rescales the PopArt
+    layer this update's loss seed still reads)."""
     import copy
     from itertools import chain
 
@@ -505,7 +508,7 @@ def test_pipelined_update_block_equals_sequential(captured):
         torch.manual_seed(5)
         agent = ssb.Agent(act_space_size=6, encoder=cu.IdentityEncoder(17), actor_network_cls=nets.mlps.ContinuousStochasticActor,
                           critic_network_cls=nets.mlps.ContinuousCritic, ensemble_size=1, num_critics=10, hidden_size=256,
-                          auto_rescale_targets=False, log_std_low=-5.0, log_std_high=2.0)
+                          auto_rescale_targets=pop, log_std_low=-5.0, log_std_high=2.0)
         agent.to("cuda")
         target = copy.deepcopy(agent)
         rng = np.random.default_rng(0)
@@ -528,12 +531,12 @@ def test_pipelined_update_block_equals_sequential(captured):
                     logs, rds = learning._critic_update_impl(
                         buffer=buf, agent=agent, target_agent=target, critic_optimizer=c_opt, encoder_optimizer=e_opt,
                         log_alphas=la, batch_size=256, gamma=0.99, critic_clip=None, encoder_clip=None,
-                        target_critic_ensemble_n=2, weighted_bellman_temp=None, weight_type=None, pop=False, augmenter=aug,
+                        target_critic_ensemble_n=2, weighted_bellman_temp=None, weight_type=None, pop=pop, augmenter=aug,
                         encoder_lambda=0.0, random_process=None, noise_clip=None, aug_mix=0.0)
                     if k % 2 == 0:
                         lu.soft_update(target.critics[0], agent.critics[0], 0.005)
                 learning._online_actor_update_impl(
-                    buffer=buf, agent=agent, pop=False, actor_optimizer=a_opt, log_alphas=la, batch_size=256, clip=None,
+                    buffer=buf, agent=agent, pop=pop, actor_optimizer=a_opt, log_alphas=la, batch_size=256, clip=None,
                     random_process=None, noise_clip=None, augmenter=aug, aug_mix=0.0, premade_replay_dicts=rds)
                 learning.alpha_update(buffer=buf, agent=agent, optimizers=al_opt, batch_size=256, log_alphas=la, augmenter=aug,
                                       aug_mix=0.0, target_entropy=-6.0, premade_replay_dicts=rds, discrete=False)
@@ -563,6 +566,10 @@ def test_pipelined_update_block_equals_sequential(captured):
     assert torch.equal(t0._critic_arena.flat, t1._critic_arena.flat)
     assert torch.equal(a0._actor_arena.flat, a1._actor_arena.flat)
     assert torch.equal(la0[0], la1[0])
+    for p0, p1 in zip(a0.popart, a1.popart):
+        assert bool(p0) == bool(p1) == pop
+        if pop:
+            assert torch.equal(p0._state, p1._state) and torch.equal(p0._ctl, p1._ctl)
     assert set(l0.keys()) == set(l1.keys())
     for k in l0:
         gu.assert_close(float(l1[k]), float(l0[k]), 1e-5, 1e-7, f"log {k}")
