@@ -882,12 +882,13 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
 def compute_backup_weights(logs, replay_dict, agent, target_agent, weight_type, weight_temp, batch_size, discrete=False,
                            _q_all=None):
     """SUNRISE / softmax weighted Bellman backups (reference learning_utils.py:357-398).  Returns 1.0 or w [B,1].
-    ``_q_all`` [E_global*N, B, 1]: the target critics' values on this member's batch, already gathered over the ranks
-    (member-sharded ensembles, parallel.enable_member_sharding)."""
+    ``_q_all`` [E_global*N, B, 1] ([E_global*N, B] for discrete agents): the target critics' values on this member's
+    batch, already gathered over the ranks (member-sharded ensembles, parallel.enable_member_sharding)."""
     if weight_type is None or weight_temp is None or parallel.members_global(agent.ensemble_size) == 1:
         return 1.0
     if discrete:   # learning_utils.py:373-376
-        return _discrete.compute_backup_weights(logs, replay_dict, agent, target_agent, weight_type, weight_temp, batch_size)
+        return _discrete.compute_backup_weights(logs, replay_dict, agent, target_agent, weight_type, weight_temp, batch_size,
+                                                _q_sel=_q_all)
     dlogs, user_logs = _logs.as_device_logs(logs, agent._critic_arena.device)
     o, a, _, o1, _ = replay_dict["primary_batch"]
     S, A = _dims(agent)
@@ -971,8 +972,9 @@ def _advantage(agent, replay_dict, ensemble_idx, n=4, want_priority=False):
 
 def adjust_priorities(logs, replay_dict, agent, buffer):
     """priorities <- relu(A(s,a)) + 1e-4 on the sampled rows, without leaving the device
-    (reference learning_utils.py:288-295)."""
-    member = random.choice(range(agent.ensemble_size))
+    (reference learning_utils.py:288-295; critics sharded over ranks with several members: one host broadcast of the
+    member, parallel.same_member_choice)."""
+    member = parallel.same_member_choice(agent.ensemble_size)
     _, _, prio = _advantage(agent, replay_dict, member, want_priority=True)
     buffer.update_priorities(replay_dict["priority_idxs"], prio)
 
@@ -1047,5 +1049,5 @@ def compute_filter_stats(buffer, agent, augmenter, batch_size):
     """Percentage of a uniformly sampled batch that the binary advantage filter accepts (reference
     learning_utils.py:217-238), through the kernel advantage estimator; one scalar read-back."""
     rd = sample_move_and_augment(buffer=buffer, batch_size=batch_size, augmenter=augmenter, aug_mix=0.0, per=False)
-    _, mask, _ = _advantage(agent, rd, random.choice(range(agent.ensemble_size)))
+    _, mask, _ = _advantage(agent, rd, parallel.same_member_choice(agent.ensemble_size))
     return float(mask.mean().item()) * 100.0

@@ -16,6 +16,7 @@ come from torch.distributed._symmetric_memory).  ``torch.distributed`` collectiv
 tests, boxes without peer access) -- ``exchange_name()`` says which one is live.
 """
 import os
+import random
 
 import torch
 import torch.distributed as dist
@@ -134,6 +135,20 @@ def n_global():
 
 def my_range():
     return local_range(_state["n_global"], _state["world"], _state["rank"])
+
+
+def same_member_choice(e):
+    """``random.choice(range(e))`` -- the reference's host draw of the member whose critics rate a batch (priority refresh,
+    filter statistics) -- made the same on every rank when the critics are sharded: the ranks then exchange that
+    member's critic rows, so they must all evaluate the same member, and Python's ``random`` state is not kept in step
+    across ranks.  Every rank draws (its RNG stream advances as unsharded) and rank 0's pick is broadcast: one host round
+    trip, on those eager paths only."""
+    member = random.choice(range(e))
+    if e > 1 and _state["on"]:
+        box = [member]
+        dist.broadcast_object_list(box, group=_state["group"], group_src=0)
+        member = int(box[0])
+    return member
 
 
 def all_gather_q(q_local, site="q", select=None):
