@@ -86,10 +86,11 @@ class DeviceLogs(dict):
         self._pending.append((key, tuple(slots), _Multi(fn)))
 
     def put_tensor(self, key, scalar_tensor, transform=None):
-        """Copy a 0-d / 1-element device tensor into a slot (no sync) and register it under ``key``."""
+        """Copy a 0-d / 1-element device tensor into a slot (no sync) and register it under ``key``; returns the slot."""
         v, s = self.slots(1)
         v.copy_(scalar_tensor.reshape(1))
         self.defer(key, s, transform)
+        return v
 
     def finalize(self):
         if _defer_depth > 0:

@@ -12,27 +12,26 @@ critic update runs on the block's front stream (as in learning._critic_update_im
 with the indirect advantage filter (adv_estimator.py:45-56) and the priority refresh are here too.  Not implemented
 (raise): softmax Bellman weights (they draw Categorical samples), the invariance regularisers.
 
-Sharded ensembles (parallel.py) use the continuous path's exchange sites -- peer stores on GPUs, torch.distributed
-collectives otherwise -- with sites of their own ("dq_*", "members*"):
+Sharded ensembles (parallel.py) exchange through the same sites as the continuous path -- peer stores on GPUs,
+torch.distributed collectives otherwise -- and follow the same rules (learning_utils' shared pieces: global loss
+normalisation, global clip norms, global member ids in the log keys, logged values summed over / taken from the owning
+rank):
 
 - critics over ranks (``enable_critic_sharding``, one member): actor, temperature, PopArt and batch stay replicated.
   The TD target gathers the REDQ subset's target rows [M,B,A] from every rank (on the front stream inside
   ``lu.pipelined_updates()``), the actor update and the advantage filter every rank's online rows [N_global,B,A]; no
-  gradient crosses ranks (the discrete actor loss takes none through the critics).  Losses are normalised by N_global,
-  DR3 and the clip norm are global sums, the logged loss and TD error are the global ones.
-- members over ranks (``enable_member_sharding``): each rank runs its members with E_global in the loss seeds.  The
-  sunrise weights gather every member's batch, run the local target critics over all of them and gather the values back
-  (``_member_target_q``); the offline filter does the same with the actors for the mean policy (``_member_policies``).
-  Logged sums cover every rank's members; per-member keys carry the global member id.
+  gradient crosses ranks (the discrete actor loss takes none through the critics).
+- members over ranks (``enable_member_sharding``): each rank runs its members.  The sunrise weights gather every
+  member's batch, run the local target critics over all of them and gather the values back (``_member_target_q``); the
+  offline filter does the same with the actors for the mean policy (``_member_policies``).
 - the member that rates a batch for the priority refresh / filter statistics (the reference's ``random.choice``) is
   rank 0's draw on every rank when the critics are sharded (parallel.same_member_choice).
-- not covered (raise): both partitionings at once, more than one member in the critic update under critic sharding, an
-  encoder with trainable parameters; with members sharded, the priority refresh, compute_filter_stats and direct
-  advantage-estimator calls.  The logged gradient norms are the rank's own nets'.
+- not covered (raise): more than one member in the critic update under critic sharding, an encoder with trainable
+  parameters; with members sharded, the priority refresh, compute_filter_stats and direct advantage-estimator calls.
 
 Only the member bodies are this module's own.  The skeleton around them -- pipeline eligibility, member batches, the
-member loop, the encoder step, the logged gradient norms and the temperature step -- is learning_utils' "shared pieces
-of the updates", which learning.py uses as well.
+member loop, the encoder step, the logged gradient norms, the temperature step, the DR3 term and the ends of the critic
+and actor updates -- is learning_utils' "shared pieces of the updates", which learning.py uses as well.
 """
 import contextlib
 
@@ -69,40 +68,15 @@ def _actions(a, B):
 def _check(agent):
     if not agent.discrete:
         raise ValueError("discrete=True needs an Agent built with discrete=True")
-    if parallel.is_sharded() and parallel.members_sharded():
-        raise NotImplementedError("critic sharding and member sharding cannot be combined")
-    if (parallel.is_sharded() or parallel.members_sharded()) and lu._encoder_trainable(agent):
+    if parallel.sharded() and lu._encoder_trainable(agent):
         raise NotImplementedError("sharded discrete ensembles need an encoder without trainable parameters: every rank "
                                   "would train its replica on its own share of the gradients and the replicas would drift")
     _ops.check_cuda(agent._critic_arena.flat)
 
 
-def _member_name(i):
-    """Global id of local member i (members sharded over ranks: rank r owns members [lo, hi)), for per-member log keys."""
-    return i + parallel.my_members()[0] if parallel.members_sharded() else i
-
-
 def _global_q(q_local, site):
     """Critics sharded over ranks: this rank's nets' Q rows [n_local, B, A] -> every net's [N_global, B, A]."""
-    return parallel.all_gather_q(q_local, site=site) if parallel.is_sharded() else q_local
-
-
-def _reduce_logged(loss_v, reduce_, td=None, owns_td=False):
-    """Sharded ensembles: the logged loss is the sum of the per-member slots ``loss_v`` over every rank, left in
-    loss_v[0] (the other slots are cleared); ``td``, a slot of the rank that owns the last net, comes from that rank.
-    One exchange of one or two floats."""
-    red = torch.empty(1 if td is None else 2, dtype=torch.float32, device=loss_v.device)
-    torch.sum(loss_v, 0, keepdim=True, out=red[0:1])
-    if td is not None:
-        if owns_td:
-            red[1:2].copy_(td)
-        else:
-            red[1:2].zero_()
-    reduce_(red)
-    loss_v.zero_()
-    loss_v[0:1].copy_(red[0:1])
-    if td is not None:
-        td.copy_(red[1:2])
+    return parallel.all_gather_q(q_local, site=site) if parallel.critics_sharded() else q_local
 
 
 def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ensemble_n, log_alphas, pop, gamma):
@@ -115,7 +89,7 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
     aa, N = agent._actor_arena, agent.num_critics
     A = agent.act_space_size
     # REDQ subset: drawn over the GLOBAL ensemble when the critics are sharded over ranks (replicated Philox state)
-    pool = parallel.n_global() if parallel.is_sharded() else N
+    pool = parallel.n_global(N)
     assert 0 < M <= pool
     L, stream = _lib.lib(), _lib.stream_ptr()
     with torch.no_grad():
@@ -130,11 +104,11 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
     logits = _forward(aa, i, 1, X1, ld1, B)
     if lu.pipeline() is not None:
         lu.pipeline().front_wait_polyak()   # the target critics' parameters: the only thing this side reads that Polyak writes
-    if parallel.is_sharded():
+    if parallel.critics_sharded():
         # every rank evaluates its own target critics and gathers the subset's rows [M,B,A] (in subset order): the state
         # value, the TD target and the PopArt update are then the same on every rank.  Inside lu.pipelined_updates() the
         # put and the wait run on the front stream with the rest of this side.
-        qt = parallel.all_gather_q(_forward(target_agent._critic_arena, i * N, N, X1, ld1, B), site="dq_target",
+        qt = parallel.all_gather_q(_forward(target_agent._critic_arena, i * N, N, X1, ld1, B), site="target_q",
                                    select=subset)
     else:
         qt = _forward(target_agent._critic_arena, i * N, M, X1, ld1, B, net_index=subset)   # [M,B,A]
@@ -150,7 +124,7 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
                 popart.state_ptr() if popart else None, popart.ctl_ptr() if popart else None, int(bool(pop)),
                 float(popart.beta) if popart else 0.0, int(popart.min_steps) if popart else 0, y.data_ptr(), lv.data_ptr(),
                 stream)
-    g = _member_name(i)
+    g = parallel.member_id(i)
     dlogs.defer(f"td_targets/mean_td_target_{g}", slot)
     dlogs.defer(f"td_targets/std_td_target_{g}", slot + 1)
     dlogs.defer(f"td_targets/entropy_bonus_{g}", eslot)
@@ -228,7 +202,7 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
     dev = ca.device
     L, stream = _lib.lib(), _lib.stream_ptr()
     E, N, B, A = agent.ensemble_size, agent.num_critics, batch_size, agent.act_space_size
-    if parallel.is_sharded() and E != 1:
+    if parallel.critics_sharded() and E != 1:
         raise NotImplementedError("critic sharding covers one member (REDQ / SAC shapes); SUNRISE members shard as a whole")
     if parallel.members_sharded() and update_priorities:
         raise NotImplementedError("member-sharded ensembles: the priority refresh needs every actor on the batch")
@@ -238,7 +212,6 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
     # loss normalisation over the GLOBAL ensemble: all members when members are sharded over ranks, all critics when the
     # critics are (each rank then holds a share of the loss and of the DR3 mean; the shares are summed below)
     En = parallel.members_global(E)
-    Ng = parallel.n_global() if parallel.is_sharded() else N
     # Inside lu.pipelined_updates(): the target side (draws, gather, actor logits and target-critic subset on s1, state
     # value, TD target -- and, critics sharded over ranks, the exchange of the target values) runs on the front stream,
     # the online side on the caller's (eligibility: lu._critic_pipeline).
@@ -260,7 +233,7 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
         presampled = [lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix, per=per)
                       for _ in range(E)]
         q_weights = _member_target_q(presampled, target_agent, N, B)
-        g_lo = parallel.my_members()[0]
+        g_lo = parallel.my_range()[0]
 
     def member_step(i):
         loss_v = loss_all[2 * i:2 * i + 2]
@@ -297,24 +270,15 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
             main.wait_event(target_ready)
         L.discrete_critic_loss_seed(q.data_ptr(), N, B, A, act.data_ptr(), td_target.data_ptr(),
                                     w.data_ptr() if torch.is_tensor(w) else None, None if imp is None else imp.data_ptr(),
-                                    popart.state_ptr() if popart else None, int(bool(pop)), En,
-                                    Ng if parallel.is_sharded() else 0, dy.data_ptr(), loss_v.data_ptr(), stream)
+                                    popart.state_ptr() if popart else None, int(bool(pop)), En, parallel.n_global(N),
+                                    dy.data_ptr(), loss_v.data_ptr(), stream)
         extra, extra_scale, f1 = None, 0.0, None
         if dr3_coeff > 0:
-            # DR3 (learning.py:100-108): second forward on s1; both feature sets carry gradient.  The mean runs over the
-            # global ensemble: a rank with sharded critics adds its share N / N_global to the loss, and the logged dot
-            # product is summed over the ranks right here (as learning._critic_update_impl)
+            # DR3 (learning.py:100-108): second forward on s1; both feature sets carry gradient
             X1, ld1 = _rows(s1_rep)
             _, h1b, h2b = _forward(ca, i * N, N, X1, ld1, B, keep=True)
-            dv, dslot = logs.slots(1)
-            L.dr3_dot(h2.data_ptr(), h2b.data_ptr(), N, B, ca.H, dv.data_ptr(), stream)
-            logs.defer(f"dr3_dotproduct_{_member_name(i)}", dslot)
-            if Ng != N:
-                dv.mul_(N / Ng)
-            loss_v[0:1].add_(dv, alpha=dr3_coeff / (En * Ng))
-            if parallel.is_sharded():
-                parallel.all_reduce_sum_(dv, site="dq_dr3")
-            extra, extra_scale, f1 = h2b, dr3_coeff / (En * Ng) / (Ng * B), (X1, ld1, h1b, h2b)
+            extra_scale = lu._dr3_term(logs, ca, i, N, B, E, h2, h2b, dr3_coeff, loss_v)
+            extra, f1 = h2b, (X1, ld1, h1b, h2b)
         dxg = torch.empty((N, B, S), dtype=torch.float32, device=dev) if need_ds else None
         _ops.mlp_backward(ca, i * N, N, X, B, h1, h2, dy, ldx=ld, dh2_extra=extra, extra_scale=extra_scale, want_dw=True,
                           accumulate=False, dx=dxg, lddx=S)
@@ -327,29 +291,8 @@ def critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimiz
         return rd
 
     replay_dicts = lu._run_members(E, dev, False, member_step)
-    logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)
-    logs.defer("losses/critic_overall_loss", [loss_slot + 2 * i for i in range(E)])
-    enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
-    if critic_clip:
-        opt.grad_norm_sq(stream)
-        if parallel.is_sharded():   # the global norm runs over every rank's critics: one float per rank
-            parallel.all_reduce_sum_(opt.gnorm_sq, site="dq_gnorm")
-    if pipe is not None:
-        pipe.main_wait_polyak(main)   # a Polyak step on the block's auxiliary stream still reads the online parameters
-    opt.step(stream, max_norm=critic_clip if critic_clip else None)   # (clipping rescales the stored gradients, as the reference's does)
-    lu._log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad")
-    # the logged loss is the sum over every rank's critics / members, the logged TD error that of the last net of the
-    # last member, which the last rank holds
-    if parallel.is_sharded():
-        _reduce_logged(loss_all[0:1], lambda t: parallel.all_reduce_sum_(t, site="dq_loss"), loss_all[1:2],
-                       parallel.my_range()[1] == parallel.n_global())
-    elif parallel.members_sharded():
-        _reduce_logged(loss_all[0:2 * E:2], parallel.all_reduce_members_, loss_all[2 * E - 1:2 * E],
-                       parallel.my_members()[1] == En)
-    lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_criticloss_grad_norm")
-    if update_priorities:
-        lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)
-    return logs.finalize(), replay_dicts
+    return lu._critic_tail(logs, loss_all, loss_slot, replay_dicts, buffer, agent, opt, pipe, critic_clip, encoder_optimizer,
+                           encoder_clip, enc_outs, update_priorities)
 
 
 def online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_size, clip, augmenter, aug_mix,
@@ -376,7 +319,7 @@ def online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_s
         logits, h1, h2 = _forward(aa, i, 1, X, ld, B, keep=True)
         # [N,B,A]; critics sharded over ranks: every rank's rows gathered.  No gradient flows back through the critics
         # (learning.py:384-387), so nothing else is exchanged: the actor backward and Adam run replicated
-        q = _global_q(_forward(ca, i * N, N, X, ld, B), "dq_actor")
+        q = _global_q(_forward(ca, i * N, N, X, ld, B), "actor_q")
         popart = agent.popart[i]
         dlogits = torch.empty((1, B, A), dtype=torch.float32, device=dev)
         L.discrete_actor_seed(logits.data_ptr(), q.data_ptr(), q.shape[0], B, A, log_alphas[i].data_ptr(),
@@ -385,12 +328,7 @@ def online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_s
         _ops.mlp_backward(aa, i, 1, X, B, h1, h2, dlogits, ldx=ld, want_dw=True, accumulate=False)
 
     lu._run_members(E, dev, False, member_step)
-    if clip:
-        opt.grad_norm_sq(stream)
-    opt.step(stream, max_norm=clip if clip else None)
-    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/random_actor_online_grad")
-    if parallel.members_sharded():   # the logged loss: the sum over every rank's members
-        _reduce_logged(loss_all, parallel.all_reduce_members_)
+    lu._actor_tail(logs, aa, opt, clip, E, "gradients/random_actor_online_grad", loss_all)
     logs.defer("losses/actor_pg_loss", [loss_slot + i for i in range(E)])
     return logs.finalize()
 
@@ -415,7 +353,7 @@ def alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, a
         logits = _forward(aa, i, 1, X, ld, B)
         plogp = torch.empty(B, dtype=torch.float32, device=dev)
         L.discrete_neg_entropy(logits.data_ptr(), B, A, plogp.data_ptr(), stream)
-        lu._alpha_step(logs, _member_name(i), optimizers[i], log_alphas[i], plogp, B, target_entropy)
+        lu._alpha_step(logs, i, optimizers[i], log_alphas[i], plogp, B, target_entropy)
 
     lu._run_members(E, dev, False, member_step)
     return logs.finalize()
@@ -439,7 +377,7 @@ def _advantage(agent, replay_dict, ensemble_idx, want_priority=False, logits_all
     X, ld = _rows(s_rep)
     B, dev = X.shape[0], X.device
     logits = _forward(agent._actor_arena, 0, E, X, ld, B) if logits_all is None else logits_all   # [E,B,A]: every actor
-    q = _global_q(_forward(agent._critic_arena, i * N, N, X, ld, B), "dq_adv")                      # [N,B,A]
+    q = _global_q(_forward(agent._critic_arena, i * N, N, X, ld, B), "adv_q")                      # [N,B,A]
     act = _actions(a, B)
     popart = agent.popart[i]
     adv = torch.empty(B, dtype=torch.float32, device=dev)
@@ -481,14 +419,14 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
     logs = _logs.DeviceLogs(dev)
     loss_all, loss_slot = logs.slots(E)
     opt = _arena.FlatAdam.attach(actor_optimizer, aa)
-    enc_outs = []
-    rds, pols, adv_v = None, None, []
+    enc_outs, adv = [], []
+    rds, pols = None, None
     if filter_ and parallel.members_sharded():
         # pibar of member i's batch needs every rank's actors on it: all local batches first (the discrete filter draws
         # nothing, so the draws keep their order), then one exchange of states and one of logits
         rds = [lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per) for i in range(E)]
         pols = _member_policies(rds, agent, B)
-        g_lo = parallel.my_members()[0]
+        g_lo = parallel.my_range()[0]
 
     def member_step(i):
         rd = rds[i] if rds is not None else lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per)
@@ -496,10 +434,7 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
         mask = None
         if filter_:
             _, mask, _ = _advantage(agent, rd, i, logits_all=None if pols is None else pols[:, g_lo + i].contiguous())
-            v, slot = logs.slots(1)
-            v.copy_(mask.mean().reshape(1))
-            logs.defer("losses/adv_weights_mean", slot)
-            adv_v[:] = [v]
+            adv[:] = [logs.put_tensor("losses/adv_weights_mean", mask.mean())]
         if update_encoder:
             s_rep = agent.encoder(o)
         else:
@@ -513,7 +448,7 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
         dlogits = torch.empty((1, B, A), dtype=torch.float32, device=dev)
         L.discrete_bc_seed(logits.data_ptr(), act.data_ptr(), None if mask is None else mask.data_ptr(), B, A, En,
                            dlogits.data_ptr(), loss_all[i:i + 1].data_ptr(), stream)
-        logs.defer(f"losses/filterd_bc_loss_{_member_name(i)}", loss_slot + i)
+        logs.defer(f"losses/filterd_bc_loss_{parallel.member_id(i)}", loss_slot + i)
         dxg = torch.empty((1, B, S), dtype=torch.float32, device=dev) if need_ds else None
         _ops.mlp_backward(aa, i, 1, X, B, h1, h2, dlogits, ldx=ld, want_dw=True, accumulate=False, dx=dxg, lddx=S)
         if need_ds:
@@ -522,25 +457,14 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
 
     replay_dicts = lu._run_members(E, dev, False, member_step)
     enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
-    if actor_clip:
-        opt.grad_norm_sq(stream)
-    opt.step(stream, max_norm=actor_clip if actor_clip else None)
-    if parallel.members_sharded():
-        # the overall loss: the mean over every rank's members; the filter's acceptance rate: the last member's (as
-        # unsharded), which the last rank holds.  One exchange of two floats.
-        tot, tslot = logs.slots(2)
-        torch.sum(loss_all, 0, keepdim=True, out=tot[0:1])
-        if adv_v and parallel.my_members()[1] == En:
-            tot[1:2].copy_(adv_v[0])
-        else:
-            tot[1:2].zero_()
-        parallel.all_reduce_members_(tot)
-        logs.defer("losses/filtered_bc_overall_loss", tslot, transform=lambda v: v / En)
-        if adv_v:
-            logs.defer("losses/adv_weights_mean", tslot + 1)
+    if parallel.members_sharded():   # the per-member slots stay: the overall loss is summed into a slot of its own
+        total, total_slot = logs.slots(1)
+        torch.sum(loss_all, 0, keepdim=True, out=total)
+        logs.defer("losses/filtered_bc_overall_loss", total_slot, transform=lambda v: v / En)
     else:
+        total = None
         logs.defer("losses/filtered_bc_overall_loss", [loss_slot + i for i in range(E)], transform=lambda v: v / E)
-    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/actor_offline_grad_norm")
+    lu._actor_tail(logs, aa, opt, actor_clip, E, "gradients/actor_offline_grad_norm", total, *adv)
     lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_offline_actorloss_grad_norm")
     if per:
         lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)

@@ -33,7 +33,7 @@ def _graphable(agent, random_process, per, update_priorities, encoder_optimizer=
     step (_encoder_opt.structurally_eligible) --, no host-side decisions."""
     return (graphed.auto_graphs_enabled() and isinstance(_rng.source(), _rng.PhiloxSource) and not per and
             not update_priorities and (random_process is None or hasattr(random_process, "scale_dev")) and
-            not parallel.is_sharded() and not parallel.members_sharded() and
+            not parallel.sharded() and
             (not lu._encoder_trainable(agent) or _encoder_opt.structurally_eligible(agent.encoder, encoder_optimizer)))
 
 
@@ -89,7 +89,7 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
     ca = agent._critic_arena
     dev = ca.device
     _ops.check_cuda(ca.flat)
-    L, stream = _lib.lib(), _lib.stream_ptr()
+    L = _lib.lib()
     E, N, B = agent.ensemble_size, agent.num_critics, batch_size
     S, A = lu._dims(agent)
     # Software pipelining across consecutive updates (lu.pipelined_updates): the target side of this update runs on the
@@ -113,7 +113,7 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         pipe.keep.append(logs)
     loss_all, loss_slot = logs.slots(2 * E)   # per member: {loss contribution, mean td error of its last net}
     opt = _arena.FlatAdam.attach(critic_optimizer, ca)
-    if parallel.is_sharded() and E != 1:
+    if parallel.critics_sharded() and E != 1:
         raise NotImplementedError("critic sharding covers one member (REDQ / SAC shapes); SUNRISE members shard as a whole")
 
     enc_outs = []
@@ -140,7 +140,7 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         q_loc = torch.stack([lu._critic_values(target_agent, 0, E * N, x_all[e].contiguous(), B).reshape(E * N, B)
                              for e in range(En)], dim=1)                                                    # [E*N,En,B]
         q_weights = parallel.all_gather_members(q_loc)                                                      # [En*N,En,B]
-        g_lo = parallel.my_members()[0]
+        g_lo = parallel.my_range()[0]
     # Members are independent once their batches are drawn (the draws share one device-side Philox offset and stay in
     # order): with more than one member each runs on its own stream lane, forked from / joined into the caller's stream.
     # (softmax weights draw policy samples inside the member's work: those stay serial, in the reference's draw order)
@@ -206,7 +206,6 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         popart = agent.popart[i]
         imp = rd["imp_weights"]
         imp_ptr = imp.float().contiguous() if per else None  # per=False: ones(1), i.e. no weighting (main.py:401)
-        n_total = parallel.n_global() if parallel.is_sharded() else 0   # sharded critics: normalise by the global N
         if piped:
             main.wait_event(target_ready)
         elif side is not None:
@@ -215,7 +214,7 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         L.critic_forward_loss(W1, b1, W2, b2, W3, b3, N, ca.D, ca.H, X.data_ptr(), S + A, B, h1.data_ptr(), h2.data_ptr(),
                               q.data_ptr(), td_target.data_ptr(), w.data_ptr() if torch.is_tensor(w) else None,
                               None if imp_ptr is None else imp_ptr.data_ptr(), popart.state_ptr() if popart else None,
-                              int(bool(pop)), En, n_total, dq.data_ptr(), loss_v.data_ptr(), 2 if side is not None else 0,
+                              int(bool(pop)), En, parallel.n_global(N), dq.data_ptr(), loss_v.data_ptr(), 2 if side is not None else 0,
                               *((tdp["qt"].data_ptr(), tdp["M"], _ops._p(tdp["logp"]), tdp["log_alpha"].data_ptr(),
                                  tdp["r"].data_ptr(), tdp["d"].data_ptr(), tdp["gamma"], td_target.data_ptr(),
                                  tdp["logs"].data_ptr()) if tdp else (None, 0, None, None, None, None, 0.0, None, None)),
@@ -226,19 +225,8 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
             # DR3 (learning.py:100-108): second forward on (s1, a1); both feature sets carry gradient
             X1 = packed["X1"] if packed else torch.cat((s1, a1), dim=-1).contiguous()
             _, h1b, h2b = lu._critic_values(agent, i * N, N, X1, B, keep=True)
-            dv, dslot = logs.slots(1)
-            L.dr3_dot(h2.data_ptr(), h2b.data_ptr(), N, B, ca.H, dv.data_ptr(), _lib.stream_ptr())
-            logs.defer(f"dr3_dotproduct_{i}", dslot)
-            # critic_loss += dr3 * dot, then the whole loss is divided by E*N (learning.py:108,112).  Critics sharded over
-            # ranks: the mean runs over the GLOBAL ensemble -- this rank contributes its share to the loss (summed over the
-            # ranks with the rest of it below) and the logged dot product is summed right here
-            Ng = parallel.n_global() if parallel.is_sharded() else N
-            if Ng != N:
-                dv.mul_(N / Ng)
-            loss_v[0:1].add_(dv, alpha=dr3_coeff / (E * Ng))
-            if parallel.is_sharded():
-                parallel.all_reduce_sum_(dv, site="dr3_dot")
-            extra, extra_scale, f1 = h2b, dr3_coeff / (E * Ng) / (Ng * B), (X1, h1b, h2b)
+            extra_scale = lu._dr3_term(logs, ca, i, N, B, E, h2, h2b, dr3_coeff, loss_v)
+            extra, f1 = h2b, (X1, h1b, h2b)
         dxg = torch.empty((N, B, S + A), dtype=torch.float32, device=dev) if need_ds else None
         if pipe is not None:
             pipe.cross_before_grads(torch.cuda.current_stream(dev))
@@ -273,47 +261,8 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
         return member_step(i, draws, rd, i % lu.MEMBER_LANES if concurrent else 0)
 
     replay_dicts = lu._run_members(E, dev, concurrent, run_member)
-    logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)
-    logs.defer("losses/critic_overall_loss", [loss_slot + 2 * i for i in range(E)])
-
-    enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
-    if critic_clip:
-        opt.grad_norm_sq(stream)
-        if parallel.is_sharded():   # the global norm runs over every rank's critics (SURVEY 8e (3)): one float per rank
-            parallel.all_reduce_sum_(opt.gnorm_sq, site="critic_gnorm")
-    main = torch.cuda.current_stream(dev)
-    side = None if critic_clip else lu.side_stream(dev)   # clipping rescales the gradients that get logged
-    if side is not None:
-        # logged gradient norm next to Adam (which only reads the gradients)
-        side.wait_stream(main)
-        lu._log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad", stream=side)
-        if parallel.is_sharded():
-            # each rank summed its own critics: the logged loss is the global sum -- a log value, so its exchange runs
-            # next to Adam on the second stream instead of behind it
-            with torch.cuda.stream(side):
-                parallel.all_reduce_sum_(loss_all[0:1], site="critic_loss")
-    if pipe is not None:
-        pipe.main_wait_polyak(main)   # a Polyak step on the auxiliary stream still reads these
-    opt.step(stream, max_norm=critic_clip if critic_clip else None)
-    if pipe is not None:
-        pipe.cross_after_adam(main)
-    if side is not None:
-        main.wait_stream(side)
-    else:
-        lu._log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad")
-        if parallel.is_sharded():
-            parallel.all_reduce_sum_(loss_all[0:1], site="critic_loss")
-    lu._mark("Adam (+ logged grad norm)")
-
-    if parallel.members_sharded():                # ... or its own members: the logged loss is the global sum
-        tot = loss_all[0:2 * E:2].sum().reshape(1)
-        parallel.all_reduce_members_(tot)
-        loss_all[0:2 * E:2].zero_()
-        loss_all[0:1].copy_(tot)
-    lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_criticloss_grad_norm")
-    if update_priorities:
-        lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)
-    return logs.finalize(), replay_dicts
+    return lu._critic_tail(logs, loss_all, loss_slot, replay_dicts, buffer, agent, opt, pipe, critic_clip, encoder_optimizer,
+                           encoder_clip, enc_outs, update_priorities)
 
 
 def online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_size, clip, random_process, noise_clip,
@@ -349,7 +298,7 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
     aa, ca = agent._actor_arena, agent._critic_arena
     dev = aa.device
     _ops.check_cuda(aa.flat)
-    L, stream = _lib.lib(), _lib.stream_ptr()
+    L = _lib.lib()
     E, N, B = agent.ensemble_size, agent.num_critics, batch_size
     En = parallel.members_global(E)   # loss normalisation: the global ensemble size when members are sharded over ranks
     S, A = lu._dims(agent)
@@ -359,7 +308,7 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
     # members are independent given their batches and their N(0,1) draws: drawn in order on the caller's stream, then one
     # stream lane per member (as in critic_update)
     concurrent = (E > 1 and premade_replay_dicts is not None and lu.side_stream(dev) is not None
-                  and not parallel.is_sharded())
+                  and not parallel.critics_sharded())
 
     def draw_member():
         eps = torch.empty((B, A), dtype=torch.float32, device=dev)
@@ -385,7 +334,7 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
         q, h1c, h2c = lu._critic_values(agent, i * N, N, XPI, B, keep=True)
         popart = agent.popart[i]
         entropy_on = pol["logp"] is not None
-        if parallel.is_sharded():
+        if parallel.critics_sharded():
             # every rank sees all N_global values, picks the arg-min net per row, and back-propagates only the rows
             # whose arg-min critic it owns; the partial dL/da are summed below
             q_all = parallel.all_gather_q(q, site="actor_q")
@@ -412,7 +361,7 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
             dxg = torch.empty((N, B, S + A), dtype=torch.float32, device=dev)
             _ops.mlp_backward(ca, i * N, N, XPI, B, h1c, h2c, dq, ldx=S + A, want_dw=False, dx=dxg, lddx=S + A)
             L.sum_groups(dxg.data_ptr(), N, B, S + A, S, A, da.data_ptr(), _lib.stream_ptr())
-        if parallel.is_sharded():
+        if parallel.critics_sharded():
             parallel.all_reduce_sum_(da, site="actor_da")
         O = aa.O
         dout = torch.empty((1, B, O), dtype=torch.float32, device=dev)
@@ -425,10 +374,7 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
         _ops.mlp_backward(aa, i, 1, XPI, B, pol["h1"], pol["h2"], dout, ldx=S + A, want_dw=True, accumulate=False)
 
     lu._run_members(E, dev, concurrent, member_step)
-    if clip:
-        opt.grad_norm_sq(stream)
-    opt.step(stream, max_norm=clip if clip else None)
-    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/random_actor_online_grad")
+    lu._actor_tail(logs, aa, opt, clip, E, "gradients/random_actor_online_grad", loss_all)
     logs.defer("losses/actor_pg_loss", [loss_slot + i for i in range(E)])
     return logs.finalize()
 
@@ -485,18 +431,19 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
     _ops.check_cuda(aa.flat)
     L, stream = _lib.lib(), _lib.stream_ptr()
     E, B = agent.ensemble_size, batch_size
+    En = parallel.members_global(E)   # loss normalisation: the global ensemble size when members are sharded over ranks
     S, A = lu._dims(agent)
     logs = _logs.DeviceLogs(dev)
     opt = _arena.FlatAdam.attach(actor_optimizer, aa)
-    total = torch.zeros(1, dtype=torch.float32, device=dev)
-    enc_outs = []
+    total, total_slot = logs.slots(1)
+    enc_outs, adv = [], []
 
     def member_step(i):
         rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per)
         o, a, *_ = rd["primary_batch"]
         if filter_:
             _, mask, _ = lu._advantage(agent, rd, i)
-            logs.put_tensor("losses/adv_weights_mean", mask.mean())
+            adv[:] = [logs.put_tensor("losses/adv_weights_mean", mask.mean())]
         else:
             mask = torch.ones((B,), dtype=torch.float32, device=dev)
         if update_encoder:
@@ -509,14 +456,14 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
         X[:, :S].copy_(s_rep.detach())
         out, h1, h2 = lu._actor_forward(agent, i, X, B, S, A)
         logp = torch.empty((B,), dtype=torch.float32, device=dev)
-        dlogp = mask * (-1.0 / (B * E))
+        dlogp = mask * (-1.0 / (B * En))
         dout = torch.empty((1, B, aa.O), dtype=torch.float32, device=dev)
         a_c = a.contiguous() if a.stride(-1) != 1 else a
         L.tanh_normal_logprob(out.data_ptr(), a_c.data_ptr(), a_c.stride(0), B, A, float(agent.log_std_low),
                               float(agent.log_std_high), logp.data_ptr(), dlogp.data_ptr(), dout.data_ptr(), stream)
         member_loss = -(logp * mask).mean()
-        logs.put_tensor(f"losses/filterd_bc_loss_{i}", member_loss)
-        total.add_(member_loss / E)
+        logs.put_tensor(f"losses/filterd_bc_loss_{parallel.member_id(i)}", member_loss)
+        total.add_(member_loss / En)
         dxg = torch.empty((1, B, S + A), dtype=torch.float32, device=dev) if need_ds else None
         _ops.mlp_backward(aa, i, 1, X, B, h1, h2, dout, ldx=S + A, want_dw=True, accumulate=False, dx=dxg, lddx=S + A)
         if need_ds:
@@ -526,11 +473,8 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
     replay_dicts = lu._run_members(E, dev, False, member_step)
     # (s_rep carries gradient only with update_encoder: the same fused clip + Adam as in critic_update)
     enc_net = lu._encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
-    if actor_clip:
-        opt.grad_norm_sq(stream)
-    opt.step(stream, max_norm=actor_clip if actor_clip else None)
-    logs.put_tensor("losses/filtered_bc_overall_loss", total)
-    lu._log_member_grad_norm(logs, aa, E, 1, "gradients/actor_offline_grad_norm")
+    logs.defer("losses/filtered_bc_overall_loss", total_slot)
+    lu._actor_tail(logs, aa, opt, actor_clip, E, "gradients/actor_offline_grad_norm", total, *adv)
     lu._log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_offline_actorloss_grad_norm")
     if per:
         lu.adjust_priorities(logs, replay_dicts[-1], agent, buffer)

@@ -202,10 +202,11 @@ MEMBER_LANES = 4
 
 def side_stream(device, lane=0):
     """One extra stream per device (and member lane) for the independent branches of an update (online trunk next to
-    the target networks, the logged gradient norm next to Adam).  None when overlap is switched off (ssac_set_overlap)."""
-    if not _lib.lib().get_overlap():
-        return None
+    the target networks, the logged gradient norm next to Adam).  None when overlap is switched off (ssac_set_overlap)
+    and for a device without streams."""
     device = torch.device(device)
+    if device.type != "cuda" or not _lib.lib().get_overlap():
+        return None
     st = _side_streams.get((device, lane))
     if st is None:
         st = _side_streams[(device, lane)] = torch.cuda.Stream(device=device)
@@ -682,7 +683,7 @@ def _critic_pipeline(agent, per, update_priorities, weight_type):
     p, dev = _pipeline, agent._critic_arena.device
     if (p is None or agent.ensemble_size != 1 or per or update_priorities or weight_type is not None
             or _encoder_trainable(agent) or any(bool(pa) for pa in agent.popart)
-            or (parallel.is_sharded() and not parallel.peer_exchange_ready()) or parallel.members_sharded()
+            or (parallel.critics_sharded() and not parallel.peer_exchange_ready()) or parallel.members_sharded()
             or side_stream(dev) is None or p.device != dev):
         pipeline_barrier()
         return None
@@ -752,6 +753,82 @@ def _log_encoder_grad_norm(logs, agent, enc_net, enc_outs, key):
         logs[key] = 0.0
 
 
+def _dr3_term(logs, arena, i, N, B, E, h2, h2b, dr3_coeff, loss_v):
+    """DR3 (learning.py:100-108) of member i's N critics from their last hidden layers on s (``h2``) and on s1 (``h2b``):
+    logs the dot product, adds dr3 * dot / (E * N) to the member's loss slot ``loss_v`` (learning.py:108,112) and returns
+    the scale of the gradient both feature sets carry.  Sharded ensembles normalise over the global ensemble: with the
+    critics sharded this rank adds its share N / N_global to the loss (summed over the ranks with the rest of it) and
+    the logged dot product is summed right here."""
+    Ng, En = parallel.n_global(N), parallel.members_global(E)
+    dv, dslot = logs.slots(1)
+    _lib.lib().dr3_dot(h2.data_ptr(), h2b.data_ptr(), N, B, arena.H, dv.data_ptr(), _lib.stream_ptr())
+    logs.defer(f"dr3_dotproduct_{parallel.member_id(i)}", dslot)
+    if Ng != N:
+        dv.mul_(N / Ng)
+    loss_v[0:1].add_(dv, alpha=dr3_coeff / (En * Ng))
+    if parallel.critics_sharded():
+        parallel.all_reduce_sum_(dv, site="dr3_dot")
+    return dr3_coeff / (En * Ng) / (Ng * B)
+
+
+def _critic_tail(logs, loss_all, loss_slot, replay_dicts, buffer, agent, opt, pipe, critic_clip, encoder_optimizer,
+                 encoder_clip, enc_outs, update_priorities):
+    """The end of a critic update once every member's gradients are in: the encoder step, clip + Adam, the logged values
+    and the priority refresh.  ``loss_all`` holds two slots per member: its loss contribution and the mean TD error of
+    its last net.  Returns what critic_update returns."""
+    ca, E, N = agent._critic_arena, agent.ensemble_size, agent.num_critics
+    dev, stream = ca.device, _lib.stream_ptr()
+    logs.defer("losses/last_member_critic_td_error", loss_slot + 2 * (E - 1) + 1)
+    logs.defer("losses/critic_overall_loss", [loss_slot + 2 * i for i in range(E)])
+
+    def logged_values(on=None):
+        _log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad", stream=on)
+        if parallel.sharded():   # the loss summed over every rank, the TD error of the ensemble's last net
+            with (torch.cuda.stream(on) if on is not None else contextlib.nullcontext()):
+                parallel.reduce_logged(loss_all[0:2 * E:2], loss_all[2 * E - 1:2 * E], site="critic_loss")
+
+    enc_net = _encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
+    if critic_clip:
+        opt.grad_norm_sq(stream)
+        if parallel.sharded():   # the global norm runs over every rank's critics (SURVEY 8e (3)): one float per rank
+            parallel.all_reduce_sum_(opt.gnorm_sq, site="critic_gnorm")
+    side = None if critic_clip else side_stream(dev)   # clipping rescales the gradients that get logged
+    main = torch.cuda.current_stream(dev) if side is not None or pipe is not None else None
+    if side is not None:   # the logged values next to Adam (which only reads the gradients)
+        side.wait_stream(main)
+        logged_values(side)
+    if pipe is not None:
+        pipe.main_wait_polyak(main)   # a Polyak step on the auxiliary stream still reads the online parameters
+    opt.step(stream, max_norm=critic_clip if critic_clip else None)   # (clipping rescales the stored gradients, as the reference's does)
+    if pipe is not None:
+        pipe.cross_after_adam(main)
+    if side is not None:
+        main.wait_stream(side)
+    else:
+        logged_values()
+    _mark("Adam (+ logged grad norm)")
+    _log_encoder_grad_norm(logs, agent, enc_net, enc_outs, "gradients/encoder_criticloss_grad_norm")
+    if update_priorities:
+        adjust_priorities(logs, replay_dicts[-1], agent, buffer)
+    return logs.finalize(), replay_dicts
+
+
+def _actor_tail(logs, arena, opt, clip, E, grad_key, loss_v, last=None):
+    """Clip + Adam of the actors and the logged gradient norm of a random member.  Members sharded over ranks: the clip
+    norm runs over every rank's actors, the logged loss in ``loss_v`` becomes the sum over every rank's members and
+    ``last``, a value of the last member, the last rank's (parallel.reduce_logged).  (With the critics sharded the
+    actors are replicas: nothing to exchange.)"""
+    stream = _lib.stream_ptr()
+    if clip:
+        opt.grad_norm_sq(stream)
+        if parallel.members_sharded():
+            parallel.all_reduce_sum_(opt.gnorm_sq, site="actor_gnorm")
+    opt.step(stream, max_norm=clip if clip else None)
+    _log_member_grad_norm(logs, arena, E, 1, grad_key)
+    if parallel.members_sharded():
+        parallel.reduce_logged(loss_v, last, site="actor_loss")
+
+
 class _AlphaState:
     """Adam state of one 1-element ``log_alpha`` optimiser (main.py:230-239), kept on the device."""
 
@@ -781,7 +858,8 @@ class _AlphaState:
 
 
 def _alpha_step(logs, i, optimizer, log_alpha, logp, B, target_entropy):
-    """Member i's temperature step (learning.py:246-262) on ``logp`` [B]: loss, scalar Adam and logs in one launch."""
+    """Member i's temperature step (learning.py:246-262) on ``logp`` [B]: loss, scalar Adam and logs (under the global
+    member id) in one launch."""
     pg = optimizer.param_groups[0]
     st = _AlphaState.attach(optimizer, log_alpha)
     lv, slot = logs.slots(2)
@@ -790,8 +868,8 @@ def _alpha_step(logs, i, optimizer, log_alpha, logp, B, target_entropy):
                           float(pg["eps"]), lv.data_ptr(), _lib.stream_ptr())
     st.steps += 1
     st._step_tensor.fill_(st.steps)
-    logs.defer(f"losses/alpha_loss_{i}", slot)
-    logs.defer(f"alphas/alpha_{i}", slot + 1)
+    logs.defer(f"losses/alpha_loss_{parallel.member_id(i)}", slot)
+    logs.defer(f"alphas/alpha_{parallel.member_id(i)}", slot + 1)
 
 
 def draw_for_critic_member(buffer, agent, B, ensemble_n, random_process, per, zero=None):
@@ -799,7 +877,7 @@ def draw_for_critic_member(buffer, agent, B, ensemble_n, random_process, per, ze
     N(0,1) draw or the TD3 noise (learning_utils.py:49,330), the REDQ target subset (agent.py:29) -- in ONE launch."""
     dev = buffer.device
     S, A = _dims(agent)
-    n_sub_pool = parallel.n_global() if parallel.is_sharded() else agent.num_critics
+    n_sub_pool = parallel.n_global(agent.num_critics)   # critics sharded over ranks: the subset of the GLOBAL ensemble
     assert 0 < ensemble_n <= n_sub_pool
     idx = None if per else torch.empty(B, dtype=torch.int64, device=dev)
     need_normal = (not agent.deterministic) or (random_process is not None)
@@ -833,7 +911,7 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
     X1 = _first_layer_input(s1_rep, None, packed["X1"] if packed else None, S, A)
     N = agent.num_critics
     # REDQ subset: drawn over the GLOBAL ensemble when the critics are sharded over ranks (replicated Philox state)
-    pool = parallel.n_global() if parallel.is_sharded() else N
+    pool = parallel.n_global(N)
     assert 0 < ensemble_n <= pool
     if _draws is not None:   # critic_update drew indices, policy noise and the subset in ONE launch
         net_index = _draws["subset"]
@@ -847,7 +925,7 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
         _rng.source().subsets(net_index, pool, ensemble_n)
     if _pipeline is not None:
         _pipeline.front_wait_polyak()   # the target critics' parameters: the only thing this side reads that Polyak writes
-    if parallel.is_sharded():
+    if parallel.critics_sharded():
         # every rank evaluates its own target critics and all-gathers the [N_global, B] values; the subset-min is then
         # identical on every rank
         q_t = parallel.all_gather_q(_critic_values(target_agent, i * N, N, X1, B), site="target_q", select=net_index)
@@ -855,14 +933,15 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
         q_t = _critic_values(target_agent, i * N, ensemble_n, X1, B, net_index=net_index)
     _mark("target critics Q(s1, a1)")
     y = torch.empty((B, 1), dtype=torch.float32, device=X1.device)
+    g = parallel.member_id(i)
     if _fuse_into_loss and not popart and user_logs is None:   # popart is False (reference convention) when off
         lv, slot = dlogs.slots(4)   # {sum (y-c), sum (y-c)^2, sum alpha*logp, c}: zero-initialised with the buffer
         y._ssac_pending = dict(qt=q_t, M=int(ensemble_n), logp=pol["logp"], log_alpha=log_alphas[i], r=r, d=d,
                                gamma=float(gamma), logs=lv)
-        dlogs.defer_fn(f"td_targets/mean_td_target_{i}", (slot, slot + 3), lambda s1, c, n=B: c + s1 / n)
-        dlogs.defer_fn(f"td_targets/std_td_target_{i}", (slot, slot + 1),
+        dlogs.defer_fn(f"td_targets/mean_td_target_{g}", (slot, slot + 3), lambda s1, c, n=B: c + s1 / n)
+        dlogs.defer_fn(f"td_targets/std_td_target_{g}", (slot, slot + 1),
                        lambda s1, s2, n=B: max((s2 - s1 * s1 / n) / (n - 1), 0.0) ** 0.5)
-        dlogs.defer_fn(f"td_targets/entropy_bonus_{i}", (slot + 2,), lambda se, n=B: se / n)
+        dlogs.defer_fn(f"td_targets/entropy_bonus_{g}", (slot + 2,), lambda se, n=B: se / n)
         return y, (X1[:, :S], X1[:, S:])
     lv, slot = dlogs.slots(3)
     _lib.lib().td_target(q_t.data_ptr(), ensemble_n, B, None if pol["logp"] is None else pol["logp"].data_ptr(),
@@ -871,9 +950,9 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
                          int(bool(pop)), float(popart.beta) if popart else 0.0, int(popart.min_steps) if popart else 0,
                          y.data_ptr(), lv.data_ptr(), _lib.stream_ptr())
     _mark("td target")
-    dlogs.defer(f"td_targets/mean_td_target_{i}", slot)
-    dlogs.defer(f"td_targets/std_td_target_{i}", slot + 1)
-    dlogs.defer(f"td_targets/entropy_bonus_{i}", slot + 2)
+    dlogs.defer(f"td_targets/mean_td_target_{g}", slot)
+    dlogs.defer(f"td_targets/std_td_target_{g}", slot + 1)
+    dlogs.defer(f"td_targets/entropy_bonus_{g}", slot + 2)
     if user_logs is not None:
         user_logs.update(dlogs.finalize())
     return y, (X1[:, :S], X1[:, S:])

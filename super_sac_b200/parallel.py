@@ -1,19 +1,32 @@
 """Ensemble sharding across the GPUs of one node (SURVEY §8e): one process per GPU, `torch.distributed` plumbing.
 
-REDQ-style critics shard naturally: each critic's forward / backward / Adam / Polyak is independent given the TD
-target.  With sharding enabled, rank r builds its ``Agent`` with only its ``n_local`` critics (``local_range``), every
-rank keeps a replica of the actor, the temperature and the batch (identical Philox seed => identical indices, eps and
-subset on every rank, no broadcast), and the update functions exchange exactly two small tensors per phase:
+One ensemble is partitioned over the ranks in one of two ways, never both at once:
 
-  critic update : all-gather of the target critics' Q(s1, a1)  [N, B]  -> subset-min on every rank (same TD target)
-  actor update  : all-gather of Q(s, pi(s))                     [N, B]  -> arg-min routing;
-                  all-reduce(sum) of dL/da                       [B, A]  -> replicated actor backward + Adam
+- critics (``enable_critic_sharding``): rank r builds its ``Agent`` with only its ``n_local`` critics (``local_range``) of
+  one member; every rank keeps a replica of the actor, the temperature and the batch (identical Philox seed =>
+  identical indices, eps and subset on every rank, no broadcast).  REDQ-style critics shard naturally: each critic's
+  forward / backward / Adam / Polyak is independent given the TD target, so the updates exchange only small tensors:
 
-Payloads are <= 10 KB, so the exchange is pure latency.  On CUDA devices with peer access the exchange does not go
+    critic update : gather of the target critics' Q(s1, a1)  [N, B]  -> subset-min on every rank (same TD target)
+    actor update  : gather of Q(s, pi(s))                     [N, B]  -> arg-min routing;
+                    sum of dL/da                              [B, A]  -> replicated actor backward + Adam
+
+- members (``enable_member_sharding``): rank r builds its ``Agent`` with only its block of whole SUNRISE members and
+  seeds its own Philox stream.  Members are independent learners (own actor, critics, batch); the single coupling is the
+  SUNRISE weight, a statistic over ALL members' target critics on each member's batch: one gather of the local batches
+  and one of the local target critics' values on every batch per update (``all_gather_members``).
+
+Either way a sharded update equals the single-GPU one: the losses are normalised by the global ensemble
+(``n_global``, ``members_global``), per-member log keys carry the global member id (``member_id``) and the logged sums
+and last-net values are the whole ensemble's (``reduce_logged``).
+
+Payloads are <= 10 KB, so every exchange is pure latency.  On CUDA devices with peer access the exchanges do not go
 through NCCL at all: every rank stores its rows straight into all peers' symmetric buffers over NVLink and raises a
 signal, the consumer spins on its signals (ssac_peer_put / ssac_peer_wait, csrc/ssac_peer.cu; the buffers' peer mappings
-come from torch.distributed._symmetric_memory).  ``torch.distributed`` collectives remain as the fallback (CPU / gloo
-tests, boxes without peer access) -- ``exchange_name()`` says which one is live.
+come from torch.distributed._symmetric_memory).  ``torch.distributed`` collectives (all-gather, all-reduce) remain as
+the fallback (CPU / gloo tests, boxes without peer access) -- ``exchange_name()`` says which one is live.  Each call
+site has an exchange site of its own (a name): a site is used from one stream only, as its two halves alternate
+between consecutive exchanges.
 """
 import os
 import random
@@ -21,7 +34,8 @@ import random
 import torch
 import torch.distributed as dist
 
-_state = {"on": False, "group": None, "world": 1, "rank": 0, "n_global": None}
+# kind: None, "critics" or "members"; n: the global number of the sharded units (critics of the member, or members)
+_state = {"kind": None, "group": None, "world": 1, "rank": 0, "n": None}
 
 
 # ---- peer-memory exchange sites ---------------------------------------------------------------------------------------
@@ -109,32 +123,68 @@ def local_range(n_global, world, rank):
     return lo, lo + base + (1 if rank < extra else 0)
 
 
+def _enable(kind, n, group):
+    if _state["kind"] not in (None, kind):
+        raise NotImplementedError(f"the {_state['kind']} are sharded already: critic sharding and member sharding "
+                                  "cannot be combined")
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    if n < world:
+        raise ValueError(f"{n} {kind} cannot be sharded over {world} ranks")
+    _state.update(kind=kind, group=group, world=world, rank=rank, n=int(n))
+    return local_range(n, world, rank)
+
+
 def enable_critic_sharding(num_critics_global, group=None):
     """Call after ``dist.init_process_group``; returns (lo, hi), the global ids of this rank's critics.  Build the Agent
     with ``num_critics = hi - lo``."""
-    world = dist.get_world_size(group)
-    rank = dist.get_rank(group)
-    if num_critics_global < world:
-        raise ValueError(f"{num_critics_global} critics cannot be sharded over {world} ranks")
-    _state.update(on=True, group=group, world=world, rank=rank, n_global=int(num_critics_global))
-    return local_range(num_critics_global, world, rank)
+    return _enable("critics", num_critics_global, group)
+
+
+def enable_member_sharding(ensemble_size_global, group=None):
+    """Call after ``dist.init_process_group``; returns (lo, hi), the global ids of this rank's members.  Build the Agent
+    with ``ensemble_size = hi - lo``."""
+    return _enable("members", ensemble_size_global, group)
 
 
 def disable():
-    _state.update(on=False, group=None, world=1, rank=0, n_global=None)
-    disable_member_sharding()
+    _state.update(kind=None, group=None, world=1, rank=0, n=None)
 
 
-def is_sharded():
-    return _state["on"]
+def sharded():
+    return _state["kind"] is not None
 
 
-def n_global():
-    return _state["n_global"]
+def critics_sharded():
+    return _state["kind"] == "critics"
+
+
+def members_sharded():
+    return _state["kind"] == "members"
+
+
+def n_global(n_local):
+    """The number of critics per member the losses are normalised with: every rank's when the critics are sharded."""
+    return _state["n"] if critics_sharded() else n_local
+
+
+def members_global(e_local):
+    """The ensemble size the losses are normalised with: every rank's members when the members are sharded."""
+    return _state["n"] if members_sharded() else e_local
 
 
 def my_range():
-    return local_range(_state["n_global"], _state["world"], _state["rank"])
+    """Global ids [lo, hi) of this rank's critics or members."""
+    return local_range(_state["n"], _state["world"], _state["rank"])
+
+
+def my_members():
+    """Global ids [lo, hi) of this rank's members (members sharded)."""
+    return my_range()
+
+
+def member_id(i):
+    """Global id of local member i, for per-member log keys."""
+    return i + my_range()[0] if members_sharded() else i
 
 
 def same_member_choice(e):
@@ -144,7 +194,7 @@ def same_member_choice(e):
     across ranks.  Every rank draws (its RNG stream advances as unsharded) and rank 0's pick is broadcast: one host round
     trip, on those eager paths only."""
     member = random.choice(range(e))
-    if e > 1 and _state["on"]:
+    if e > 1 and critics_sharded():
         box = [member]
         dist.broadcast_object_list(box, group=_state["group"], group_src=0)
         member = int(box[0])
@@ -154,12 +204,12 @@ def same_member_choice(e):
 def all_gather_q(q_local, site="q", select=None):
     """q_local [n_local, B, ...] -> [N_global, B, ...] in global net order (or only the rows ``select``).  ``site`` names
     the call site: every site has its own symmetric buffer and signals."""
-    return _all_gather_rows(q_local, _state["n_global"], _state["world"], _state["group"], site_name=site, select=select)
+    return _all_gather_rows(q_local, site, select=select)
 
 
-def _all_gather_rows(q_local, n, world, group, site_name="rows", select=None):
+def _all_gather_rows(q_local, site_name, select=None):
     """``select`` (device int32 [m]): return only those global rows (cheaper than gathering everything and indexing)."""
-    rank = dist.get_rank(group)
+    n, world, rank, group = _state["n"], _state["world"], _state["rank"], _state["group"]
     row = q_local[0].numel() * q_local.element_size() if q_local.shape[0] else 0
     site = _site(site_name, n * row, group, q_local.device) if row else None
     if site is not None:
@@ -186,70 +236,48 @@ def _all_gather_rows(q_local, n, world, group, site_name="rows", select=None):
     return out if select is None else out.index_select(0, select.long())
 
 
-def _all_reduce_sum_(t, world, group, site_name):
-    site = _site(site_name, world * t.numel() * t.element_size(), group, t.device)
-    if site is not None:
+def all_reduce_sum_(t, site="sum"):
+    world, group = _state["world"], _state["group"]
+    peer = _site(site, world * t.numel() * t.element_size(), group, t.device)
+    if peer is not None:
         # every rank lands its partial in slot `rank` of every peer, then sums the slots in rank order: the same
         # arithmetic on every rank (replicas stay bit-identical), no ring order to depend on
         parts = torch.empty((world,) + tuple(t.shape), dtype=t.dtype, device=t.device)
-        site.put(t, dist.get_rank(group) * t.numel() * t.element_size())
-        site.wait(parts)
+        peer.put(t, _state["rank"] * t.numel() * t.element_size())
+        peer.wait(parts)
         t.copy_(parts.sum(0))
         return t
     dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
     return t
 
 
-def all_reduce_sum_(t, site="sum"):
-    return _all_reduce_sum_(t, _state["world"], _state["group"], site)
+def all_reduce_members_(t):
+    """Sum ``t`` over the ranks of a member-sharded ensemble."""
+    return all_reduce_sum_(t, site="members_sum")
 
 
-# ---- SUNRISE-style ensembles: whole members sharded over the ranks (SURVEY 8e, C3) ---------------------------------
-# Members are independent learners (own actor, critics, batch); rank r builds its Agent with only its block of members
-# and seeds its own Philox stream.  The single coupling is the SUNRISE weight, a statistic over ALL members' target
-# critics evaluated on each member's batch: one all-gather of the local batches [E_local, B, S+A] and one all-gather of
-# the local target critics' values on every batch [E_local*N, E_global, B] per update.  Loss normalisation keeps the
-# global ensemble size.
-_mstate = {"on": False, "group": None, "world": 1, "rank": 0, "e_global": None}
-
-
-def enable_member_sharding(ensemble_size_global, group=None):
-    """Call after ``dist.init_process_group``; returns (lo, hi), the global ids of this rank's members.  Build the Agent
-    with ``ensemble_size = hi - lo``."""
-    world = dist.get_world_size(group)
-    rank = dist.get_rank(group)
-    if ensemble_size_global < world:
-        raise ValueError(f"{ensemble_size_global} members cannot be sharded over {world} ranks")
-    _mstate.update(on=True, group=group, world=world, rank=rank, e_global=int(ensemble_size_global))
-    return local_range(ensemble_size_global, world, rank)
-
-
-def disable_member_sharding():
-    _mstate.update(on=False, group=None, world=1, rank=0, e_global=None)
-
-
-def members_sharded():
-    return _mstate["on"]
-
-
-def members_global(e_local):
-    """The ensemble size the losses are normalised with."""
-    return _mstate["e_global"] if _mstate["on"] else e_local
-
-
-def my_members():
-    return local_range(_mstate["e_global"], _mstate["world"], _mstate["rank"])
+def reduce_logged(loss_v, last=None, site="logged"):
+    """The logged values of a sharded update made the single-GPU ones, in one exchange of one or two floats: the sum of
+    this rank's loss slots ``loss_v`` over every rank is left in loss_v[0] (the other slots are cleared), and ``last``, a
+    value of this rank's last net or member, becomes that of the rank that owns the ensemble's last one."""
+    red = torch.empty(1 if last is None else 2, dtype=torch.float32, device=loss_v.device)
+    torch.sum(loss_v, 0, keepdim=True, out=red[0:1])
+    if last is not None:
+        if my_range()[1] == _state["n"]:
+            red[1:2].copy_(last)
+        else:
+            red[1:2].zero_()
+    all_reduce_sum_(red, site)
+    loss_v.zero_()
+    loss_v[0:1].copy_(red[0:1])
+    if last is not None:
+        last.copy_(red[1:2])
 
 
 def all_gather_members(x_local):
     """x_local [E_local * k, ...] (k rows per member, member-major) -> [E_global * k, ...] in global member order."""
-    e_local = my_members()[1] - my_members()[0]
-    k = x_local.shape[0] // e_local
-    x = x_local.reshape((e_local, k) + tuple(x_local.shape[1:]))
-    out = _all_gather_rows(x.contiguous(), _mstate["e_global"], _mstate["world"], _mstate["group"],
-                           site_name="members%d" % (x[0].numel() if x.shape[0] else 0))
-    return out.reshape((_mstate["e_global"] * k,) + tuple(x_local.shape[1:]))
-
-
-def all_reduce_members_(t):
-    return _all_reduce_sum_(t, _mstate["world"], _mstate["group"], "members_sum")
+    lo, hi = my_range()
+    k = x_local.shape[0] // (hi - lo)
+    x = x_local.reshape((hi - lo, k) + tuple(x_local.shape[1:]))
+    out = _all_gather_rows(x.contiguous(), "members%d" % (x[0].numel() if x.shape[0] else 0))
+    return out.reshape((_state["n"] * k,) + tuple(x_local.shape[1:]))

@@ -466,9 +466,8 @@ def test_sharded_discrete_limits_fail_loudly(monkeypatch):
             critic(agent(2))
         with pytest.raises(NotImplementedError, match="trainable"):
             critic(agent(1, Trainable(3)))
-        parallel.enable_member_sharding(2)
         with pytest.raises(NotImplementedError, match="cannot be combined"):
-            critic(agent(1))
+            parallel.enable_member_sharding(2)
         parallel.disable()
         parallel.enable_member_sharding(2)
         with pytest.raises(NotImplementedError, match="priority refresh"):

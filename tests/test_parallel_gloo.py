@@ -4,6 +4,7 @@ sum to the single-process gradient).  No CUDA involved: the exchanged tensors ar
 import os
 import socket
 
+import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
@@ -116,3 +117,29 @@ def test_member_sharding_exchange_world2_gloo():
     got = sorted(q.get(timeout=5) for _ in range(world))
     assert got == [(0, 0, 3), (1, 3, 5)]
     assert not parallel.members_sharded()
+
+
+def test_one_partition_at_a_time(monkeypatch):
+    """An ensemble is sharded one way at a time: enabling the other kind raises and leaves the first in place.  With
+    sharding off the global sizes and member ids are the local ones."""
+    monkeypatch.setenv("MASTER_ADDR", "127.0.0.1")
+    monkeypatch.setenv("MASTER_PORT", str(_free_port()))
+    dist.init_process_group("gloo", rank=0, world_size=1)
+    try:
+        assert not parallel.sharded()
+        assert parallel.n_global(3) == 3 and parallel.members_global(4) == 4
+        assert [parallel.member_id(i) for i in range(3)] == [0, 1, 2]
+        for first, other, on in ((parallel.enable_critic_sharding, parallel.enable_member_sharding, parallel.critics_sharded),
+                                 (parallel.enable_member_sharding, parallel.enable_critic_sharding, parallel.members_sharded)):
+            first(5)
+            with pytest.raises(NotImplementedError, match="cannot be combined"):
+                other(5)
+            assert on() and parallel.my_range() == (0, 5)
+            parallel.disable()
+        parallel.enable_critic_sharding(5)
+        assert parallel.n_global(2) == 5 and parallel.members_global(2) == 2 and parallel.member_id(1) == 1
+        parallel.disable()
+        assert parallel.n_global(3) == 3 and not parallel.sharded()
+    finally:
+        parallel.disable()
+        dist.destroy_process_group()
