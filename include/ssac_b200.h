@@ -270,7 +270,7 @@ int ssac_critic_forward_loss(const float* W1, const float* b1, const float* W2, 
  * caller forms the logged mean / unbiased std / entropy bonus (learning_utils.py:351-353). */
 
 /* ---- row-local forwards on the CUDA cores (exact fp32): the single-net, latency-bound pieces ------------------------
- * One launch of ceil(B/8) clusters x 4 CTAs; every cluster walks the whole chain for 8 batch rows (layer slices per CTA,
+ * One launch of ceil(B/16) clusters x 4 CTAs; every cluster walks the whole chain for 16 batch rows (layer slices per CTA,
  * activations exchanged over distributed shared memory).  H in 32..256 (multiple of 8), first-layer width <= 64, O <= 16;
  * ssac_rows_supported(D, H, O) tells.  No activations are kept (forward-only uses).
  * ssac_policy_rows: one actor with its head (acting path agent.py:204-327, forward-only policy samples); out_dev
