@@ -415,6 +415,17 @@ int ssac_peer_put(const void* src_dev, int64_t nbytes, int64_t dst_off, int64_t 
 int ssac_peer_wait(const void* my_buf_dev, int64_t half_bytes, int64_t nbytes, const uint32_t* my_sigs_dev, int world,
                    const uint32_t* epoch_dev, void* out_dev, const int32_t* row_index_dev, int n_rows, int64_t row_bytes,
                    void* stream);
+/* Bulk all-reduce (sum) of n floats for the batch-sharded learner's gradients: dst_dev = sum over the ranks of src_dev
+ * (dst may alias src), bitwise identical on every rank.  Two-shot over a symmetric buffer (my_buf_dev on this rank,
+ * peer_bufs_dev: device array of the `world` mapped pointers) of 4 x cap_bytes (two epoch halves of {in, out} regions of
+ * cap_bytes >= 4n, a multiple of 16): stage src into this rank's `in`; rank r sums its 1/W slice of every rank's `in` in
+ * rank order 0..W-1 in fp32 (rank W-1 also the n % 4 tail) and stores it into every rank's `out`; then `out` is copied to
+ * dst.  Signals: symmetric uint32[128] per rank (my_sigs_dev / peer_sigs_dev as for put/wait: slots 0..63 "staged",
+ * 64..127 "reduced"); epoch_dev as for put/wait; ticket_dev: device uint32[2] of this rank, zero-initialised once (the
+ * kernels reset it).  Multi-block, 16-byte loads and stores, no allocation and no host synchronisation (capturable). */
+int ssac_peer_allreduce(const float* src_dev, float* dst_dev, int64_t n, void* my_buf_dev, int64_t cap_bytes,
+                        void* const* peer_bufs_dev, const uint32_t* my_sigs_dev, uint32_t* const* peer_sigs_dev, int rank,
+                        int world, uint32_t* epoch_dev, uint32_t* ticket_dev, void* stream);
 
 /* ---- DrQ pixel encoder: nets/cnns.py:37-69 (BigPixelEncoder), SURVEY 8f N3 ------------------------------------------ */
 /* obs [B,C,H,W] fp32 in 0..255 -> obs/255 - 0.5 -> conv3x3 stride 2 (C -> 32) -> 3 x conv3x3 stride 1 (32 -> 32), each + ReLU

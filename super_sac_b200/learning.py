@@ -79,6 +79,8 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
                         critic_clip, encoder_clip, target_critic_ensemble_n, weighted_bellman_temp, weight_type, pop,
                         augmenter, encoder_lambda, random_process, noise_clip, aug_mix=0.75, discrete=False, per=False,
                         update_priorities=False, dr3_coeff=0.0):
+    lu.check_batch_sharding(agent, encoder_optimizer, per, update_priorities, weight_type, weighted_bellman_temp, dr3_coeff,
+                            discrete, augmenter, batch_size)
     if discrete:   # SAC-Discrete (learning.py:84-92, learning_utils.py:322-328): discrete.py
         return _discrete.critic_update(buffer, agent, target_agent, critic_optimizer, encoder_optimizer, log_alphas,
                                        batch_size, gamma, critic_clip, encoder_clip, target_critic_ensemble_n,
@@ -90,7 +92,9 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
     dev = ca.device
     _ops.check_cuda(ca.flat)
     L = _lib.lib()
-    E, N, B = agent.ensemble_size, agent.num_critics, batch_size
+    E, N, B_all = agent.ensemble_size, agent.num_critics, batch_size
+    lo, hi = parallel.batch_range(B_all)   # batch sharded over ranks: this rank's rows of the global batch
+    B = hi - lo
     S, A = lu._dims(agent)
     # Software pipelining across consecutive updates (lu.pipelined_updates): the target side of this update runs on the
     # front stream, which is NOT joined at the end of the update -- the next update's target side starts next to this
@@ -122,10 +126,10 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
     presampled, q_weights = None, None
 
     def draw_member():
-        draws = lu.draw_for_critic_member(buffer, agent, B, target_critic_ensemble_n, random_process, per,
+        draws = lu.draw_for_critic_member(buffer, agent, B_all, target_critic_ensemble_n, random_process, per,
                                           zero=logs.take_unzeroed())
         lu._mark("draws (indices, eps, subset)")
-        return draws, lu.sample_move_and_augment(buffer=buffer, batch_size=B, augmenter=augmenter, aug_mix=aug_mix,
+        return draws, lu.sample_move_and_augment(buffer=buffer, batch_size=B_all, augmenter=augmenter, aug_mix=aug_mix,
                                                  per=per, _idx=draws["idx"])
 
     if parallel.members_sharded() and weight_type is not None and weighted_bellman_temp is not None and En > 1:
@@ -193,7 +197,9 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
             td_target, (s1, a1) = lu.compute_td_targets(
                 logs=logs, replay_dict=rd, agent=agent, target_agent=target_agent, log_alphas=log_alphas, ensemble_idx=i,
                 ensemble_n=target_critic_ensemble_n, pop=pop, gamma=gamma, random_process=random_process,
-                noise_clip=noise_clip, _draws=draws, _fuse_into_loss=side is not None)
+                noise_clip=noise_clip, _draws=draws,
+                # (batch sharded over several ranks: the TD target kernel's statistics are pooled over the ranks)
+                _fuse_into_loss=side is not None and not (parallel.batches_sharded() and parallel.world_size() > 1))
             if piped:
                 target_ready = torch.cuda.Event()
                 target_ready.record(pipe.front)
@@ -219,6 +225,7 @@ def _critic_update_impl(buffer, agent, target_agent, critic_optimizer, encoder_o
                                  tdp["r"].data_ptr(), tdp["d"].data_ptr(), tdp["gamma"], td_target.data_ptr(),
                                  tdp["logs"].data_ptr()) if tdp else (None, 0, None, None, None, None, 0.0, None, None)),
                               0, _lib.stream_ptr())
+        lu._batch_share_(B, B_all, dq, loss_v)
         lu._mark("join online hidden layers + output layer + loss seed")
         extra, extra_scale, f1 = None, 0.0, None
         if dr3_coeff > 0:
@@ -291,6 +298,8 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
                               use_baseline=False):
     if use_baseline:
         raise NotImplementedError("advantage baselines are out of scope")
+    lu.check_batch_sharding(agent, per=per, discrete=discrete,
+                            augmenter=augmenter if premade_replay_dicts is None else None, batch_size=batch_size)
     if discrete:   # learning.py:382-390
         return _discrete.online_actor_update(buffer, agent, pop, actor_optimizer, log_alphas, batch_size, clip, augmenter,
                                              aug_mix, premade_replay_dicts, per)
@@ -299,7 +308,9 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
     dev = aa.device
     _ops.check_cuda(aa.flat)
     L = _lib.lib()
-    E, N, B = agent.ensemble_size, agent.num_critics, batch_size
+    E, N, B_all = agent.ensemble_size, agent.num_critics, batch_size
+    lo, hi = parallel.batch_range(B_all)   # batch sharded over ranks: this rank's rows of the global batch
+    B = hi - lo
     En = parallel.members_global(E)   # loss normalisation: the global ensemble size when members are sharded over ranks
     S, A = lu._dims(agent)
     logs = _logs.DeviceLogs(dev)
@@ -310,20 +321,21 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
     concurrent = (E > 1 and premade_replay_dicts is not None and lu.side_stream(dev) is not None
                   and not parallel.critics_sharded())
 
-    def draw_member():
-        eps = torch.empty((B, A), dtype=torch.float32, device=dev)
+    def draw_member():   # (batch sharded: drawn for the global batch, rows [lo, hi) kept)
+        eps = torch.empty((B_all, A), dtype=torch.float32, device=dev)
         _rng.source().normal(eps)
         noise = None
         if agent.deterministic and random_process is not None:
-            noise = torch.empty((B, A), dtype=torch.float32, device=dev)
+            noise = torch.empty((B_all, A), dtype=torch.float32, device=dev)
             _rng.source().normal(noise)
-        return eps, noise
+        return eps[lo:hi], None if noise is None else noise[lo:hi]
 
     predrawn = [draw_member() for _ in range(E)] if concurrent else None
 
     def member_step(i):
-        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, per)
-        eps, noise = predrawn[i] if concurrent else (None, None)
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B_all, augmenter, aug_mix, per)
+        # batch sharded: the N(0,1) draws follow the batch's, as _policy_sample's do on one GPU (one Philox stream)
+        eps, noise = predrawn[i] if concurrent else draw_member() if parallel.batches_sharded() else (None, None)
         loss_v = loss_all[i:i + 1]
         o, *_ = rd["primary_batch"]
         packed = lu._packed_of(rd)
@@ -350,6 +362,7 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
             L.actor_loss_seed(q.data_ptr(), N, B, pol["logp"].data_ptr() if entropy_on else None,
                               log_alphas[i].data_ptr(), popart.state_ptr() if popart else None, int(bool(pop)), En, None,
                               dq.data_ptr(), loss_v.data_ptr(), _lib.stream_ptr())
+            lu._batch_share_(B, B_all, dq, loss_v)
         # through the critics to the action: input-gradient only (the reference's critic dW here is discarded anyway)
         da = torch.empty((B, A), dtype=torch.float32, device=dev)
         if ca.O == 1 and A <= 32:
@@ -369,7 +382,7 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
             L.det_head_backward(pol["tanh_out"].data_ptr(), da.data_ptr(), A, B, A, dout.data_ptr(), _lib.stream_ptr())
         else:
             L.tanh_normal_backward(pol["out"].data_ptr(), pol["eps"].data_ptr(), B, A, float(agent.log_std_low),
-                                   float(agent.log_std_high), da.data_ptr(), A, 1.0 / (En * B),
+                                   float(agent.log_std_high), da.data_ptr(), A, 1.0 / (En * B_all),
                                    log_alphas[i].data_ptr(), dout.data_ptr(), _lib.stream_ptr())
         _ops.mlp_backward(aa, i, 1, XPI, B, pol["h1"], pol["h2"], dout, ldx=S + A, want_dw=True, accumulate=False)
 
@@ -381,33 +394,40 @@ def _online_actor_update_impl(buffer, agent, pop, actor_optimizer, log_alphas, b
 
 def alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, aug_mix, target_entropy,
                  premade_replay_dicts, discrete):
+    lu.check_batch_sharding(agent, discrete=discrete, augmenter=augmenter if premade_replay_dicts is None else None,
+                            batch_size=batch_size)
     if discrete:   # learning.py:252-253
         return _discrete.alpha_update(buffer, agent, optimizers, batch_size, log_alphas, augmenter, aug_mix, target_entropy,
                                       premade_replay_dicts)
     lu.pipeline_barrier()
     dev = agent._actor_arena.device
-    E, B = agent.ensemble_size, batch_size
+    E, B_all = agent.ensemble_size, batch_size
+    lo, hi = parallel.batch_range(B_all)   # batch sharded over ranks: this rank's rows, the mean over the global batch
+    B = hi - lo
     S, A = lu._dims(agent)
     logs = _logs.DeviceLogs(dev)
     # one stream lane per member once the N(0,1) draws are made (in order, on the caller's stream), as in critic_update
     concurrent = E > 1 and premade_replay_dicts is not None and lu.side_stream(dev) is not None
-    predrawn = None
-    if concurrent and not agent.deterministic:
-        predrawn = []
-        for _ in range(E):
-            eps = torch.empty((B, A), dtype=torch.float32, device=dev)
-            _rng.source().normal(eps)
-            predrawn.append(eps)
+
+    def draw_eps():   # (batch sharded: drawn for the global batch, rows [lo, hi) kept)
+        eps = torch.empty((B_all, A), dtype=torch.float32, device=dev)
+        _rng.source().normal(eps)
+        return eps[lo:hi]
+
+    predrawn = [draw_eps() for _ in range(E)] if concurrent and not agent.deterministic else None
 
     def member_step(i):
-        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B, augmenter, aug_mix, False)
+        rd = lu._member_replay_dict(premade_replay_dicts, i, buffer, B_all, augmenter, aug_mix, False)
+        eps = predrawn[i] if predrawn is not None else None
+        if eps is None and parallel.batches_sharded() and not agent.deterministic:
+            eps = draw_eps()   # after the batch's draws, as _policy_sample's on one GPU (one Philox stream)
         o, *_ = rd["primary_batch"]
         with torch.no_grad():
             s_rep = agent.encoder(o)
         X = torch.empty((B, S + A), dtype=torch.float32, device=dev)
         X[:, :S].copy_(s_rep)
-        pol = lu._policy_sample(agent, i, X, B, S, A, None, None, eps=predrawn[i] if predrawn is not None else None)
-        lu._alpha_step(logs, i, optimizers[i], log_alphas[i], pol["logp"], B, target_entropy)
+        pol = lu._policy_sample(agent, i, X, B, S, A, None, None, eps=eps)
+        lu._alpha_step(logs, i, optimizers[i], log_alphas[i], pol["logp"], B_all, target_entropy)
 
     lu._run_members(E, dev, concurrent, member_step)
     return logs.finalize()
@@ -417,6 +437,8 @@ def offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batc
                          encoder_clip, augmenter, actor_lambda, aug_mix, premade_replay_dicts=None, per=True,
                          discrete=False, filter_=True):
     """AFBC / behaviour cloning actor update (reference learning.py:144-219, learning_utils.py:241-269)."""
+    if parallel.batches_sharded():
+        raise NotImplementedError("batch sharding does not cover the offline actor update")
     if discrete:   # learning_utils.py:257-258: Categorical log-likelihood, indirect advantage filter
         return _discrete.offline_actor_update(buffer, agent, actor_optimizer, encoder_optimizer, batch_size, actor_clip,
                                               update_encoder, encoder_clip, augmenter, actor_lambda, aug_mix,

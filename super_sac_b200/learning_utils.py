@@ -427,6 +427,63 @@ def _pixel_gather(stack, idx, shift, aug, B, aug_rows, use_aug):
     return out
 
 
+def _batch_rows(B, augmenter, per):
+    """This rank's rows [lo, hi) of a batch-sharded update's batch of B; refuses what cannot be split row for row."""
+    if per:
+        raise NotImplementedError("batch sharding: prioritised sampling is not supported (uniform sampling only)")
+    if not (isinstance(augmenter, augmentations.AugmentationSequence) and augmenter.fusable()):
+        raise NotImplementedError("batch sharding needs a fusable AugmentationSequence (Identity / DrQ / DrQv2)")
+    aug = augmenter.aug_list[0]
+    if getattr(aug, "noise", False):
+        raise NotImplementedError("batch sharding: noisy DrQ augmentation is not supported")
+    if getattr(aug, "batch_size", B) != B:
+        raise ValueError(f"batch sharding: the augmentation draws {aug.batch_size} shifts for a batch of {B}")
+    return parallel.batch_range(B)
+
+
+def _batch_share_(B, B_all, *ts):
+    """Scale per-row gradient seeds and logged means normalised over this rank's B rows to the global batch's B_all (the
+    ranks' shares then sum to the single-GPU values); nothing to do when the rank holds the whole batch."""
+    if B == B_all:
+        return
+    scale = torch.full((1,), B / B_all, dtype=torch.float32, device=ts[0].device)
+    for t in ts:
+        _lib.lib().scale_by_dev(t.data_ptr(), t.numel(), scale.data_ptr(), _lib.stream_ptr())
+
+
+def check_batch_sharding(agent, encoder_optimizer=None, per=False, update_priorities=False, weight_type=None,
+                         weight_temp=None, dr3_coeff=0.0, discrete=False, augmenter=None, batch_size=None):
+    """What a batch-sharded update covers (one member, uniform sampling, plain Bellman backups, no PopArt, no DR3, a
+    continuous agent, an encoder without parameters or the native pixel encoder with its fused optimiser step, and --
+    ``augmenter`` given: the update samples its own batch of ``batch_size`` -- an augmentation that splits row for row):
+    anything else raises before the update launches anything."""
+    if not parallel.batches_sharded():
+        return
+    if augmenter is not None:
+        _batch_rows(batch_size, augmenter, per)
+    why = None
+    if discrete:
+        why = "SAC-Discrete agents"
+    elif agent.ensemble_size != 1:
+        why = "ensembles of several members (E > 1)"
+    elif per or update_priorities:
+        why = "prioritised replay"
+    elif weight_type is not None and weight_temp is not None:
+        why = "weighted Bellman backups"
+    elif dr3_coeff:
+        why = "DR3"
+    elif any(bool(p) for p in agent.popart):
+        why = "PopArt"
+    elif _encoder_trainable(agent):
+        for net in _encoder_opt.native_nets(agent.encoder):   # (flattened lazily by the first forward otherwise)
+            if net._native_params()[0].is_cuda:
+                net._flatten()
+        if not _encoder_opt.structurally_eligible(agent.encoder, encoder_optimizer):
+            why = "trainable encoders other than the native pixel encoder with its fused optimiser step"
+    if why is not None:
+        raise NotImplementedError(f"batch sharding does not cover {why}")
+
+
 def sample_move_and_augment(buffer, batch_size, augmenter, aug_mix, per=True, _idx=None):
     """Sample a batch on the device, cast to fp32, augment o and o1 with shared parameters and mix the first
     int(B*aug_mix) augmented rows into the batch (reference learning_utils.py:174-214)."""
@@ -436,13 +493,17 @@ def sample_move_and_augment(buffer, batch_size, augmenter, aug_mix, per=True, _i
     st, dev, B = buffer._storage, buffer.device, batch_size
     if not torch.cuda.is_current_stream_capturing():
         buffer.total_sample_calls += 1
+    fused = isinstance(augmenter, augmentations.AugmentationSequence) and augmenter.fusable()
+    shard = _batch_rows(B, augmenter, per) if parallel.batches_sharded() else None
     if per:
         idx, imp_weights = buffer.sample_indices_per(B)
     else:
         idx = _idx if _idx is not None else buffer.sample_indices_uniform(B)
         imp_weights = _ones1(dev)
     aug_rows = int(B * aug_mix)
-    fused = isinstance(augmenter, augmentations.AugmentationSequence) and augmenter.fusable()
+    if shard is not None:   # indices drawn for the global batch: this rank gathers its rows of it
+        lo, hi = shard
+        idx, aug_rows, B = idx[lo:hi], parallel.local_aug_rows(B, aug_mix, lo, hi), hi - lo
     rd = ReplayDict()
 
     a = r = d = None
@@ -450,6 +511,8 @@ def sample_move_and_augment(buffer, batch_size, augmenter, aug_mix, per=True, _i
         aug = augmenter.aug_list[0]
         aug.change_randomization_params(dev)  # once per call; o and o1 share the shifts
         shift = getattr(aug, "shift", None)
+        if shard is not None and shift is not None:   # drawn for the global batch (aug.batch_size rows)
+            shift = shift[shard[0]:shard[1]]
         aug_keys = st.s_stack.keys() if augmenter.keys is None else augmenter.keys
         o, o1 = {}, {}
         srcs, dsts, rows, lds, modes = [], [], [], [], []
@@ -684,6 +747,7 @@ def _critic_pipeline(agent, per, update_priorities, weight_type):
     if (p is None or agent.ensemble_size != 1 or per or update_priorities or weight_type is not None
             or _encoder_trainable(agent) or any(bool(pa) for pa in agent.popart)
             or (parallel.critics_sharded() and not parallel.peer_exchange_ready()) or parallel.members_sharded()
+            or parallel.batches_sharded()
             or side_stream(dev) is None or p.device != dev):
         pipeline_barrier()
         return None
@@ -724,6 +788,11 @@ def _encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs):
     if not enc_outs:
         return None
     torch.autograd.backward([s for s, _ in enc_outs], [g for _, g in enc_outs])
+    if parallel.batches_sharded():   # the native encoder's flat gradient summed over the ranks' rows
+        net = _encoder_opt.eligible(agent.encoder, encoder_optimizer)
+        if net is None:
+            raise NotImplementedError("batch sharding trains only the native pixel encoder with its fused optimiser step")
+        parallel.all_reduce_flat_(net._flat_grad, site="encoder_grad")
     net = _encoder_opt.fused_step(agent.encoder, encoder_optimizer, encoder_clip)
     if net is None:
         if encoder_clip:
@@ -783,14 +852,19 @@ def _critic_tail(logs, loss_all, loss_slot, replay_dicts, buffer, agent, opt, pi
 
     def logged_values(on=None):
         _log_member_grad_norm(logs, ca, E, N, "gradients/critic_random_grad", stream=on)
-        if parallel.sharded():   # the loss summed over every rank, the TD error of the ensemble's last net
+        if parallel.batches_sharded():   # each rank's share of the global-batch means: summed over the ranks
+            with (torch.cuda.stream(on) if on is not None else contextlib.nullcontext()):
+                parallel.all_reduce_sum_(loss_all[0:2], site="critic_loss")
+        elif parallel.sharded():   # the loss summed over every rank, the TD error of the ensemble's last net
             with (torch.cuda.stream(on) if on is not None else contextlib.nullcontext()):
                 parallel.reduce_logged(loss_all[0:2 * E:2], loss_all[2 * E - 1:2 * E], site="critic_loss")
 
     enc_net = _encoder_step(agent, encoder_optimizer, encoder_clip, enc_outs)
+    if parallel.batches_sharded():   # every rank's share of the batch: clip, log and step the sum
+        parallel.all_reduce_flat_(ca.grad, site="critic_grad")
     if critic_clip:
         opt.grad_norm_sq(stream)
-        if parallel.sharded():   # the global norm runs over every rank's critics (SURVEY 8e (3)): one float per rank
+        if parallel.sharded() and not parallel.batches_sharded():   # the global norm runs over every rank's critics (SURVEY 8e (3)): one float per rank
             parallel.all_reduce_sum_(opt.gnorm_sq, site="critic_gnorm")
     side = None if critic_clip else side_stream(dev)   # clipping rescales the gradients that get logged
     main = torch.cuda.current_stream(dev) if side is not None or pipe is not None else None
@@ -819,6 +893,9 @@ def _actor_tail(logs, arena, opt, clip, E, grad_key, loss_v, last=None):
     ``last``, a value of the last member, the last rank's (parallel.reduce_logged).  (With the critics sharded the
     actors are replicas: nothing to exchange.)"""
     stream = _lib.stream_ptr()
+    if parallel.batches_sharded():   # every rank's share of the batch; the loss slot holds this rank's share of the mean
+        parallel.all_reduce_flat_(arena.grad, site="actor_grad")
+        parallel.all_reduce_sum_(loss_v, site="actor_loss")
     if clip:
         opt.grad_norm_sq(stream)
         if parallel.members_sharded():
@@ -860,6 +937,8 @@ class _AlphaState:
 def _alpha_step(logs, i, optimizer, log_alpha, logp, B, target_entropy):
     """Member i's temperature step (learning.py:246-262) on ``logp`` [B]: loss, scalar Adam and logs (under the global
     member id) in one launch."""
+    if parallel.batches_sharded():   # the temperature's mean runs over the global batch B: every rank, the same step
+        logp = parallel.all_gather_batch(logp, B, site="alpha_logp")
     pg = optimizer.param_groups[0]
     st = _AlphaState.attach(optimizer, log_alpha)
     lv, slot = logs.slots(2)
@@ -885,7 +964,10 @@ def draw_for_critic_member(buffer, agent, B, ensemble_n, random_process, per, ze
     subset = torch.empty(ensemble_n, dtype=torch.int32, device=dev)
     _rng.source().fill(dev, idx=idx, n_filled=len(buffer), n_filled_dev=buffer._n_filled_dev, normal=normal,
                        subset=subset, N=n_sub_pool, M=ensemble_n, zero=zero)
-    return dict(idx=idx, normal=normal, subset=subset)
+    if normal is not None and parallel.batches_sharded():   # drawn for the global batch: this rank's rows
+        lo, hi = parallel.batch_range(B)
+        normal = normal[lo:hi]
+    return dict(idx=idx, normal=normal, subset=subset, batch_size=B)
 
 
 def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ensemble_n, log_alphas, pop, gamma,
@@ -950,12 +1032,38 @@ def compute_td_targets(logs, replay_dict, agent, target_agent, ensemble_idx, ens
                          int(bool(pop)), float(popart.beta) if popart else 0.0, int(popart.min_steps) if popart else 0,
                          y.data_ptr(), lv.data_ptr(), _lib.stream_ptr())
     _mark("td target")
-    dlogs.defer(f"td_targets/mean_td_target_{g}", slot)
-    dlogs.defer(f"td_targets/std_td_target_{g}", slot + 1)
-    dlogs.defer(f"td_targets/entropy_bonus_{g}", slot + 2)
+    if parallel.batches_sharded() and parallel.world_size() > 1:
+        if _draws is None:
+            raise NotImplementedError("batch sharding: TD targets are computed inside critic_update")
+        _defer_global_td_stats(dlogs, g, lv, _draws["batch_size"])
+    else:
+        dlogs.defer(f"td_targets/mean_td_target_{g}", slot)
+        dlogs.defer(f"td_targets/std_td_target_{g}", slot + 1)
+        dlogs.defer(f"td_targets/entropy_bonus_{g}", slot + 2)
     if user_logs is not None:
         user_logs.update(dlogs.finalize())
     return y, (X1[:, :S], X1[:, S:])
+
+
+def _defer_global_td_stats(dlogs, g, lv, Bg):
+    """The logged TD-target statistics of the global batch of Bg rows from every rank's {mean, unbiased std, entropy
+    bonus} over its rows: one gather of three floats per rank, pooled (mean, pooled variance) on the host at finalize."""
+    world = parallel.world_size()
+    allv, slot = dlogs.slots(3 * world)
+    allv.view(world, 3).copy_(parallel.all_gather_batch(lv.view(1, 3), world, site="td_stats"))
+    n = [hi - lo for lo, hi in (parallel.local_range(Bg, world, r) for r in range(world))]
+    slots = tuple(range(slot, slot + 3 * world))
+    for j, name in enumerate(("mean_td_target", "std_td_target", "entropy_bonus")):
+        dlogs.defer_fn(f"td_targets/{name}_{g}", slots, lambda *v, j=j: pooled_stats(n, v[0::3], v[1::3], v[2::3])[j])
+
+
+def pooled_stats(n, means, stds, ents):
+    """(mean, unbiased std, mean entropy bonus) of a batch split into parts of n[r] rows with the given per-part mean,
+    unbiased std and entropy bonus.  A part of one row has no spread of its own (its std, 0/0, is not read)."""
+    total = sum(n)
+    m = sum(k * x for k, x in zip(n, means)) / total
+    ss = sum((k - 1) * s * s if k > 1 else 0.0 for k, s in zip(n, stds)) + sum(k * (x - m) ** 2 for k, x in zip(n, means))
+    return m, max(ss / (total - 1), 0.0) ** 0.5, sum(k * e for k, e in zip(n, ents)) / total
 
 
 def compute_backup_weights(logs, replay_dict, agent, target_agent, weight_type, weight_temp, batch_size, discrete=False,

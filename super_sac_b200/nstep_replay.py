@@ -39,7 +39,7 @@ import ctypes
 import numpy as np
 import torch
 
-from . import _lib, _ops, _rng, augmentations, graphed
+from . import _lib, _ops, _rng, augmentations, graphed, parallel
 from .replay import PriorityMax
 
 
@@ -329,15 +329,21 @@ class NStepReplayBuffer(PriorityMax):
             self.total_sample_calls += 1
         if not (isinstance(augmenter, augmentations.AugmentationSequence) and augmenter.fusable()):
             raise NotImplementedError("NStepReplayBuffer needs a fusable AugmentationSequence (Identity / DrQ / DrQv2)")
+        rows = lu._batch_rows(B, augmenter, per) if parallel.batches_sharded() else None
+        aug_rows = int(B * aug_mix)
         if per:
             res, imp_weights = self.sample_per(B)
         else:
-            res = self._resolve(_idx if _idx is not None else self.sample_indices_uniform(B))
+            idx = _idx if _idx is not None else self.sample_indices_uniform(B)
+            if rows is not None:   # indices drawn for the global batch: this rank gathers its rows of it
+                idx, aug_rows, B = idx[rows[0]:rows[1]], parallel.local_aug_rows(B, aug_mix, *rows), rows[1] - rows[0]
+            res = self._resolve(idx)
         aug = augmenter.aug_list[0]
         aug.change_randomization_params(dev)   # once per call; o and o1 share the shifts
         shift = getattr(aug, "shift", None)
+        if rows is not None and shift is not None:   # drawn for the global batch (aug.batch_size rows)
+            shift = shift[rows[0]:rows[1]]
         aug_keys = self.keys if augmenter.keys is None else augmenter.keys
-        aug_rows = int(B * aug_mix)
         rd = lu.ReplayDict()
         A = self.action.shape[1]
         o, o1 = {}, {}

@@ -16,7 +16,15 @@ One ensemble is partitioned over the ranks in one of two ways, never both at onc
   SUNRISE weight, a statistic over ALL members' target critics on each member's batch: one gather of the local batches
   and one of the local target critics' values on every batch per update (``all_gather_members``).
 
-Either way a sharded update equals the single-GPU one: the losses are normalised by the global ensemble
+- batch (``enable_batch_sharding``): ONE learner whose batch rows are split over the ranks (``batch_range``).  Every rank
+  keeps full replicas of the agent, the target agent, the optimisers, the temperatures and the replay ring; every draw
+  is made for the global batch on every rank (identical Philox state) and each rank keeps its rows, so rank r's batch is
+  rows [lo, hi) of the single-GPU batch.  Losses are normalised by the global batch, and the flat gradient arenas
+  (critics, native pixel encoder, actor) are summed over the ranks before clipping and Adam (``all_reduce_flat_``: a
+  two-shot all-reduce over NVLink, ssac_peer_allreduce) -- every rank then steps identical data and the replicas stay
+  bitwise identical.  This is the axis on which a shared, trainable encoder splits: its gradient is a sum over rows.
+
+Any of these sharded updates equals the single-GPU one: the losses are normalised by the global ensemble
 (``n_global``, ``members_global``), per-member log keys carry the global member id (``member_id``) and the logged sums
 and last-net values are the whole ensemble's (``reduce_logged``).
 
@@ -34,7 +42,8 @@ import random
 import torch
 import torch.distributed as dist
 
-# kind: None, "critics" or "members"; n: the global number of the sharded units (critics of the member, or members)
+# kind: None, "critics", "members" or "batch"; n: the global number of the sharded units (critics of the member, or
+# members; None for the batch, whose size each call names)
 _state = {"kind": None, "group": None, "world": 1, "rank": 0, "n": None}
 
 
@@ -110,7 +119,7 @@ def peer_exchange_ready():
 
 def exchange_name():
     if _peer["sites"] and _peer["why_not"] is None:
-        return "NVLink peer stores + signals (ssac_peer_put / ssac_peer_wait over symmetric memory)"
+        return "NVLink peer stores + signals (ssac_peer_put / ssac_peer_wait / ssac_peer_allreduce over symmetric memory)"
     why = "disabled" if _peer["disabled"] else (_peer["why_not"] or "not used yet / CPU tensors")
     return f"torch.distributed collectives (peer exchange unavailable: {why})"
 
@@ -125,9 +134,12 @@ def local_range(n_global, world, rank):
 
 def _enable(kind, n, group):
     if _state["kind"] not in (None, kind):
-        raise NotImplementedError(f"the {_state['kind']} are sharded already: critic sharding and member sharding "
+        raise NotImplementedError(f"the {_state['kind']} are sharded already: critic, member and batch sharding "
                                   "cannot be combined")
     world, rank = dist.get_world_size(group), dist.get_rank(group)
+    if n is None:
+        _state.update(kind=kind, group=group, world=world, rank=rank, n=None)
+        return None
     if n < world:
         raise ValueError(f"{n} {kind} cannot be sharded over {world} ranks")
     _state.update(kind=kind, group=group, world=world, rank=rank, n=int(n))
@@ -146,6 +158,26 @@ def enable_member_sharding(ensemble_size_global, group=None):
     return _enable("members", ensemble_size_global, group)
 
 
+def enable_batch_sharding(group=None):
+    """Call after ``dist.init_process_group``: every update splits its batch over the ranks (``batch_range``).  Build the
+    same Agent, target agent, optimisers and replay buffer on every rank and push the same transitions on every rank."""
+    _enable("batch", None, group)
+
+
+def batch_range(batch_size):
+    """Rows [lo, hi) of a batch of ``batch_size`` that this rank computes (all of them unless the batch is sharded)."""
+    if not batches_sharded():
+        return 0, int(batch_size)
+    if batch_size < _state["world"]:
+        raise ValueError(f"a batch of {batch_size} rows cannot be sharded over {_state['world']} ranks")
+    return local_range(int(batch_size), _state["world"], _state["rank"])
+
+
+def local_aug_rows(batch_size, aug_mix, lo, hi):
+    """How many of rows [lo, hi) are augmented: the batch's first int(B * aug_mix) rows, counted in global row numbers."""
+    return min(max(int(batch_size * aug_mix) - lo, 0), hi - lo)
+
+
 def disable():
     _state.update(kind=None, group=None, world=1, rank=0, n=None)
 
@@ -160,6 +192,15 @@ def critics_sharded():
 
 def members_sharded():
     return _state["kind"] == "members"
+
+
+def batches_sharded():
+    return _state["kind"] == "batch"
+
+
+def world_size():
+    """The number of ranks the active sharding spans (1 when nothing is sharded)."""
+    return _state["world"]
 
 
 def n_global(n_local):
@@ -207,9 +248,11 @@ def all_gather_q(q_local, site="q", select=None):
     return _all_gather_rows(q_local, site, select=select)
 
 
-def _all_gather_rows(q_local, site_name, select=None):
-    """``select`` (device int32 [m]): return only those global rows (cheaper than gathering everything and indexing)."""
-    n, world, rank, group = _state["n"], _state["world"], _state["rank"], _state["group"]
+def _all_gather_rows(q_local, site_name, select=None, n=None):
+    """``select`` (device int32 [m]): return only those global rows (cheaper than gathering everything and indexing).
+    ``n``: the global number of rows (default: the sharded units)."""
+    world, rank, group = _state["world"], _state["rank"], _state["group"]
+    n = _state["n"] if n is None else int(n)
     row = q_local[0].numel() * q_local.element_size() if q_local.shape[0] else 0
     site = _site(site_name, n * row, group, q_local.device) if row else None
     if site is not None:
@@ -281,3 +324,80 @@ def all_gather_members(x_local):
     x = x_local.reshape((hi - lo, k) + tuple(x_local.shape[1:]))
     out = _all_gather_rows(x.contiguous(), "members%d" % (x[0].numel() if x.shape[0] else 0))
     return out.reshape((_state["n"] * k,) + tuple(x_local.shape[1:]))
+
+
+def all_gather_batch(x_local, batch_size, site):
+    """x_local [hi - lo, ...] (this rank's rows of a batch-sharded update) -> [batch_size, ...] in global row order: the
+    per-row values whose statistics are logged (TD targets, log-probs) then go through the unchanged single-GPU kernels."""
+    return _all_gather_rows(x_local.contiguous(), site, n=batch_size)
+
+
+class _AllreduceSite:
+    """Symmetric buffer of ssac_peer_allreduce: two epoch halves of {in, out} regions of ``cap`` bytes, a symmetric
+    signal row of 128 uint32 (staged / reduced), a device epoch and the local ticket counters of the kernels' last block."""
+
+    def __init__(self, n, group, device):
+        import torch.distributed._symmetric_memory as symm
+
+        from . import _lib
+
+        self.lib = _lib
+        self.group = group if group is not None else dist.group.WORLD
+        self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
+        self.n = int(n)
+        self.cap = (4 * self.n + 15) // 16 * 16
+        name = self.group.group_name
+        try:
+            symm.enable_symm_mem_for_group(name)
+        except Exception:  # noqa: BLE001  (newer torch enables groups lazily)
+            pass
+        self.buf = symm.empty(4 * self.cap, dtype=torch.uint8, device=device)
+        self.sig = symm.empty(128, dtype=torch.int32, device=device)
+        self.sig.zero_()
+        self._hb = symm.rendezvous(self.buf, name)
+        self._hs = symm.rendezvous(self.sig, name)
+        self.buf_ptrs = torch.tensor([int(p) for p in self._hb.buffer_ptrs], dtype=torch.int64, device=device)
+        self.sig_ptrs = torch.tensor([int(p) for p in self._hs.buffer_ptrs], dtype=torch.int64, device=device)
+        self.epoch = torch.zeros(1, dtype=torch.int32, device=device)
+        self.ticket = torch.zeros(2, dtype=torch.int32, device=device)
+        torch.cuda.synchronize(device)
+        dist.barrier(group=group)   # every rank's signals are zeroed and mapped before the first stage
+
+    def __call__(self, src, dst):
+        self.lib.lib().peer_allreduce(src.data_ptr(), dst.data_ptr(), self.n, self.buf.data_ptr(), self.cap,
+                                      self.buf_ptrs.data_ptr(), self.sig.data_ptr(), self.sig_ptrs.data_ptr(), self.rank,
+                                      self.world, self.epoch.data_ptr(), self.ticket.data_ptr(), self.lib.stream_ptr())
+
+
+def _allreduce_site(name, n, group, device):
+    """The all-reduce site ``name`` for n floats (created on first use, outside any stream capture), or None when peer
+    memory is not available (the reason is kept for ``exchange_name()``), as ``_site``."""
+    if _peer["disabled"] or _peer["why_not"] is not None or device.type != "cuda":
+        return None
+    key = ("allreduce", name, int(n), id(group))
+    site = _peer["sites"].get(key)
+    if site is None:
+        if torch.cuda.is_current_stream_capturing():
+            return None
+        try:
+            site = _peer["sites"][key] = _AllreduceSite(n, group, device)
+        except Exception as e:  # noqa: BLE001
+            _peer["why_not"] = f"{type(e).__name__}: {str(e)[:120]}"
+            return None
+    return site
+
+
+def all_reduce_flat_(t, site):
+    """Sum the contiguous fp32 tensor ``t`` (a flat gradient arena) over the ranks in place, with the same bits on every
+    rank: ssac_peer_allreduce over NVLink peer memory, else ``torch.distributed.all_reduce``.  ``site`` names the call
+    site (one symmetric buffer each, used from one stream)."""
+    if not t.is_contiguous() or t.dtype != torch.float32:
+        raise ValueError("all_reduce_flat_: a contiguous fp32 tensor")
+    if t.numel() == 0:
+        return t
+    peer = _allreduce_site(site, t.numel(), _state["group"], t.device)
+    if peer is not None:
+        peer(t, t)
+        return t
+    dist.all_reduce(t, op=dist.ReduceOp.SUM, group=_state["group"])
+    return t
